@@ -188,12 +188,15 @@ __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO&
 // diagnostics outputs (zs_launch picks it when a launch has that shape).
 // PROD: the observation of every step is handed to the CTA's producer warp (zs_obs.cuh: obs_producer) instead of being
 // written by the game warp: no bulk-copy issue, no wait for it, no global stores on the game warps' dependent chain.
-template <int MPC, int G, bool CV, bool FAST, bool SURR, bool PROD = false>
+// ROS: a game roster compiled in (zs_world.cuh: Roster; the standard rollout shape only), 0 = the game from ZsParams.
+template <int MPC, int G, bool CV, bool FAST, bool SURR, bool PROD = false, int ROS = 0>
 __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io, Env& e) {
     ZS_CONSTS; ZS_VIEWS;
     const int lane = e.gl, env = e.env;
     ObsMail* const mail = PROD ? reinterpret_cast<ObsMail*>(zs_smem + p.prod_off + (int)(e.b / (uint32_t)p.smem_per_env) * ((int)sizeof(ObsMail) + 8 * p.prod_cap)) : nullptr;
-    const int A = FAST ? 1 : p.A, P = p.P, NP = P + A;
+    using R = Roster<ROS>;
+    static_assert(!R::on || (FAST && !PROD), "rosters are compiled into the standard rollout shape");
+    const int A = FAST ? 1 : p.A, P = R::on ? R::P : p.P, NP = P + A;
     const int aidx = lane - P;
     const bool is_agent = aidx >= 0 && aidx < A;
     const bool per_agent = FAST ? false : p.obs_per_agent != 0;
@@ -243,7 +246,7 @@ __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io,
         PH(19);
         PH(0);
 
-        int k = world_step_one<MPC, G, CV>(p, e, my_at, my_dx, my_dy);
+        int k = world_step_one<MPC, G, CV, ROS>(p, e, my_at, my_dx, my_dy);
         e.ep_steps += 1;
         if (step == io.n_steps - 1) TR(25);
 
@@ -271,7 +274,7 @@ __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io,
 
         // ---- rules and end reward (gym_env.py:130-141, multiagent_env.py:143-162)
         bool ended, won, agents_alive;
-        rules_eval<MPC, G, CV>(p, e, ended, won, agents_alive);
+        rules_eval<MPC, G, CV, ROS>(p, e, ended, won, agents_alive);
         bool done = false, trunc = false;
         double end_reward = 0.0;
         if (ended) { done = true; end_reward = won ? 10.0 : -10.0; }
@@ -305,7 +308,7 @@ __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io,
                 atomicAdd(p.stats + 2, (unsigned long long)e.ep_steps);
                 atomicAdd(p.stats + 3, (unsigned long long)e.zd);
             }
-            if (p.fast_init) initialize_world_fast<MPC, G, CV>(p, e, need_init);  // both envs of the warp, converged
+            if (R::on || p.fast_init) initialize_world_fast<MPC, G, CV, ROS>(p, e, need_init);  // both envs of the warp, converged
             else if (need_init) {  // possibly only one env of the warp: the divergent flavour
                 initialize_world<MPC, G, false>(p, id_of(e), e.episode + 1, e.flags);
                 scalars_from_smem<MPC, G, false>(p, e);
@@ -387,7 +390,8 @@ __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io,
 // SHAPE 3 = the standard rollout shape with a producer warp: CTAs of four game warps (eight envs) plus one warp that writes
 // the observations (160 threads; compiled for 4 CTAs per SM: 20 warps, five per scheduler = 96 registers, and 4,096 envs
 // are one wave.  Three-warp CTAs at seven per SM would put six warps on one scheduler: 80 registers and spills).
-template <int MODE, int MPC, int G, int SHAPE, int OCC>
+// ROS: the game roster compiled into a standard-rollout-shape kernel (zs_world.cuh: Roster), 0 = read from ZsParams.
+template <int MODE, int MPC, int G, int SHAPE, int OCC, int ROS = 0>
 __global__ void __launch_bounds__(SHAPE == 3 ? 160 : ZS_WPC * 32, OCC) zs_sim_kernel(const __grid_constant__ ZsParams p, const __grid_constant__ ZsIO io) {
     ZS_CONSTS;
     constexpr bool PROD = SHAPE == 3;
@@ -497,7 +501,7 @@ __global__ void __launch_bounds__(SHAPE == 3 ? 160 : ZS_WPC * 32, OCC) zs_sim_ke
 #ifdef ZS_PHASE_CLOCKS
     e.ph_last = clock64();
 #endif
-    if constexpr (ONE) step_loop_one<MPC, G, CV, FAST, SURR, PROD>(p, io, e);
+    if constexpr (ONE) step_loop_one<MPC, G, CV, FAST, SURR, PROD, ROS>(p, io, e);
     else step_loop_general<MPC, G, CV, SURR>(p, io, e);
 #ifdef ZS_PHASE_CLOCKS
     e.ph_last = clock64();
@@ -602,6 +606,7 @@ struct ZsHandle {
     double host_stats[5] = {0, 0, 0, 0, 0};  // zs_step_host: calls, and summed us from entry to: launched / previous cells restored / flag seen / return
     std::vector<int32_t> tmpl_obs_host;  // the pristine observation planes [obs_C][cells] (zs_expand_compact)
     int tmpl_single_step;  // launches of fewer than four steps stage the observation template for the TMA as well
+    int roster;            // the game as a roster (zs_world.cuh: Roster) when the standard rollout kernel has it compiled in, else 0
     bool img_valid;  // the parked images (ZsParams::img) match the canonical state of every env
 };
 
@@ -710,6 +715,8 @@ static void launch_sim(const ZsHandle* h, const ZsIO& io, cudaStream_t st) {
     const bool fast = MODE == MODE_STEP && pp.mpc <= 32 && pp.A == 1 && !pp.obs_per_agent && pp.minimum_zombies == 0 &&
                       pp.obs_scope == ZS_OBS_WORLD && io.actions && io.fmt == ZS_ACTIONS_DISCRETE && io.obs && io.reward &&
                       io.terminated && io.truncated && !io.draws && !io.agent_mask;
+    // ... and with the handle's game compiled in when it is an instantiated roster (only the bench game's, at 16 slots)
+    const bool roster = fast && h->roster == ZS_ROSTER_BENCH && pp.mpc == 16;
     const int occ = MODE == MODE_STEP ? sh.occ : ZS_MIN_CTAS;
     const bool surr = pp.obs_scope == ZS_OBS_SURROUNDINGS;
     // the standard rollout shape of a batch that one wave of producer-warp CTAs holds: observations through a third warp
@@ -728,8 +735,10 @@ static void launch_sim(const ZsHandle* h, const ZsIO& io, cudaStream_t st) {
     // rollouts lose 1-1.5 % — the early CTAs of the next launch sit on the SMs — so only short step launches ask for it)
     const bool pdl = h->use_pdl == 1 || (h->use_pdl == 2 && MODE == MODE_STEP && io.n_steps < h->short_steps);
     lc.attrs = la; lc.numAttrs = pdl ? 1 : 0;
-#define ZS_LAUNCH(MPC_, G_, SH_, O_) cudaLaunchKernelEx(&lc, zs_sim_kernel<MODE, MPC_, G_, ((SH_) == 1 && MODE != MODE_STEP) ? 0 : (SH_), MODE == MODE_STEP ? (O_) : ZS_MIN_CTAS>, pp, io)
-#define ZS_LAUNCH_F(MPC_, G_, O_) do { if (fast) ZS_LAUNCH(MPC_, G_, 1, O_); else if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); else ZS_LAUNCH(MPC_, G_, 0, O_); } while (0)
+#define ZS_LAUNCH_R(MPC_, G_, SH_, O_, R_) cudaLaunchKernelEx(&lc, zs_sim_kernel<MODE, MPC_, G_, ((SH_) == 1 && MODE != MODE_STEP) ? 0 : (SH_), MODE == MODE_STEP ? (O_) : ZS_MIN_CTAS, MODE == MODE_STEP ? (R_) : 0>, pp, io)
+#define ZS_LAUNCH(MPC_, G_, SH_, O_) ZS_LAUNCH_R(MPC_, G_, SH_, O_, 0)
+#define ZS_LAUNCH_F(MPC_, G_, O_) do { if (roster) ZS_LAUNCH_R(MPC_, G_, 1, O_, (MPC_) == 16 ? ZS_ROSTER_BENCH : 0); else if (fast) ZS_LAUNCH(MPC_, G_, 1, O_); \
+                                       else if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); else ZS_LAUNCH(MPC_, G_, 0, O_); } while (0)
 #define ZS_LAUNCH_G(MPC_, G_, O_) do { if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); else ZS_LAUNCH(MPC_, G_, 0, O_); } while (0)
     if (prod) {
         pp.prod_off = sh.prod_off; pp.prod_cap = sh.prod_cap; pp.tmpl_smem_off = ZS_PROD_ENVS * sh.smem_per_env;
@@ -758,6 +767,7 @@ static void launch_sim(const ZsHandle* h, const ZsIO& io, cudaStream_t st) {
 #undef ZS_LAUNCH_G
 #undef ZS_LAUNCH_F
 #undef ZS_LAUNCH
+#undef ZS_LAUNCH_R
     if (pp.img != nullptr && (MODE == MODE_STEP || MODE == MODE_RESET) && io.env_mask == nullptr) const_cast<ZsHandle*>(h)->img_valid = true;
 }
 template <int MPC, int G, int OCC>
@@ -765,6 +775,7 @@ static cudaError_t set_smem_attr_step(int bytes) {
     const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
     cudaError_t e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, 0, OCC>, attr, bytes);
     if (e == cudaSuccess && MPC <= 32) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (MPC <= 32 ? 1 : 0), OCC>, attr, bytes);
+    if (e == cudaSuccess && MPC == 16) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (MPC == 16 ? 1 : 0), OCC, (MPC == 16 ? ZS_ROSTER_BENCH : 0)>, attr, bytes);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, 2, OCC>, attr, bytes);
     return e;
 }
@@ -973,6 +984,11 @@ extern "C" __attribute__((visibility("default"))) int zs_create(const ZsConfig* 
     for (int i = 0; i < p.P; ++i) if (p.bot_kinds[i] != ZS_KIND_TERMINATOR && p.bot_kinds[i] != ZS_KIND_SNIPER) p.fast_init = 0;
     for (int i = 0; i < p.A; ++i) if (p.agent_weapons[i] == ZS_WEAPON_RANDOM) p.fast_init = 0;
     if (getenv("ZS_NO_FAST_INIT")) p.fast_init = 0;
+    // the game as a roster (launch_sim: the standard rollout kernel with it compiled in); ZS_NO_ROSTER keeps the kernel that
+    // reads the game from the parameters (the reference the roster kernels are tested against)
+    bool all_terminators = true;
+    for (int i = 0; i < p.P; ++i) all_terminators &= p.bot_kinds[i] == ZS_KIND_TERMINATOR;
+    h->roster = p.fast_init && p.A == 1 && all_terminators && !getenv("ZS_NO_ROSTER") ? zs_roster(p.rules, p.P + p.A) : 0;
     if (p.fast_init) {
         cand = p.n_ps + p.n_zs;  // both index lists side by side
     }

@@ -10,6 +10,17 @@
     constexpr bool ONE = MPC <= G;                  \
     (void)ONE
 
+// A game roster compiled into the standard rollout kernel: the rules, the player count NP (bots + ONE agent) and every
+// bot a terminator.  ROS = 0 reads the game from ZsParams instead.  Under a roster the player loops, the lane tests and
+// the bot-kind predicates of the step fold to constants, and the randoman path and the rules dispatch drop out.
+// launch_sim picks a roster kernel when the handle's game is one (ZsHandle::roster, set by zs_create).
+constexpr int zs_roster(int rules, int np) { return 1 + rules + 4 * np; }
+template <int ROS> struct Roster {
+    static constexpr bool on = ROS != 0;
+    static constexpr int rules = on ? (ROS - 1) & 3 : -1, NP = on ? (ROS - 1) >> 2 : -1, P = NP - 1;
+};
+#define ZS_ROSTER_BENCH zs_roster(ZS_RULES_EXTERMINATION, 3)  // the bench game: agent + 2 terminators, extermination
+
 // identity of a lane group, passed by value to the out-of-line functions (keeps the caller's Env in registers)
 struct GrpId { uint32_t b; int32_t env; int32_t gl; uint32_t gm; int32_t gshift; };
 __device__ __forceinline__ Env env_of(const ZsParams& p, const GrpId& id) {
@@ -1188,11 +1199,13 @@ ZS_TPL __device__ __noinline__ void execute_sequential(const ZsParams& p, GrpId 
 }
 
 // (at, adx, ady): the action of the agent whose slot this lane is (Agent.set_action, agent.py:22-25).
-ZS_TPL __device__ __forceinline__ int world_step_one(const ZsParams& p, Env& e, int at, int adx, int ady) {
+template <int MPC, int G, bool CV, int ROS = 0>
+__device__ __forceinline__ int world_step_one(const ZsParams& p, Env& e, int at, int adx, int ady) {
     ZS_VIEWS;
     static_assert(MPC <= G, "one lane per slot");
+    using R = Roster<ROS>;
     const int s = e.gl;  // slot in slot space, list position in position space
-    const int NP = p.P + p.A;
+    const int P = R::on ? R::P : p.P, NP = R::on ? R::NP : p.P + p.A;
     const unsigned below_s = (1u << s) - 1u;
     e.t += 1;
     const uint32_t t_word = (uint32_t)(e.t + 1);
@@ -1203,8 +1216,8 @@ ZS_TPL __device__ __forceinline__ int world_step_one(const ZsParams& p, Env& e, 
     const bool live = rk != RK_NONE;
     const uint32_t xy = live ? TXY(s) : 0u;
     const int x = xy_x(xy), y = xy_y(xy);
-    const bool zombie = s >= NP, agent = !zombie && s >= p.P;
-    const int bkind = s < p.P ? (int)p.bot_kinds[s] : -1;
+    const bool zombie = s >= NP, agent = !zombie && s >= P;
+    const int bkind = s < P ? (R::on ? (int)ZS_KIND_TERMINATOR : (int)p.bot_kinds[s]) : -1;
     if (!(live && agent)) at = ZS_ACT_NONE;
     else if (at == ZS_ACT_ABSENT) { at = ZS_ACT_HEAL; adx = 0; ady = 0; }  // multiagent_env.py:129-131
     // what is on the four adjacent cells (utils.py:34-44) does not depend on the target: read it now, so the loads
@@ -1323,7 +1336,7 @@ ZS_TPL __device__ __forceinline__ int world_step_one(const ZsParams& p, Env& e, 
     PH(2);
     // wandering zombies and hamsters draw random.choice(positions) in dict order (things.py:101-103, hamster.py:12-14)
     int nd = 0;
-    if (p.has_randoman) {
+    if (!R::on && p.has_randoman) {
         if (wany<G, CV>(e, type == D_WANDER || type == D_RANDOM)) {
             if (in_cap) { MPOS(s) = (uint8_t)type; BK(s) = freemask; }  // (MPOS = DTYPE, free until the list is built)
             gsync<G, CV>(e);
@@ -1820,10 +1833,14 @@ ZS_TPL __device__ __noinline__ int spawn_zombies(const ZsParams& p, GrpId id, in
 // Runs CONVERGED (CV): both envs of a warp go through it when either ends an episode, the writes predicated on
 // `need`.  Same results as the general initialize_world below.  Returns the draws consumed; the scalars of the new
 // world go straight into e.
-ZS_TPL __device__ __forceinline__ int initialize_world_fast(const ZsParams& p, Env& e, bool need) {
+// Under a roster (ROS) the group sizes but the zombies' are constants: the trace-back runs for a constant count and the
+// agents' candidates come from the bots' picks broadcast once, with the fixpoint in registers.
+template <int MPC, int G, bool CV, int ROS = 0>
+__device__ __forceinline__ int initialize_world_fast(const ZsParams& p, Env& e, bool need) {
     ZS_VIEWS;
+    using R = Roster<ROS>;
     const int s = e.gl;
-    const int P = p.P, A = p.A, NP = P + A, Z0 = p.initial_zombies;
+    const int P = R::on ? R::P : p.P, A = R::on ? 1 : p.A, NP = P + A, Z0 = p.initial_zombies;
     const uint32_t episode = (uint32_t)(e.episode + 1);
     // draw indices (A.7 of SURVEY.md): players shuffle, agents shuffle, zombie lives, zombies shuffle; a shuffle of n
     // candidates consumes n - 1 draws whatever is placed
@@ -1843,7 +1860,15 @@ ZS_TPL __device__ __forceinline__ int initialize_world_fast(const ZsParams& p, E
     const int life = s < NP ? 100 : 50 + below(word_of(o2, kl & 3), 51);
     int q = placed ? j : -1;
     const int tmax = max(max(P, A), Z0);
-    if constexpr (MPC <= 16 && CV) {
+    if constexpr (R::on) {
+        // a group of n things needs iterations t < n - 1 only (t < it): the bots have P, the zombies at most MPC - NP
+        constexpr int TB = R::P > MPC - R::NP ? R::P : MPC - R::NP;
+#pragma unroll
+        for (int t = TB - 2; t >= 0; --t) {
+            const int jt = gbcast<G, CV>(e, j, (base + t) & (G - 1));
+            if (t < it && jt == q) q = n - 1 - t;
+        }
+    } else if constexpr (MPC <= 16 && CV) {
         // (the step loop's converged call, which is latency-bound: unrolled, the shuffles do not depend on one another and go
         // out back to back, only the compare-select chain is serial.  The reset kernel, which is throughput-bound and runs the
         // member-mask flavour, is 8 % faster with the loop)
@@ -1861,7 +1886,22 @@ ZS_TPL __device__ __forceinline__ int initialize_world_fast(const ZsParams& p, E
             if (t < it && jt == q) q = n - 1 - t;
         }
     }
-    if (P > 0) {  // (an agent's q counts the player spawn cells the bots left)
+    if constexpr (R::on) {
+        if constexpr (R::P > 0) {
+            int qb[R::P > 0 ? R::P : 1];
+#pragma unroll
+            for (int b = 0; b < R::P; ++b) qb[b] = gbcast<G, CV>(e, q, b);
+            int x = q;
+#pragma unroll
+            for (int r = 0; r < R::P; ++r) {
+                int c = 0;
+#pragma unroll
+                for (int b = 0; b < R::P; ++b) c += qb[b] <= x;
+                x = q + c;
+            }
+            if (is_agent) q = x;
+        }
+    } else if (P > 0) {  // (an agent's q counts the player spawn cells the bots left)
         int x = q;
 #pragma unroll 1
         for (int r = 0; r < P; ++r) {
@@ -1904,8 +1944,8 @@ ZS_TPL __device__ __forceinline__ int initialize_world_fast(const ZsParams& p, E
     TR(22);
     if (need && in_cap) {
         int w = ZS_WEAPON_CLAWS;
-        if (is_bot) w = p.bot_kinds[s] == ZS_KIND_SNIPER ? ZS_WEAPON_RIFLE : ZS_WEAPON_SHOTGUN;  // sniper.py:23-24, terminator.py:41-42
-        else if (is_agent) w = p.agent_weapons[s - P];
+        if (is_bot) w = !R::on && p.bot_kinds[s] == ZS_KIND_SNIPER ? ZS_WEAPON_RIFLE : ZS_WEAPON_SHOTGUN;  // sniper.py:23-24, terminator.py:41-42
+        else if (is_agent) w = p.agent_weapons[R::on ? 0 : s - P];
         TM(s) = (uint8_t)(placed ? (w | 0x80) : w);
         RK(s) = placed ? (uint8_t)s : (uint8_t)RK_NONE;
         MVQ(s) = RK_NONE;
@@ -2018,30 +2058,39 @@ ZS_TPL __device__ __noinline__ int initialize_world(const ZsParams& p, GrpId id,
 }
 
 // ---------------------------------------------------------------- rules (zombsole/rules/*.py)
-ZS_TPL __device__ __forceinline__ void rules_eval(const ZsParams& p, Env& e, bool& ended, bool& won, bool& agents_alive) {
+template <int MPC, int G, bool CV, int ROS = 0>
+__device__ __forceinline__ void rules_eval(const ZsParams& p, Env& e, bool& ended, bool& won, bool& agents_alive) {
     ZS_CONSTS; ZS_VIEWS;
+    using R = Roster<ROS>;
+    static_assert(!R::on || ONE, "a roster kernel has one lane per slot");
     const int lane = e.gl;
-    const int NP = p.P + p.A;
+    const int P = R::on ? R::P : p.P, NP = R::on ? R::NP : p.P + p.A;
+    const int rules = R::on ? R::rules : p.rules;
     int alive = 0, ag = 0;
 #pragma unroll 1
     for (int s0 = 0; s0 < (ONE ? 1 : (NP)); s0 += G) {
         const int s = s0 + lane;
         const bool al = s < NP && TL(s) > 0;
         alive += __popc(gballot<G, CV>(e, al));
-        ag += __popc(gballot<G, CV>(e, al && s >= p.P));
+        ag += __popc(gballot<G, CV>(e, al && s >= P));
     }
     agents_alive = ag > 0;                    // rules/rules.py:13-18
     const bool players_alive = alive > 0;     // rules/rules.py:6-11
     won = players_alive;
-    if (p.rules == ZS_RULES_EXTERMINATION) {  // extermination.py:12-26
+    if (rules == ZS_RULES_EXTERMINATION) {  // extermination.py:12-26
         bool z = false;
+        if constexpr (R::on) {  // (one lane per slot: every zombie slot is NP + lane of some lane)
+            const int s = NP + e.gl;
+            z = s < p.M && (TM(s) & 0x80) && TL(s) > 0;
+        } else {
 #pragma unroll 1
-        for (int s = NP + e.gl; s < p.M; s += G) z |= (TM(s) & 0x80) && TL(s) > 0;
+            for (int s = NP + e.gl; s < p.M; s += G) z |= (TM(s) & 0x80) && TL(s) > 0;
+        }
         const bool any_z = gany<G, CV>(e, z);  // (every lane of the warp votes: no short-circuit around a primitive)
         ended = !players_alive || !any_z;
-    } else if (p.rules == ZS_RULES_SURVIVAL) {  // survival.py:5-7
+    } else if (rules == ZS_RULES_SURVIVAL) {  // survival.py:5-7
         ended = !players_alive;
-    } else if (p.rules == ZS_RULES_SAFEHOUSE) {  // safehouse.py:10-32
+    } else if (rules == ZS_RULES_SAFEHOUSE) {  // safehouse.py:10-32
         bool out = false;
 #pragma unroll 1
         for (int s = e.gl; s < NP; s += G) {
