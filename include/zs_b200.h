@@ -22,6 +22,9 @@
  *   zs_rollout       a K-step loop of the above with same-step auto-reset (what an RL rollout does
  *                    around gym_env.py:99-164); one launch, state stays on chip between steps
  *   zs_fill_synthetic_actions   Discrete(6|7).sample() for synthetic rollouts (gym_env.py:367)
+ *   zs_step_compact_agents / zs_expand_compact_agents / zs_step_host_agents
+ *                    MultiagentZombsoleEnv.step with its per-agent windows  zombsole/gym/multiagent_env.py:111-171,
+ *                    returned to a caller on the host                         zombsole/gym/observation.py:99-119
  *
  * Conventions: every `*_dev` / output pointer is a DEVICE pointer owned by the
  * caller (torch allocates); ZsConfig/ZsMap and the pointers inside them are HOST
@@ -276,6 +279,49 @@ int zs_step_host(ZsHandle* h, const int32_t* actions_host, int32_t action_format
                  uint32_t* prev_host, int32_t compact_words, int32_t* obs_dev, int32_t* obs_host, double* reward_host,
                  uint8_t* terminated_host, uint8_t* truncated_host, int32_t* overflow_envs_host, int32_t* n_overflow,
                  int32_t first_call, int32_t n_threads, void* stream);
+/* ---- compact host outputs for per-agent surroundings observations (the multi-agent env)
+ * Every agent's observation is the (w, w) window of the map around it: MultiagentZombsoleEnv.step builds one per agent
+ * (zombsole/gym/multiagent_env.py:111-171) from observation.py:99-119.  Most of a window is the map's pristine layer
+ * (out-of-bounds cells are a fresh Wall), so one fixed-size record per env carries the agents' window centres and the
+ * cells any window shows that differ from that layer.  With A = n_agents, H = ZS_AGENT_COMPACT_HEADER(A) words:
+ *   word 0          bits 0-15 number of entries, bit 16 terminated, bit 17 truncated, bit 18 overflow
+ *   word 1          agent mask: bit a = agent a was alive before the step (zs_step's agent_mask_dev)
+ *   words 2..2+2A-1 the reward of agent a as float64 bits, two words each, little endian
+ *   words 2+2A..H-1 per agent: bits 0-15 the cell (y * width + x) its window is centred on (the agent slot's position,
+ *                   where it died if it is dead), bits 16-31 its life after the step (and after the step's auto-reset)
+ *                   as int16
+ *   words H..       the entries, encoded as in the world record: box/wall patches, dead bodies, mobile things, each one
+ *                   only if its cell lies inside at least one agent's window
+ * Overflow follows the world record's rules (too many entries, or a value outside its field): the env's full rows
+ * [A, C, w, w] are written to obs_dev for the caller to fetch.  Available for obs_scope = ZS_OBS_SURROUNDINGS with
+ * obs_per_agent = 1, at most 32 slots and fewer than 65,536 cells; both encodings.
+ * zs_agent_compact_words: a good record size for this handle (0 outside that scope); zs_agent_compact_max_words: the
+ * size no env overflows by count.  As for the world record, the caller may grow compact_words between steps. */
+#define ZS_AGENT_COMPACT_HEADER(A) (2 + 3 * (A))
+int32_t zs_agent_compact_words(const ZsHandle* h);
+int32_t zs_agent_compact_max_words(const ZsHandle* h);
+int zs_step_compact_agents(ZsHandle* h, const int32_t* actions_dev, int32_t action_format, uint32_t* compact_dev,
+                           int32_t compact_words, int32_t* obs_dev, void* stream);
+/* HOST code, threaded: records -> obs_host int32 [N, A, C, w, w], byte-identical to what zs_step writes, reward_host
+ * float64 [N, A], terminated_host / truncated_host uint8 [N], agent_mask_host uint8 [N, A], agent_life_host int16 [N, A].
+ * Incremental per env and agent: a window whose centre moved (or on the first call, or after the env's previous record
+ * overflowed) is copied from the pristine layer; otherwise only the previous record's cells inside it are restored.  Then
+ * the new entries are written into every window that shows them.  prev_host, overflow_envs_host, n_overflow, first_call
+ * and n_threads as for zs_expand_compact. */
+int zs_expand_compact_agents(const ZsHandle* h, const uint32_t* compact_host, uint32_t* prev_host, int32_t* obs_host,
+                             double* reward_host, uint8_t* terminated_host, uint8_t* truncated_host,
+                             uint8_t* agent_mask_host, int16_t* agent_life_host, int32_t* overflow_envs_host,
+                             int32_t* n_overflow, int32_t compact_words, int32_t first_call, int32_t n_threads);
+/* zs_step_compact_agents + zs_expand_compact_agents in one call for a caller whose buffers live in host memory: the same
+ * transport as zs_step_host (actions copied ahead of the launch, records written by the kernel into compact_pinned, a flag
+ * in pinned memory, host threads waiting for it, ten seconds until it gives up).  The threads expand every env after the
+ * flag: whether a window is restored cell by cell or copied whole depends on the new record.  ZS_HOST_DIFF has no effect
+ * here. */
+int zs_step_host_agents(ZsHandle* h, const int32_t* actions_host, int32_t action_format, uint32_t* compact_pinned,
+                        uint32_t* prev_host, int32_t compact_words, int32_t* obs_dev, int32_t* obs_host, double* reward_host,
+                        uint8_t* terminated_host, uint8_t* truncated_host, uint8_t* agent_mask_host,
+                        int16_t* agent_life_host, int32_t* overflow_envs_host, int32_t* n_overflow, int32_t first_call,
+                        int32_t n_threads, void* stream);
 /* diagnostics: out[5] = zs_step_host calls since the last read, and the mean microseconds from entry until the launches
  * were issued / thread 0 had restored the cells of its previous records / the flag showed (every record in host memory) /
  * the call returned (every env expanded) */

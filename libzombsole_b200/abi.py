@@ -83,6 +83,14 @@ PROTOTYPES = {
     "zs_step_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
     "zs_step_host_stats": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "zs_agent_compact_words": (C.c_int32, [C.c_void_p]),
+    "zs_agent_compact_max_words": (C.c_int32, [C.c_void_p]),
+    "zs_step_compact_agents": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
+    "zs_expand_compact_agents": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32]),
+    "zs_step_host_agents": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                      C.c_int32, C.c_void_p]),
     "zs_init_static_life": (C.c_int, [C.c_void_p, C.c_void_p]),
     "zs_reset": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "zs_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,

@@ -180,6 +180,23 @@ __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO&
     }
 }
 
+// zs_step_host: the env's record is complete.  ONE system-scope fence per group of envs, by whoever completes the group (a fence
+// per warp takes 8-34 us when 4,096 warps fence at once): the others order their record words before the counter at gpu scope.
+template <int G, bool CV>
+__device__ __forceinline__ void compact_signal(const ZsParams& p, const ZsIO& io, const Env& e, int env) {
+    __threadfence();
+    gsync<G, CV>(e);
+    if (e.gl == 0) {
+        const int grp = env / io.group_envs;
+        const int size = min(io.group_envs, p.N - grp * io.group_envs);
+        if (atomicAdd(io.group_count + grp, 1) == size - 1) {
+            io.group_count[grp] = 0;
+            __threadfence_system();
+            *reinterpret_cast<volatile uint32_t*>(io.host_flags + 16 * grp) = io.ticket;
+        }
+    }
+}
+
 // ---------------------------------------------------------------- the K-step loop, one lane per slot
 // Agent a is handled by the lane of its slot (P + a): its action, its tracker life and its reward never leave
 // that lane's registers.  Output cursors advance by one step's stride instead of being recomputed.
@@ -189,7 +206,8 @@ __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO&
 // PROD: the observation of every step is handed to the CTA's producer warp (zs_obs.cuh: obs_producer) instead of being
 // written by the game warp: no bulk-copy issue, no wait for it, no global stores on the game warps' dependent chain.
 // ROS: a game roster compiled in (zs_world.cuh: Roster; the standard rollout shape only), 0 = the game from ZsParams.
-template <int MPC, int G, bool CV, bool FAST, bool SURR, bool PROD = false, int ROS = 0>
+// REC: surroundings scope with the per-agent compact record compiled in (zs_sim_kernel SHAPE 4).
+template <int MPC, int G, bool CV, bool FAST, bool SURR, bool PROD = false, int ROS = 0, bool REC = false>
 __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io, Env& e) {
     ZS_CONSTS; ZS_VIEWS;
     const int lane = e.gl, env = e.env;
@@ -317,37 +335,41 @@ __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io,
         PH(10);
         if (step == io.n_steps - 1) TR(27);
         bool compacted = false;
-        if constexpr (!FAST && world_obs) {
-            if (io.compact) {  // the observation as a compact record (include/zs_b200.h: zs_step_compact), reward and flags with it
+        if constexpr (!FAST && (world_obs || REC)) {
+            // the observation as a compact record (include/zs_b200.h: zs_step_compact, zs_step_compact_agents), with the
+            // reward(s) and flags in its header
+            if (io.compact) {
                 compacted = true;
                 uint32_t* const rec = io.compact + (size_t)env * io.compact_words;
+                uint32_t* const stage = reinterpret_cast<uint32_t*>(zs_smem + e.b);  // (EnvS::act: see obs_world_compact)
                 int n_ent = 0;
-                const bool over = obs_world_compact<MPC, G, CV>(p, e, rec, io.compact_words - ZS_COMPACT_HEADER, n_ent);
-                {
-                    uint32_t* const stage = reinterpret_cast<uint32_t*>(zs_smem + e.b);  // (EnvS::act: see obs_world_compact)
+                bool over;
+                int hdr;
+                if constexpr (world_obs) {
+                    hdr = ZS_COMPACT_HEADER;
+                    over = obs_world_compact<MPC, G, CV>(p, e, rec, io.compact_words - hdr, n_ent);
                     if (lane == 0) { stage[0] = (uint32_t)n_ent | (done ? 1u << 16 : 0u) | (trunc ? 1u << 17 : 0u) | (over ? 1u << 18 : 0u); stage[1] = 0u; }
                     if (lane_sum ? lane == 0 : aidx == 0) { stage[2] = (uint32_t)__double2loint(rew); stage[3] = (uint32_t)__double2hiint(rew); }
-                    compact_flush<MPC, G, CV>(e, rec, ZS_COMPACT_HEADER + n_ent * (p.obs_enc == ZS_OBS_SIMPLE ? 1 : 2));
-                }
-                if (wany<G, CV>(e, over) && obs_out) {  // rare: the full row, for the caller to fetch
-                    obs_world_template<MPC, G, CV>(p, e, obs_out);
-                    obs_world_patch<MPC, G, CV>(p, e, obs_out);
-                }
-                if (io.host_flags) {
-                    // ONE system-scope fence per group of envs, by whoever completes the group (a fence per warp takes 8-34 us
-                    // when 4,096 warps fence at once): the others order their record words before the counter at gpu scope
-                    __threadfence();
-                    gsync<G, CV>(e);
-                    if (lane == 0) {
-                        const int grp = env / io.group_envs;
-                        const int size = min(io.group_envs, p.N - grp * io.group_envs);
-                        if (atomicAdd(io.group_count + grp, 1) == size - 1) {
-                            io.group_count[grp] = 0;
-                            __threadfence_system();
-                            *reinterpret_cast<volatile uint32_t*>(io.host_flags + 16 * grp) = io.ticket;
-                        }
+                } else {
+                    hdr = ZS_AGENT_COMPACT_HEADER(A);
+                    n_ent = obs_surroundings_compact<MPC, G, CV>(p, id_of(e), e.flags, rec, io.compact_words - hdr);
+                    over = n_ent < 0;
+                    if (over) n_ent = 0;
+                    if (lane == 0) { stage[0] = (uint32_t)n_ent | (done ? 1u << 16 : 0u) | (trunc ? 1u << 17 : 0u) | (over ? 1u << 18 : 0u); stage[1] = alive_before; }
+                    if (is_agent) {  // reward, window centre and life after the step (and after its auto-reset)
+                        stage[2 + 2 * aidx] = (uint32_t)__double2loint(rew); stage[3 + 2 * aidx] = (uint32_t)__double2hiint(rew);
+                        const uint32_t xy = TXY(lane);
+                        stage[2 + 2 * A + aidx] = (uint32_t)(xy_y(xy) * p.W + xy_x(xy)) | ((uint32_t)(uint16_t)TL(lane) << 16);
                     }
                 }
+                compact_flush<MPC, G, CV>(e, rec, hdr + n_ent * (p.obs_enc == ZS_OBS_SIMPLE ? 1 : 2));
+                if (wany<G, CV>(e, over) && obs_out) {  // rare: the full row, for the caller to fetch
+                    if constexpr (world_obs) {
+                        obs_world_template<MPC, G, CV>(p, e, obs_out);
+                        obs_world_patch<MPC, G, CV>(p, e, obs_out);
+                    } else encode_surroundings<MPC, G, CV>(p, e, obs_out);
+                }
+                if (io.host_flags) compact_signal<G, CV>(p, io, e, env);
             }
         }
         if constexpr (PROD) {
@@ -390,12 +412,15 @@ __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io,
 // SHAPE 3 = the standard rollout shape with a producer warp: CTAs of four game warps (eight envs) plus one warp that writes
 // the observations (160 threads; compiled for 4 CTAs per SM: 20 warps, five per scheduler = 96 registers, and 4,096 envs
 // are one wave.  Three-warp CTAs at seven per SM would put six warps on one scheduler: 80 registers and spills).
+// SHAPE 4 = surroundings observation with the per-agent compact record (zs_step_compact_agents / zs_step_host_agents; step
+// launches of at most 32 slots only): a kernel of its own, since with the record compiled into SHAPE 2 that kernel spilled more
+// and its device-output steps of config 3's game at 65,536 envs took 6 % longer (profiles/r04_ab_surroundings.txt).
 // ROS: the game roster compiled into a standard-rollout-shape kernel (zs_world.cuh: Roster), 0 = read from ZsParams.
 template <int MODE, int MPC, int G, int SHAPE, int OCC, int ROS = 0>
 __global__ void __launch_bounds__(SHAPE == 3 ? 160 : ZS_WPC * 32, OCC) zs_sim_kernel(const __grid_constant__ ZsParams p, const __grid_constant__ ZsIO io) {
     ZS_CONSTS;
     constexpr bool PROD = SHAPE == 3;
-    constexpr bool FAST = SHAPE == 1 || PROD, SURR = SHAPE == 2;
+    constexpr bool FAST = SHAPE == 1 || PROD, SURR = SHAPE == 2 || SHAPE == 4;
     // the step kernel keeps both envs of a warp converged (zs_device.cuh); masked resets and encodes may not
     constexpr bool CV = MODE == MODE_STEP;
     constexpr int EPW = 32 / G;  // envs per warp
@@ -501,7 +526,7 @@ __global__ void __launch_bounds__(SHAPE == 3 ? 160 : ZS_WPC * 32, OCC) zs_sim_ke
 #ifdef ZS_PHASE_CLOCKS
     e.ph_last = clock64();
 #endif
-    if constexpr (ONE) step_loop_one<MPC, G, CV, FAST, SURR, PROD, ROS>(p, io, e);
+    if constexpr (ONE) step_loop_one<MPC, G, CV, FAST, SURR, PROD, ROS, SHAPE == 4>(p, io, e);
     else step_loop_general<MPC, G, CV, SURR>(p, io, e);
 #ifdef ZS_PHASE_CLOCKS
     e.ph_last = clock64();
@@ -595,6 +620,7 @@ struct ZsHandle {
     int short_steps;       // launches of fewer steps than this take shape[1]
     int use_pdl;           // launch with programmatic stream serialization (launch_sim): 0 never, 1 always, 2 short step launches
     int compact_words;     // words per compact observation record, 0 = this configuration has no compact form
+    int agent_compact_words;  // the same for the per-agent surroundings record (zs_step_compact_agents)
     int32_t* host_actions_dev = nullptr;  // zs_step_host: this step's actions on the device
     uint32_t host_ticket = 0;  // zs_step_host: the value that marks the current step's records as arrived
     volatile uint32_t* host_flag = nullptr;  // pinned, one cache line each: [0] zs_host_flag_kernel's, [1 + g] group g's (the step kernel's)
@@ -605,6 +631,7 @@ struct ZsHandle {
     const void* host_records_checked = nullptr;
     double host_stats[5] = {0, 0, 0, 0, 0};  // zs_step_host: calls, and summed us from entry to: launched / previous cells restored / flag seen / return
     std::vector<int32_t> tmpl_obs_host;  // the pristine observation planes [obs_C][cells] (zs_expand_compact)
+    std::vector<int32_t> pad_host;       // surroundings scope: the padded pristine planes p.tmpl_pad as int32 (zs_expand_compact_agents)
     int tmpl_single_step;  // launches of fewer than four steps stage the observation template for the TMA as well
     int roster;            // the game as a roster (zs_world.cuh: Roster) when the standard rollout kernel has it compiled in, else 0
     bool img_valid;  // the parked images (ZsParams::img) match the canonical state of every env
@@ -721,7 +748,8 @@ static void launch_sim(const ZsHandle* h, const ZsIO& io, cudaStream_t st) {
     const bool surr = pp.obs_scope == ZS_OBS_SURROUNDINGS;
     // the standard rollout shape of a batch that one wave of producer-warp CTAs holds: observations through a third warp
     const bool prod = fast && MODE == MODE_STEP && sh.prod_smem_bytes > 0 && pp.tmpl_smem_off >= 0 && io.env_mask == nullptr;
-    // SH_: 0 world scope, 1 the standard rollout shape (step launches only), 2 surroundings (zs_sim_kernel: SHAPE)
+    // SH_: 0 world scope, 1 the standard rollout shape (step launches only), 2 surroundings, 4 surroundings with the per-agent
+    // record (step launches only) (zs_sim_kernel: SHAPE)
     // Programmatic dependent launch: the kernel's CTAs may be scheduled while the previous kernel of the stream is still
     // draining (they stage the observation template and then wait in griddepcontrol.wait for that kernel to have
     // completed, all its writes visible) — the launch latency and the ramp hide under the predecessor's tail.
@@ -735,10 +763,11 @@ static void launch_sim(const ZsHandle* h, const ZsIO& io, cudaStream_t st) {
     // rollouts lose 1-1.5 % — the early CTAs of the next launch sit on the SMs — so only short step launches ask for it)
     const bool pdl = h->use_pdl == 1 || (h->use_pdl == 2 && MODE == MODE_STEP && io.n_steps < h->short_steps);
     lc.attrs = la; lc.numAttrs = pdl ? 1 : 0;
-#define ZS_LAUNCH_R(MPC_, G_, SH_, O_, R_) cudaLaunchKernelEx(&lc, zs_sim_kernel<MODE, MPC_, G_, ((SH_) == 1 && MODE != MODE_STEP) ? 0 : (SH_), MODE == MODE_STEP ? (O_) : ZS_MIN_CTAS, MODE == MODE_STEP ? (R_) : 0>, pp, io)
+#define ZS_LAUNCH_R(MPC_, G_, SH_, O_, R_) cudaLaunchKernelEx(&lc, zs_sim_kernel<MODE, MPC_, G_, MODE == MODE_STEP ? (SH_) : (SH_) == 1 ? 0 : (SH_) == 4 ? 2 : (SH_), MODE == MODE_STEP ? (O_) : ZS_MIN_CTAS, MODE == MODE_STEP ? (R_) : 0>, pp, io)
 #define ZS_LAUNCH(MPC_, G_, SH_, O_) ZS_LAUNCH_R(MPC_, G_, SH_, O_, 0)
 #define ZS_LAUNCH_F(MPC_, G_, O_) do { if (roster) ZS_LAUNCH_R(MPC_, G_, 1, O_, (MPC_) == 16 ? ZS_ROSTER_BENCH : 0); else if (fast) ZS_LAUNCH(MPC_, G_, 1, O_); \
-                                       else if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); else ZS_LAUNCH(MPC_, G_, 0, O_); } while (0)
+                                       else if (surr && io.compact) ZS_LAUNCH(MPC_, G_, 4, O_); else if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); \
+                                       else ZS_LAUNCH(MPC_, G_, 0, O_); } while (0)
 #define ZS_LAUNCH_G(MPC_, G_, O_) do { if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); else ZS_LAUNCH(MPC_, G_, 0, O_); } while (0)
     if (prod) {
         pp.prod_off = sh.prod_off; pp.prod_cap = sh.prod_cap; pp.tmpl_smem_off = ZS_PROD_ENVS * sh.smem_per_env;
@@ -777,6 +806,7 @@ static cudaError_t set_smem_attr_step(int bytes) {
     if (e == cudaSuccess && MPC <= 32) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (MPC <= 32 ? 1 : 0), OCC>, attr, bytes);
     if (e == cudaSuccess && MPC == 16) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (MPC == 16 ? 1 : 0), OCC, (MPC == 16 ? ZS_ROSTER_BENCH : 0)>, attr, bytes);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, 2, OCC>, attr, bytes);
+    if (e == cudaSuccess && MPC <= 32) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (MPC <= 32 ? 4 : 2), OCC>, attr, bytes);
     return e;
 }
 template <int MPC, int G>
@@ -918,6 +948,7 @@ extern "C" __attribute__((visibility("default"))) int zs_create(const ZsConfig* 
         p.pad_w = pw; p.pad_plane = pw * ph;
         p.sw_magic = (uint32_t)((0x100000000ull + (unsigned)sw - 1) / (unsigned)sw);
         rc |= upload(h, pad, &p.tmpl_pad);
+        h->pad_host.assign(pad.begin(), pad.end());
         // one pristine window block per cell, as long as the table stays a small part of the L2
         p.win_ints = (simple ? 1 : 2) * sw * sw;
         p.win_pitch = round_up(p.win_ints, 32);
@@ -1040,6 +1071,9 @@ extern "C" __attribute__((visibility("default"))) int zs_create(const ZsConfig* 
     h->tmpl_single_step = getenv("ZS_NO_TMA_SINGLE") ? 0 : 1;
     h->compact_words = (p.mpc <= 32 && p.obs_scope == ZS_OBS_WORLD && !p.obs_per_agent)
                            ? (p.obs_enc == ZS_OBS_SIMPLE ? 96 : 192) : 0;  // header + 92 entries; the caller grows them
+    // (the entry count and the window centres are 16-bit fields: fewer than 65,536 cells is what zs_layout accepts)
+    h->agent_compact_words = (p.mpc <= 32 && p.obs_scope == ZS_OBS_SURROUNDINGS && p.obs_per_agent)
+                                 ? round_up(ZS_AGENT_COMPACT_HEADER(p.A) + (p.obs_enc == ZS_OBS_SIMPLE ? 1 : 2) * 92, 32) : 0;
     const int smem_per_env_base = p.smem_per_env;
     for (int si = 0; si < 2; ++si) {
         ZsHandle::Shape& sh = h->shape[si];
@@ -1364,6 +1398,25 @@ static inline bool expand_one(const ExpandCtx& cx, int e, const uint32_t* r, uin
     return expand_write(cx, e, r, pv);
 }
 
+// every env's record through expand(e, record, prev) on n_threads host threads; returns the number of envs whose record
+// overflowed, their indices in overflow_envs_host
+template <class Expand>
+static int expand_records(int N, int n_threads, int words, const uint32_t* compact_host, uint32_t* prev_host,
+                          int32_t* overflow_envs_host, const Expand& expand) {
+    n_threads = host_threads(n_threads, N);
+    int n_over = 0;
+#pragma omp parallel for num_threads(n_threads) schedule(static)
+    for (int e = 0; e < N; ++e) {
+        if (expand(e, compact_host + (size_t)e * words, prev_host + (size_t)e * words)) {
+            int at;
+#pragma omp atomic capture
+            at = n_over++;
+            overflow_envs_host[at] = e;
+        }
+    }
+    return n_over;
+}
+
 // HOST code: records -> the reference's observation tensor (include/zs_b200.h).  Incremental: the cells the previous
 // record of an env patched go back to the pristine value, the new record's cells are written; a full row is only
 // rewritten on the first call and after an overflow.
@@ -1377,20 +1430,10 @@ extern "C" __attribute__((visibility("default"))) int zs_expand_compact(const Zs
     if (compact_words < ZS_COMPACT_HEADER + 8) return fail("compact_words out of range");
     const int N = h->p.N, words = compact_words, cells = h->p.cells, C = h->p.obs_C;
     const bool simple = h->p.obs_enc == ZS_OBS_SIMPLE;
-    n_threads = host_threads(n_threads, N);
-    int n_over = 0;
     const ExpandCtx cx{h->tmpl_obs_host.data(), cells, C, simple ? 1 : 2, words, first_call != 0, obs_host, reward_host, terminated_host,
                        truncated_host};
-#pragma omp parallel for num_threads(n_threads) schedule(static)
-    for (int e = 0; e < N; ++e) {
-        if (expand_one(cx, e, compact_host + (size_t)e * words, prev_host + (size_t)e * words)) {
-            int at;
-#pragma omp atomic capture
-            at = n_over++;
-            overflow_envs_host[at] = e;
-        }
-    }
-    *n_overflow = n_over;
+    *n_overflow = expand_records(N, n_threads, words, compact_host, prev_host, overflow_envs_host,
+                                 [&](int e, const uint32_t* r, uint32_t* pv) { return expand_one(cx, e, r, pv); });
     return 0;
 }
 
@@ -1402,18 +1445,14 @@ extern "C" __attribute__((visibility("default"))) int zs_expand_compact(const Zs
 // that envs could be expanded as they arrive, costs 8-34 us per warp with 4,096 warps fencing at once; a flag per group
 // of envs does not arrive earlier than the last one either (a system-scope fence waits for the whole burst to drain), so
 // one group is the default (ZS_HOST_GROUPS).
-extern "C" __attribute__((visibility("default"))) int zs_step_host(ZsHandle* h, const int32_t* actions_host, int32_t action_format,
-                                                                    uint32_t* compact_pinned, uint32_t* prev_host, int32_t compact_words,
-                                                                    int32_t* obs_dev, int32_t* obs_host, double* reward_host,
-                                                                    uint8_t* terminated_host, uint8_t* truncated_host,
-                                                                    int32_t* overflow_envs_host, int32_t* n_overflow, int32_t first_call,
-                                                                    int32_t n_threads, void* stream) {
-    if (int rc = check_bound(h)) return rc;
-    DeviceGuard guard(h);
-    if (!h->compact_words) return fail("this configuration has no compact observation form (world scope, one reward per env, at most 32 slots)");
-    if (!actions_host || !compact_pinned || !prev_host || !obs_host || !overflow_envs_host || !n_overflow) return fail("null argument");
-    if (compact_words < ZS_COMPACT_HEADER + 8 || compact_words > 65535) return fail("compact_words out of range");
-    if (action_format != ZS_ACTIONS_FULL && action_format != ZS_ACTIONS_DISCRETE) return fail("bad action format");
+// The transport of zs_step_host and zs_step_host_agents: `ahead(e)` (when use_ahead) runs for every env while the device works
+// on the step, `expand(e, record, prev)` after the flag; it returns true when the env's record overflowed.  *us_total: the
+// microseconds from entry to return.
+template <class Ahead, class Expand>
+static int host_step_run(ZsHandle* h, const int32_t* actions_host, int32_t action_format, uint32_t* compact_pinned,
+                         uint32_t* prev_host, int32_t compact_words, int32_t* obs_dev, int32_t* overflow_envs_host,
+                         int32_t* n_overflow, int32_t n_threads, void* stream, bool use_ahead, const Ahead& ahead,
+                         const Expand& expand, double* us_total) {
     struct timespec ts0;
     clock_gettime(CLOCK_MONOTONIC, &ts0);
     auto us_since = [&ts0]() {
@@ -1448,7 +1487,6 @@ extern "C" __attribute__((visibility("default"))) int zs_step_host(ZsHandle* h, 
         h->host_groups = force ? atoi(force) : 1;
         if (h->host_groups > ZS_HOST_GROUPS_MAX) h->host_groups = ZS_HOST_GROUPS_MAX;
         if (h->host_groups > h->p.N) h->host_groups = h->p.N;
-        if (const char* v = getenv("ZS_HOST_DIFF")) h->host_diff = atoi(v) != 0;
     }
     CU(cudaMemcpyAsync(h->host_actions_dev, actions_host, act_bytes, cudaMemcpyHostToDevice, st));
     const int N = h->p.N, words = compact_words;
@@ -1468,34 +1506,7 @@ extern "C" __attribute__((visibility("default"))) int zs_step_host(ZsHandle* h, 
     const double us_launched = us_since();
     double us_flag = 0, us_restored = 0;
     n_threads = host_threads(n_threads, N);
-    const ExpandCtx cx{h->tmpl_obs_host.data(), h->p.cells, h->p.obs_C, h->p.obs_enc == ZS_OBS_SIMPLE ? 1 : 2, words, first_call != 0,
-                       obs_host, reward_host, terminated_host, truncated_host};
     int n_over = 0, gave_up = 0;
-    // restore ahead + write, or every env as the difference of its two records after the flag (expand_diff).
-    // Which of the two is faster depends on the host (its caches, how many ranks share it, the threads this rank got): the
-    // handle times both — 32 calls alternating between them, then the faster one for 512 calls, then the next sample.
-    // (Both leave the same rows and the same previous records, so the choice never shows in a result.)
-    bool diff = h->host_diff != 0;
-    if (h->host_diff < 0) {
-        // a sample is 32 calls that ALTERNATE between the two (the records grow over the first steps of a batch: sixteen calls of
-        // one and then sixteen of the other would compare different work); the medians decide (one hiccup of the host must not
-        // decide 512 calls)
-        ZsHandle::HostTune& t = h->host_tune;
-        if (t.left <= 0) {
-            if (t.exploring) {
-                double med[2];
-                for (int m = 0; m < 2; ++m) {
-                    const int n = t.n[m] < 16 ? t.n[m] : 16;
-                    std::sort(t.last[m], t.last[m] + n);
-                    med[m] = n ? t.last[m][n / 2] : 1e30;
-                }
-                t.mode = med[1] < med[0] ? 1 : 0; t.exploring = false; t.left = 512;
-            } else { t.exploring = true; t.left = 32; }
-            t.n[0] = t.n[1] = 0;
-        }
-        if (t.exploring) t.mode = t.left & 1;
-        diff = t.mode != 0;
-    }
     const volatile uint32_t* const flags = h->host_flag;
     const int n_flags = groups > 0 ? (N + group_envs - 1) / group_envs : 1;
 #pragma omp parallel num_threads(n_threads)
@@ -1506,11 +1517,11 @@ extern "C" __attribute__((visibility("default"))) int zs_step_host(ZsHandle* h, 
         const int nt = omp_get_num_threads(), tid = omp_get_thread_num();
         // while the device works on the step: what the previous records patched goes back to the pristine layer (half of an
         // expansion's stores need nothing from the new records)
-        if (!diff)
+        if (use_ahead)
         for (int g = 0; g < n_flags; ++g) {
             const int g0 = g * group_envs, gn = (g0 + group_envs < N ? g0 + group_envs : N) - g0;
             const int e0 = g0 + (int)((long long)gn * tid / nt), e1 = g0 + (int)((long long)gn * (tid + 1) / nt);
-            for (int e = e0; e < e1; ++e) expand_restore(cx, e, prev_host + (size_t)e * words);
+            for (int e = e0; e < e1; ++e) ahead(e);
         }
         if (tid == 0) us_restored = us_since();
         struct timespec t0;
@@ -1535,9 +1546,7 @@ extern "C" __attribute__((visibility("default"))) int zs_step_host(ZsHandle* h, 
             const int g0 = g * group_envs, gn = (g0 + group_envs < N ? g0 + group_envs : N) - g0;
             const int e0 = g0 + (int)((long long)gn * tid / nt), e1 = g0 + (int)((long long)gn * (tid + 1) / nt);
             for (int e = e0; e < e1; ++e) {
-                const uint32_t* const r = compact_pinned + (size_t)e * words;
-                uint32_t* const pv = prev_host + (size_t)e * words;
-                if (diff ? expand_diff(cx, e, r, pv) : expand_write(cx, e, r, pv)) {
+                if (expand(e, compact_pinned + (size_t)e * words, prev_host + (size_t)e * words)) {
                     int at;
 #pragma omp atomic capture
                     at = n_over++;
@@ -1553,13 +1562,201 @@ extern "C" __attribute__((visibility("default"))) int zs_step_host(ZsHandle* h, 
     }
     // rows of overflowing envs: obs_dev is complete when the launch is (the caller reads them next)
     if (n_over > 0) CU(cudaStreamSynchronize(st));
+    *us_total = us_since();
+    h->host_stats[0] += 1; h->host_stats[1] += us_launched; h->host_stats[2] += us_restored; h->host_stats[3] += us_flag; h->host_stats[4] += *us_total;
+    return 0;
+}
+
+extern "C" __attribute__((visibility("default"))) int zs_step_host(ZsHandle* h, const int32_t* actions_host, int32_t action_format,
+                                                                    uint32_t* compact_pinned, uint32_t* prev_host, int32_t compact_words,
+                                                                    int32_t* obs_dev, int32_t* obs_host, double* reward_host,
+                                                                    uint8_t* terminated_host, uint8_t* truncated_host,
+                                                                    int32_t* overflow_envs_host, int32_t* n_overflow, int32_t first_call,
+                                                                    int32_t n_threads, void* stream) {
+    if (int rc = check_bound(h)) return rc;
+    DeviceGuard guard(h);
+    if (!h->compact_words) return fail("this configuration has no compact observation form (world scope, one reward per env, at most 32 slots)");
+    if (!actions_host || !compact_pinned || !prev_host || !obs_host || !overflow_envs_host || !n_overflow) return fail("null argument");
+    if (compact_words < ZS_COMPACT_HEADER + 8 || compact_words > 65535) return fail("compact_words out of range");
+    if (action_format != ZS_ACTIONS_FULL && action_format != ZS_ACTIONS_DISCRETE) return fail("bad action format");
+    const ExpandCtx cx{h->tmpl_obs_host.data(), h->p.cells, h->p.obs_C, h->p.obs_enc == ZS_OBS_SIMPLE ? 1 : 2, compact_words, first_call != 0,
+                       obs_host, reward_host, terminated_host, truncated_host};
+    // restore ahead + write, or every env as the difference of its two records after the flag (expand_diff).
+    // Which of the two is faster depends on the host (its caches, how many ranks share it, the threads this rank got): the
+    // handle times both — 32 calls alternating between them, then the faster one for 512 calls, then the next sample.
+    // (Both leave the same rows and the same previous records, so the choice never shows in a result.)
+    if (!h->host_actions_dev) { if (const char* v = getenv("ZS_HOST_DIFF")) h->host_diff = atoi(v) != 0; }  // (read on the first call)
+    bool diff = h->host_diff != 0;
+    if (h->host_diff < 0) {
+        // a sample is 32 calls that ALTERNATE between the two (the records grow over the first steps of a batch: sixteen calls of
+        // one and then sixteen of the other would compare different work); the medians decide (one hiccup of the host must not
+        // decide 512 calls)
+        ZsHandle::HostTune& t = h->host_tune;
+        if (t.left <= 0) {
+            if (t.exploring) {
+                double med[2];
+                for (int m = 0; m < 2; ++m) {
+                    const int n = t.n[m] < 16 ? t.n[m] : 16;
+                    std::sort(t.last[m], t.last[m] + n);
+                    med[m] = n ? t.last[m][n / 2] : 1e30;
+                }
+                t.mode = med[1] < med[0] ? 1 : 0; t.exploring = false; t.left = 512;
+            } else { t.exploring = true; t.left = 32; }
+            t.n[0] = t.n[1] = 0;
+        }
+        if (t.exploring) t.mode = t.left & 1;
+        diff = t.mode != 0;
+    }
+    double us_total = 0;
+    const int rc = host_step_run(h, actions_host, action_format, compact_pinned, prev_host, compact_words, obs_dev, overflow_envs_host,
+                                 n_overflow, n_threads, stream, !diff, [&](int e) { expand_restore(cx, e, prev_host + (size_t)e * compact_words); },
+                                 [&](int e, const uint32_t* r, uint32_t* pv) { return diff ? expand_diff(cx, e, r, pv) : expand_write(cx, e, r, pv); },
+                                 &us_total);
+    if (rc) return rc;
     if (h->host_diff < 0) {
         ZsHandle::HostTune& t = h->host_tune;
-        if (t.exploring && !first_call && n_over == 0 && t.left <= 28) { t.last[t.mode][t.n[t.mode] & 15] = us_since(); t.n[t.mode] += 1; }  // (the first four settle the caches)
+        if (t.exploring && !first_call && *n_overflow == 0 && t.left <= 28) { t.last[t.mode][t.n[t.mode] & 15] = us_total; t.n[t.mode] += 1; }  // (the first four settle the caches)
         t.left -= 1;
     }
-    h->host_stats[0] += 1; h->host_stats[1] += us_launched; h->host_stats[2] += us_restored; h->host_stats[3] += us_flag; h->host_stats[4] += us_since();
     return 0;
+}
+
+// ---------------------------------------------------------------- per-agent surroundings records (include/zs_b200.h)
+extern "C" __attribute__((visibility("default"))) int32_t zs_agent_compact_words(const ZsHandle* h) { return h ? h->agent_compact_words : 0; }
+// the record size that no env can overflow by count: every thing, every box/wall, every listed dead body
+extern "C" __attribute__((visibility("default"))) int32_t zs_agent_compact_max_words(const ZsHandle* h) {
+    if (!h || !h->agent_compact_words) return 0;
+    const int wpe = h->p.obs_enc == ZS_OBS_SIMPLE ? 1 : 2;
+    const int entries = h->p.M + h->p.S + h->p.cells;
+    const int cap = h->p.M + h->p.S + 64;
+    return round_up(ZS_AGENT_COMPACT_HEADER(h->p.A) + wpe * (cap < entries ? cap : entries), 32);
+}
+static int check_agent_words(const ZsHandle* h, int32_t compact_words) {
+    if (!h->agent_compact_words)
+        return fail("this configuration has no per-agent compact observation form (surroundings scope, one observation per agent, "
+                    "at most 32 slots)");
+    if (compact_words < ZS_AGENT_COMPACT_HEADER(h->p.A) + 8 || compact_words > 65535) return fail("compact_words out of range");
+    return 0;
+}
+
+extern "C" __attribute__((visibility("default"))) int zs_step_compact_agents(ZsHandle* h, const int32_t* actions_dev, int32_t action_format,
+                                                                              uint32_t* compact_dev, int32_t compact_words, int32_t* obs_dev,
+                                                                              void* stream) {
+    if (int rc = check_bound(h)) return rc;
+    DeviceGuard guard(h);
+    if (int rc = check_agent_words(h, compact_words)) return rc;
+    if (!actions_dev || !compact_dev) return fail("zs_step_compact_agents needs an action tensor and a record buffer");
+    if (action_format != ZS_ACTIONS_FULL && action_format != ZS_ACTIONS_DISCRETE) return fail("bad action format");
+    ZsIO io;
+    memset(&io, 0, sizeof(io));
+    io.actions = actions_dev; io.fmt = action_format; io.obs = obs_dev; io.obs_slots = 1;
+    io.compact = compact_dev; io.compact_words = compact_words;
+    io.n_steps = 1;
+    launch_sim<MODE_STEP>(h, io, (cudaStream_t)stream);
+    return launched(h);
+}
+
+// HOST code: one env's agent record -> its A windows, rewards, flags, mask and lives.  Returns true on overflow (the caller
+// copies the env's rows from the device).
+struct AgentExpandCtx {
+    const int32_t* T;  // the padded pristine planes [Cp][ph][pw] (Cp = 1 simple, 2 channels: label, life; weapons are 0)
+    int pw, plane, W, w, half, C, Cp, A, hdr, wpe;
+    bool first_call;
+    int32_t* obs; double* reward; uint8_t* terminated; uint8_t* truncated; uint8_t* mask; int16_t* life;
+};
+static inline bool expand_agents(const AgentExpandCtx& cx, int e, const uint32_t* r, uint32_t* pv) {
+    const int A = cx.A, w = cx.w, ww = w * w, half = cx.half, W = cx.W, wpe = cx.wpe;
+    const uint32_t h0 = r[0];
+    const int n = (int)(h0 & 0xffffu);
+    if (cx.terminated) cx.terminated[e] = (uint8_t)((h0 >> 16) & 1u);
+    if (cx.truncated) cx.truncated[e] = (uint8_t)((h0 >> 17) & 1u);
+    for (int a = 0; a < A; ++a) {
+        if (cx.reward) memcpy(cx.reward + (size_t)e * A + a, r + 2 + 2 * a, sizeof(double));
+        if (cx.mask) cx.mask[(size_t)e * A + a] = (uint8_t)((r[1] >> a) & 1u);
+        if (cx.life) cx.life[(size_t)e * A + a] = (int16_t)(r[2 + 2 * A + a] >> 16);
+    }
+    if ((h0 >> 18) & 1u) { pv[0] = h0; return true; }  // the record could not hold this env: the caller copies its rows from the device
+    const bool prev_ok = !cx.first_call && !((pv[0] >> 18) & 1u);
+    const int pn = prev_ok ? (int)(pv[0] & 0xffffu) : 0;
+    int32_t* const o = cx.obs + (size_t)e * A * cx.C * ww;
+    auto pristine = [&](int32_t* oa, int idx, int x, int y) {  // cell (x, y) of the map at index idx of window oa
+        for (int pl = 0; pl < cx.Cp; ++pl) oa[pl * ww + idx] = cx.T[(size_t)pl * cx.plane + (size_t)(y + half) * cx.pw + x + half];
+        if (cx.C == 3) oa[2 * ww + idx] = 0;
+    };
+    for (int a = 0; a < A; ++a) {
+        const int c = (int)(r[2 + 2 * A + a] & 0xffffu), cy = c / W, cx0 = c - cy * W;
+        int32_t* const oa = o + (size_t)a * cx.C * ww;
+        if (!prev_ok || (pv[2 + 2 * A + a] & 0xffffu) != (uint32_t)c) {  // a new window: its rows from the padded planes
+            for (int pl = 0; pl < cx.Cp; ++pl)
+                for (int y = 0; y < w; ++y) memcpy(oa + pl * ww + y * w, cx.T + (size_t)pl * cx.plane + (size_t)(cy + y) * cx.pw + cx0, w * sizeof(int32_t));
+            if (cx.C == 3) memset(oa + 2 * ww, 0, ww * sizeof(int32_t));
+            continue;
+        }
+        // the same window: the cells the previous record patched in it go back to the pristine layer (the previous record
+        // holds every patched cell this window showed)
+        for (int i = 0; i < pn; ++i) {
+            const int cell = (int)(pv[cx.hdr + i * wpe] & 0xffffu), y = cell / W, x = cell - y * W;
+            const int wx = x - (cx0 - half), wy = y - (cy - half);
+            if ((unsigned)wx < (unsigned)w && (unsigned)wy < (unsigned)w) pristine(oa, wy * w + wx, x, y);
+        }
+    }
+    for (int i = 0; i < n; ++i) {
+        const uint32_t w0 = r[cx.hdr + i * wpe], w1 = wpe == 2 ? r[cx.hdr + 2 * i + 1] : 0u;
+        const int cell = (int)(w0 & 0xffffu), y = cell / W, x = cell - y * W;
+        for (int a = 0; a < A; ++a) {
+            const int c = (int)(r[2 + 2 * A + a] & 0xffffu), cy = c / W, cx0 = c - cy * W;
+            const int wx = x - (cx0 - half), wy = y - (cy - half);
+            if ((unsigned)wx >= (unsigned)w || (unsigned)wy >= (unsigned)w) continue;
+            int32_t* const oa = o + (size_t)a * cx.C * ww;
+            const int idx = wy * w + wx;
+            oa[idx] = (int32_t)(w0 >> 16);
+            if (wpe == 2) { oa[ww + idx] = (int32_t)(int16_t)(w1 & 0xffffu); oa[2 * ww + idx] = (int32_t)(w1 >> 16); }
+        }
+    }
+    memcpy(pv, r, (size_t)(cx.hdr + n * wpe) * sizeof(uint32_t));
+    return false;
+}
+static AgentExpandCtx agent_ctx(const ZsHandle* h, int32_t first_call, int32_t* obs_host, double* reward_host, uint8_t* terminated_host,
+                                uint8_t* truncated_host, uint8_t* agent_mask_host, int16_t* agent_life_host) {
+    const ZsParams& p = h->p;
+    const bool simple = p.obs_enc == ZS_OBS_SIMPLE;
+    return AgentExpandCtx{h->pad_host.data(), p.pad_w, p.pad_plane, p.W, p.sw, p.sw >> 1, p.obs_C, simple ? 1 : 2, p.A,
+                          ZS_AGENT_COMPACT_HEADER(p.A), simple ? 1 : 2, first_call != 0, obs_host, reward_host, terminated_host,
+                          truncated_host, agent_mask_host, agent_life_host};
+}
+
+extern "C" __attribute__((visibility("default"))) int zs_expand_compact_agents(const ZsHandle* h, const uint32_t* compact_host, uint32_t* prev_host,
+                                                                                int32_t* obs_host, double* reward_host, uint8_t* terminated_host,
+                                                                                uint8_t* truncated_host, uint8_t* agent_mask_host,
+                                                                                int16_t* agent_life_host, int32_t* overflow_envs_host,
+                                                                                int32_t* n_overflow, int32_t compact_words, int32_t first_call,
+                                                                                int32_t n_threads) {
+    if (!h) return fail("null handle");
+    if (int rc = check_agent_words(h, compact_words)) return rc;
+    if (!compact_host || !prev_host || !obs_host || !overflow_envs_host || !n_overflow) return fail("null argument");
+    const AgentExpandCtx cx = agent_ctx(h, first_call, obs_host, reward_host, terminated_host, truncated_host, agent_mask_host, agent_life_host);
+    *n_overflow = expand_records(h->p.N, n_threads, compact_words, compact_host, prev_host, overflow_envs_host,
+                                 [&](int e, const uint32_t* r, uint32_t* pv) { return expand_agents(cx, e, r, pv); });
+    return 0;
+}
+
+extern "C" __attribute__((visibility("default"))) int zs_step_host_agents(ZsHandle* h, const int32_t* actions_host, int32_t action_format,
+                                                                           uint32_t* compact_pinned, uint32_t* prev_host, int32_t compact_words,
+                                                                           int32_t* obs_dev, int32_t* obs_host, double* reward_host,
+                                                                           uint8_t* terminated_host, uint8_t* truncated_host,
+                                                                           uint8_t* agent_mask_host, int16_t* agent_life_host,
+                                                                           int32_t* overflow_envs_host, int32_t* n_overflow, int32_t first_call,
+                                                                           int32_t n_threads, void* stream) {
+    if (int rc = check_bound(h)) return rc;
+    DeviceGuard guard(h);
+    if (int rc = check_agent_words(h, compact_words)) return rc;
+    if (!actions_host || !compact_pinned || !prev_host || !obs_host || !overflow_envs_host || !n_overflow) return fail("null argument");
+    if (action_format != ZS_ACTIONS_FULL && action_format != ZS_ACTIONS_DISCRETE) return fail("bad action format");
+    const AgentExpandCtx cx = agent_ctx(h, first_call, obs_host, reward_host, terminated_host, truncated_host, agent_mask_host, agent_life_host);
+    double us_total = 0;
+    return host_step_run(h, actions_host, action_format, compact_pinned, prev_host, compact_words, obs_dev, overflow_envs_host, n_overflow,
+                         n_threads, stream, false, [](int) {}, [&](int e, const uint32_t* r, uint32_t* pv) { return expand_agents(cx, e, r, pv); },
+                         &us_total);
 }
 
 // diagnostics: out[5] = zs_step_host calls since the last read, and the mean microseconds from entry until the launches were

@@ -182,9 +182,23 @@ ZS_TPL __device__ __forceinline__ void compact_flush(Env& e, uint32_t* __restric
     gsync<G, CV>(e);
     for (int i = e.gl; i < n; i += G) rec[i] = stage[i];
 }
-ZS_TPL __device__ __forceinline__ bool obs_world_compact(const ZsParams& p, Env& e, uint32_t* __restrict__ rec, int cap_words, int& n_out) {
+// WIN: keep only the items whose cell lies in at least one agent's surroundings window (obs_surroundings_compact);
+// hdr: the record's header words, in front of the entries.
+template <int MPC, int G, bool CV, bool WIN>
+__device__ __forceinline__ bool obs_compact_entries(const ZsParams& p, Env& e, uint32_t* __restrict__ rec, int hdr, int cap_words, int& n_out) {
     ZS_CONSTS; ZS_VIEWS;
     const int lane = e.gl;
+    // the window test of encode_surroundings (into_windows), windows centred on every agent slot's (possibly stale) position
+    auto seen = [&](int cell) {
+        if (!WIN) return true;
+        const int half = p.sw >> 1, y = cell / p.W, x = cell - y * p.W;
+#pragma unroll 1
+        for (int a = 0; a < p.A; ++a) {
+            const uint32_t axy = TXY(p.P + a);
+            if ((unsigned)(x - (xy_x(axy) - half)) < (unsigned)p.sw && (unsigned)(y - (xy_y(axy) - half)) < (unsigned)p.sw) return true;
+        }
+        return false;
+    };
     const unsigned below_l = (1u << lane) - 1u;
     const bool simple = p.obs_enc == ZS_OBS_SIMPLE;
     const int cap = simple ? cap_words : (cap_words >> 1);
@@ -193,17 +207,18 @@ ZS_TPL __device__ __forceinline__ bool obs_world_compact(const ZsParams& p, Env&
     uint32_t* const stage = reinterpret_cast<uint32_t*>(&S.act[0]);
     auto put = [&](int w, uint32_t v) { if (w < compact_stage_words<MPC>()) stage[w] = v; else rec[w] = v; };
     auto emit = [&](bool on, int cell, int v0, int v1, int v2) {
+        if (WIN) on = on && seen(cell);
         const unsigned m = gballot<G, CV>(e, on);
         const int pos = n + __popc(m & below_l);
         if (on) {
             if (simple) {
                 bad |= (unsigned)v0 > 0xffffu;
-                if (pos < cap) put(ZS_COMPACT_HEADER + pos, (uint32_t)cell | ((uint32_t)v0 << 16));
+                if (pos < cap) put(hdr + pos, (uint32_t)cell | ((uint32_t)v0 << 16));
             } else {
                 bad |= (unsigned)v0 > 0xffffu || (unsigned)v2 > 0xffffu || v1 < -32768 || v1 > 32767;
                 if (pos < cap) {
-                    put(ZS_COMPACT_HEADER + 2 * pos, (uint32_t)cell | ((uint32_t)v0 << 16));
-                    put(ZS_COMPACT_HEADER + 2 * pos + 1, ((uint32_t)v1 & 0xffffu) | ((uint32_t)v2 << 16));
+                    put(hdr + 2 * pos, (uint32_t)cell | ((uint32_t)v0 << 16));
+                    put(hdr + 2 * pos + 1, ((uint32_t)v1 & 0xffffu) | ((uint32_t)v2 << 16));
                 }
             }
         }
@@ -261,6 +276,19 @@ ZS_TPL __device__ __forceinline__ bool obs_world_compact(const ZsParams& p, Env&
     const bool over = gany<G, CV>(e, bad) || n > cap;
     n_out = over ? 0 : n;
     return over;
+}
+ZS_TPL __device__ __forceinline__ bool obs_world_compact(const ZsParams& p, Env& e, uint32_t* __restrict__ rec, int cap_words, int& n_out) {
+    return obs_compact_entries<MPC, G, CV, false>(p, e, rec, ZS_COMPACT_HEADER, cap_words, n_out);
+}
+// Surroundings scope, one window per agent, as a compact record (include/zs_b200.h: zs_step_compact_agents): the items pass 2
+// of encode_surroundings patches, in the world record's entry encoding, behind a header of ZS_AGENT_COMPACT_HEADER(A) words
+// (the caller stages it).  An item no window shows is left out: that keeps the records of large maps small.  Returns the entry
+// count, -1 on overflow.  (Out of line: inlined into the step loop it made the surroundings kernels spill more.)
+ZS_TPL __device__ __noinline__ int obs_surroundings_compact(const ZsParams& p, GrpId id, int flags, uint32_t* __restrict__ rec, int cap_words) {
+    Env e = env_of(p, id);
+    e.flags = flags;
+    int n = 0;
+    return obs_compact_entries<MPC, G, CV, true>(p, e, rec, ZS_AGENT_COMPACT_HEADER(p.A), cap_words, n) ? -1 : n;
 }
 
 // World scope as a record for the producer warp (zs_device.cuh: ObsMail): the cells pass 2 would patch as two-word entries

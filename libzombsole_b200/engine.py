@@ -203,34 +203,51 @@ class ZsEngine(object):
                                        1 if first_call else 0, int(n_threads)))
         return overflow_host[:n_over.value]
 
-    def host_stepper(self, records, prev_host, obs_dev, obs_host, reward_host, term_host, trunc_host, overflow_host, n_threads=0):
+    def host_stepper(self, records, prev_host, obs_dev, obs_host, reward_host, term_host, trunc_host, overflow_host, n_threads=0,
+                     agent_mask_host=None, agent_life_host=None):
         """zs_step_host bound to one set of buffers: ``step(actions, fmt, first_call)`` runs one transition whose actions
         come from host memory and whose records are written to pinned host memory by the kernel itself, the host
-        threads expanding each env as its record arrives.  Returns the envs whose rows must be fetched from ``obs_dev``, or None."""
+        threads expanding each env as its record arrives.  Returns the envs whose rows must be fetched from ``obs_dev``, or None.
+        With ``agent_mask_host`` (uint8 [N, A]) and ``agent_life_host`` (int16 [N, A]) it is zs_step_host_agents: per-agent
+        surroundings records, rewards [N, A]."""
         words = int(records.shape[-1])
         for name, t in (("records", records),):
             if not (t.device.type == "cpu" and t.is_pinned()):
                 raise ValueError("%s must be pinned host memory" % name)
-        N = self.N
+        N, agents = self.N, agent_mask_host is not None or agent_life_host is not None
         ptrs = (self._arg(records, torch.int32, N * words, "records"), self._host_arg(prev_host, torch.int32, N * words, "prev"), words,
                 self._arg(obs_dev, torch.int32, N * self.obs_elems, "obs_dev"),
                 self._host_arg(obs_host, torch.int32, N * self.obs_elems, "obs_host"),
-                self._host_arg(reward_host, torch.float64, N, "reward"), self._host_arg(term_host, self._FLAG_DTYPES, N, "terminated"),
+                self._host_arg(reward_host, torch.float64, N * self.R, "reward"), self._host_arg(term_host, self._FLAG_DTYPES, N, "terminated"),
                 self._host_arg(trunc_host, self._FLAG_DTYPES, N, "truncated"), self._host_arg(overflow_host, torch.int32, N, "overflow"))
         n_over = C.c_int32(0)
         n_over_p = C.addressof(n_over)
         call, h, A, nthr = self.L.zs_step_host, self.h, self.A, int(n_threads)
-        keep = (records, prev_host, obs_dev, obs_host, reward_host, term_host, trunc_host, overflow_host, n_over)
+        keep = (records, prev_host, obs_dev, obs_host, reward_host, term_host, trunc_host, overflow_host, n_over,
+                agent_mask_host, agent_life_host)
 
         stream_of = self._stream
 
-        def raw(actions_ptr, fmt, first_call):
-            """(no checks: ``actions_ptr`` addresses N * A (* 3) int32 in host memory)"""
-            rc = call(h, actions_ptr, fmt, ptrs[0], ptrs[1], ptrs[2], ptrs[3], ptrs[4], ptrs[5], ptrs[6], ptrs[7], ptrs[8],
-                      n_over_p, 1 if first_call else 0, nthr, stream_of())
-            if rc:
-                check(rc)
-            return overflow_host[:n_over.value] if n_over.value else None
+        if agents:
+            call = self.L.zs_step_host_agents
+            mask_p = self._host_arg(agent_mask_host, self._FLAG_DTYPES, N * A, "agent_mask")
+            life_p = self._host_arg(agent_life_host, torch.int16, N * A, "agent_life")
+
+            def raw(actions_ptr, fmt, first_call):
+                """(no checks: ``actions_ptr`` addresses N * A (* 3) int32 in host memory)"""
+                rc = call(h, actions_ptr, fmt, ptrs[0], ptrs[1], ptrs[2], ptrs[3], ptrs[4], ptrs[5], ptrs[6], ptrs[7], mask_p, life_p,
+                          ptrs[8], n_over_p, 1 if first_call else 0, nthr, stream_of())
+                if rc:
+                    check(rc)
+                return overflow_host[:n_over.value] if n_over.value else None
+        else:
+            def raw(actions_ptr, fmt, first_call):
+                """(no checks: ``actions_ptr`` addresses N * A (* 3) int32 in host memory)"""
+                rc = call(h, actions_ptr, fmt, ptrs[0], ptrs[1], ptrs[2], ptrs[3], ptrs[4], ptrs[5], ptrs[6], ptrs[7], ptrs[8],
+                          n_over_p, 1 if first_call else 0, nthr, stream_of())
+                if rc:
+                    check(rc)
+                return overflow_host[:n_over.value] if n_over.value else None
 
         def step(actions, fmt, first_call):
             per = 3 if fmt == abi.ACTIONS_FULL else 1
@@ -241,6 +258,39 @@ class ZsEngine(object):
         step.raw = raw
         step.keep = keep
         return step
+
+    # ---- compact host outputs for per-agent surroundings observations (include/zs_b200.h: zs_step_compact_agents)
+    def agent_compact_words(self):
+        """Words per per-agent compact record, 0 if this configuration has no such form."""
+        return int(self.L.zs_agent_compact_words(self.h))
+
+    def agent_compact_max_words(self):
+        return int(self.L.zs_agent_compact_max_words(self.h))
+
+    def step_compact_agents(self, actions, fmt, records, obs=None):
+        """One transition whose per-agent windows, rewards, agent mask, lives and flags come out as one small record per env
+        (device tensor ``records`` int32 [N, words]); ``obs`` receives the full rows of the rare env a record cannot hold."""
+        words = int(records.shape[-1])
+        check(self.L.zs_step_compact_agents(self.h, self._action_arg(actions, fmt, 1), fmt,
+                                            self._arg(records, torch.int32, self.N * words, "records"), words,
+                                            self._arg(obs, torch.int32, self.N * self.obs_elems, "obs"), self._stream()))
+
+    def expand_compact_agents(self, records_host, prev_host, obs_host, reward_host, term_host, trunc_host, mask_host, life_host,
+                              overflow_host, first_call, n_threads=0):
+        """HOST side: per-agent records (already in host memory) -> observation [N, A, C, w, w], reward [N, A], flags, agent
+        mask [N, A] and lives [N, A].  Returns the indices of the envs whose rows must be fetched from the device."""
+        N, A, words = self.N, self.A, int(records_host.shape[-1])
+        n_over = C.c_int32(0)
+        check(self.L.zs_expand_compact_agents(
+            self.h, self._host_arg(records_host, torch.int32, N * words, "records"),
+            self._host_arg(prev_host, torch.int32, N * words, "prev"),
+            self._host_arg(obs_host, torch.int32, N * self.obs_elems, "obs_host"),
+            self._host_arg(reward_host, torch.float64, N * self.R, "reward"),
+            self._host_arg(term_host, self._FLAG_DTYPES, N, "terminated"), self._host_arg(trunc_host, self._FLAG_DTYPES, N, "truncated"),
+            self._host_arg(mask_host, self._FLAG_DTYPES, N * A, "agent_mask"), self._host_arg(life_host, torch.int16, N * A, "agent_life"),
+            self._host_arg(overflow_host, torch.int32, N, "overflow"), C.addressof(n_over), words, 1 if first_call else 0,
+            int(n_threads)))
+        return overflow_host[:n_over.value]
 
     def step_host_stats(self):
         """(calls, mean us from entry to: launches issued, previous cells restored, flag seen = records in host memory,

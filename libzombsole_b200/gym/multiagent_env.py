@@ -15,12 +15,12 @@ import torch
 
 from .. import abi
 from ..engine import ZsEngine
-from ..gym_env import encode_action
+from ..gym_env import CompactHostOutputs, encode_action
 from ..spaces import Box, Dict, Discrete, Text
 from ..things import Game
 
 
-class MultiagentZombsoleVectorEnv(object):
+class MultiagentZombsoleVectorEnv(CompactHostOutputs):
     metadata = {"render.modes": ["human"]}
     reward_range = (-float("inf"), float("inf"))
     game_actions = [
@@ -36,7 +36,7 @@ class MultiagentZombsoleVectorEnv(object):
     def __init__(self, rules_name, player_names, map_name, agent_ids, initial_zombies=0, minimum_zombies=0,
                  render_mode=None, observation_surroundings_width=21, observation_position_encoding_style="channels",
                  agent_weapons="rifle", debug=False, *, num_envs=1, device="cuda", seed=0, env_index_base=0,
-                 max_episode_steps=None, auto_reset=True, host_outputs=False):
+                 max_episode_steps=None, auto_reset=True, host_outputs=False, host_threads=0, compact_words=0):
         if render_mode is not None:
             if render_mode not in self.metadata["render.modes"]:
                 raise ValueError("render_mode={} is not supported".format(render_mode))
@@ -71,12 +71,32 @@ class MultiagentZombsoleVectorEnv(object):
         # host_outputs: the kernel writes observations, rewards, flags and the agent mask straight into pinned host memory and
         # reads the actions from there; step() synchronises the stream once and also leaves the agents' lives after the step
         # in `agent_life_host` (what a host loop needs to know who is still playing, multiagent_env.py:169)
+        # host_outputs="compact": the same host tensors, but what crosses PCIe every step is one small record per env (the
+        # agents' window centres and lives, the rewards, the mask, the flags and the cells any window shows that differ from
+        # the map's pristine layer) which the library's host threads expand into the windows (zs_step_host_agents);
+        # "compact-copy" is the same with explicit copies and a stream synchronisation between the stages
+        # (zs_step_compact_agents / zs_expand_compact_agents, include/zs_b200.h)
+        if isinstance(host_outputs, str) and host_outputs not in ("compact", "compact-copy"):
+            raise ValueError("host_outputs must be False, True, 'compact' or 'compact-copy'")
+        self.compact = host_outputs in ("compact", "compact-copy")
+        self.streamed = host_outputs == "compact"
         self.host_outputs = bool(host_outputs)
+        self.host_threads = int(host_threads)
+        if self.compact and not self.engine.agent_compact_words():
+            raise ValueError("host_outputs=%r needs at most 32 things per env (one lane per thing in the step kernel); this game "
+                             "has %d (bots + agents + zombies)" % (host_outputs, self.engine.M))
         if self.host_outputs:
             self.obs, self.reward, self._term, self._trunc = self.engine.new_host_outputs()
             self._mask = torch.ones((num_envs, self.num_agents), dtype=torch.uint8).pin_memory()
             self._actions = torch.zeros((num_envs, self.num_agents, 3), dtype=torch.int32).pin_memory()
             self.agent_life_host = torch.zeros((num_envs, self.num_agents), dtype=torch.int16).pin_memory()
+            if self.compact:
+                self._dev_obs = self.engine.new_obs()  # full rows of the rare envs a record cannot hold
+                self._overflow = torch.zeros(num_envs, dtype=torch.int32)
+                self.compact_overflows = 0
+                self._act_pin = torch.zeros((num_envs, self.num_agents), dtype=torch.int32).pin_memory()
+                self._actions_pin = self._actions
+                self._size_records(int(compact_words) if compact_words else self.engine.agent_compact_words())
         else:
             self.obs = self.engine.new_obs()
             self.reward, self._term, self._trunc = self.engine.new_outputs()
@@ -92,18 +112,24 @@ class MultiagentZombsoleVectorEnv(object):
         self.engine.encode_obs(self.obs)
         if self.host_outputs:
             torch.cuda.current_stream(self.device).synchronize()
+        if self.compact:
+            self._compact_first = True  # the rows are complete again: the next step's records start from scratch
         return self.obs
+
+    def _action_rows(self, actions):
+        """One dict per env, keyed by agent id -> (type, dx, dy) rows [N, A, 3]; a missing key is ZS_ACT_ABSENT (heal self,
+        multiagent_env.py:129-131)."""
+        rows = np.zeros((self.num_envs, self.num_agents, 3), np.int32)
+        for n, d in enumerate(actions):
+            for i, aid in enumerate(self.possible_agents):
+                rows[n, i] = encode_action(dict(d[aid], parameter=d[aid].get("parameter", [0, 0]))) \
+                    if aid in d else (abi.ACT_ABSENT, 0, 0)
+        return rows
 
     def _stage_actions(self, actions):
         N, A = self.num_envs, self.num_agents
         if isinstance(actions, (list, tuple)) and len(actions) and isinstance(actions[0], dict):
-            # one dict per env, keyed by agent id; a missing key is ZS_ACT_ABSENT (heal self, multiagent_env.py:129-131)
-            rows = np.zeros((N, A, 3), np.int32)
-            for n, d in enumerate(actions):
-                for i, aid in enumerate(self.possible_agents):
-                    rows[n, i] = encode_action(dict(d[aid], parameter=d[aid].get("parameter", [0, 0]))) \
-                        if aid in d else (abi.ACT_ABSENT, 0, 0)
-            self._actions.copy_(torch.from_numpy(rows), non_blocking=not self.host_outputs)
+            self._actions.copy_(torch.from_numpy(self._action_rows(actions)), non_blocking=not self.host_outputs)
             return self._actions, abi.ACTIONS_FULL
         t = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.asarray(actions))
         if self.host_outputs and t.dtype == torch.int32 and t.device.type == "cpu" and t.is_pinned():
@@ -124,7 +150,11 @@ class MultiagentZombsoleVectorEnv(object):
 
     def step(self, actions):
         """One transition of every world (multiagent_env.py:111-171); discrete id -1 = key missing."""
+        if self.streamed:
+            return self._step_streamed(actions)
         a, fmt = self._stage_actions(actions)
+        if self.compact:
+            return self._step_compact(a, fmt)
         self.engine.step(a, fmt, self.obs, self.reward, self._term, self._trunc, self._mask)
         if self.host_outputs:  # the host owns the results (and any pinned action buffer) when step() returns
             P = self.cfg.n_bots
@@ -137,7 +167,33 @@ class MultiagentZombsoleVectorEnv(object):
         return (self.obs, self.reward, self._term.view(torch.bool), self._trunc.view(torch.bool),
                 {"agent_mask": self._mask.view(torch.bool)})  # (0/1 bytes: views, no kernels)
 
+    # (CompactHostOutputs)
+    def _max_words(self):
+        return self.engine.agent_compact_max_words()
+
+    def _host_stepper(self):
+        return self.engine.host_stepper(self._records_host, self._records_prev, self._dev_obs, self.obs, self.reward, self._term,
+                                        self._trunc, self._overflow, self.host_threads, self._mask, self.agent_life_host)
+
+    def _info(self):
+        return {"agent_mask": self._mask.view(torch.bool)}
+
+    def _step_compact(self, a, fmt):
+        eng = self.engine
+        eng.step_compact_agents(a, fmt, self._records, self._dev_obs)
+        self._records_host.copy_(self._records, non_blocking=True)
+        torch.cuda.current_stream(self.device).synchronize()
+        self._h2d_pending = False
+        over = eng.expand_compact_agents(self._records_host, self._records_prev, self.obs, self.reward, self._term, self._trunc,
+                                         self._mask, self.agent_life_host, self._overflow, self._compact_first, self.host_threads)
+        self._compact_first = False
+        if len(over):
+            self._fetch_overflow_rows(over)
+        return (self.obs, self.reward, self._term.view(torch.bool), self._trunc.view(torch.bool), self._info())
+
     def reset(self, seed=None, options=None, mask=None):
+        if self.compact:
+            return self._compact_reset(mask)
         self.engine.reset(mask, self.obs)
         if self.host_outputs:
             torch.cuda.current_stream(self.device).synchronize()

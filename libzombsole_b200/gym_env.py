@@ -48,7 +48,88 @@ def encode_action(action):
     return code, dx, dy
 
 
-class ZombsoleVectorEnv(object):
+class CompactHostOutputs(object):
+    """What host_outputs="compact" / "compact-copy" share between the vector envs: the record buffers, the streamed step's
+    action staging, the full rows of envs a record cannot hold and the resets.  A subclass sets ``obs`` / ``reward`` /
+    ``_term`` / ``_trunc`` (host), ``_dev_obs``, ``_overflow``, ``_act_pin`` (discrete ids) / ``_actions_pin`` ((type, dx, dy)
+    rows) and provides ``_max_words()``, ``_host_stepper()``, ``_action_rows(dicts)`` and ``_info()``."""
+
+    def _size_records(self, words):
+        """(Re)allocate the record buffers: ``words`` 32-bit words per env (header + entries)."""
+        words = min(int(words), self._max_words())
+        self.compact_words = words
+        self._records_host = torch.zeros((self.num_envs, words), dtype=torch.int32).pin_memory()
+        self._records_prev = torch.zeros((self.num_envs, words), dtype=torch.int32)
+        self._compact_first = True
+        self._overflows_since_resize = 0
+        if self.streamed:
+            torch.cuda.current_stream(self.device).synchronize()  # (nothing in flight still writes the old records)
+            self._host_step = self._host_stepper()
+            self._host_step_raw = self._host_step.raw
+            # (what step() returns never changes: the env's own buffers, the flag bytes as bool views)
+            self._step_result = (self.obs, self.reward, self._term.view(torch.bool), self._trunc.view(torch.bool))
+        else:
+            self._records = torch.zeros((self.num_envs, words), dtype=torch.int32, device=self.device)
+
+    def _step_streamed(self, actions):
+        """host_outputs="compact": the actions go over from host memory as they are, the kernel writes the pinned records in
+        place (zs_step_host)."""
+        n = self._act_pin.numel()  # discrete ids per step
+        if isinstance(actions, torch.Tensor) and actions.dtype == torch.int32 and actions.device.type == "cpu" \
+                and actions.is_contiguous() and actions.numel() in (n, 3 * n):
+            a = actions  # the caller's own buffer, in place: it is free again when step() returns
+        elif isinstance(actions, (list, tuple)) and len(actions) and isinstance(actions[0], dict):
+            a = self._actions_pin
+            a.copy_(torch.from_numpy(self._action_rows(actions)))
+        else:
+            t = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.asarray(actions))
+            if t.numel() == n:
+                a = self._act_pin
+            elif t.numel() == 3 * n:
+                a = self._actions_pin
+            else:
+                raise ValueError("actions must hold %d discrete ids or %d (type, dx, dy) rows" % (n, n))
+            a.copy_(t.reshape(a.shape))  # (any dtype / device: converted into the env's pinned buffer)
+        over = self._host_step_raw(a.data_ptr(), abi.ACTIONS_DISCRETE if a.numel() == n else abi.ACTIONS_FULL, self._compact_first)
+        self._compact_first = False
+        if over is not None:
+            self._fetch_overflow_rows(over)
+        return self._step_result + (self._info(),)
+
+    def _fetch_overflow_rows(self, over):
+        """Rare: more differing cells than a record holds — those rows come over as they are."""
+        stream = torch.cuda.current_stream(self.device)
+        stream.synchronize()
+        self.compact_overflows += len(over)
+        if len(over) > 16:  # many: one gather on the device, one copy
+            idx = over.to(self.device, dtype=torch.long)
+            self.obs[over.long()] = self._dev_obs[idx].cpu()
+        else:
+            for e in over.tolist():
+                self.obs[e].copy_(self._dev_obs[e], non_blocking=True)
+            stream.synchronize()
+        # box/wall damage persists across episodes, so the differing cells of long-running envs creep up: when more
+        # than one env in 64 no longer fits, or full rows keep being fetched, the records double (up to the size nothing
+        # can overflow)
+        self._overflows_since_resize += len(over)
+        if ((len(over) * 64 > self.num_envs or self._overflows_since_resize > 64)
+                and self.compact_words < self._max_words()):
+            self._size_records(2 * self.compact_words)
+
+    def _compact_reset(self, mask):
+        """(resets are rare next to steps: the full rows come over, and the next step starts afresh)"""
+        self.engine.reset(mask, self._dev_obs)
+        if mask is None:
+            self.obs.copy_(self._dev_obs, non_blocking=True)
+        else:
+            sel = torch.as_tensor(mask).to(torch.bool).cpu()
+            self.obs[sel] = self._dev_obs.cpu()[sel]
+        torch.cuda.current_stream(self.device).synchronize()
+        self._compact_first = True
+        return self.obs, {}
+
+
+class ZombsoleVectorEnv(CompactHostOutputs):
     """``num_envs`` independent ZombsoleGymEnv worlds on one GPU (constructor: gym_env.py:49-53)."""
 
     metadata = {"render.modes": ["human"]}
@@ -183,68 +264,19 @@ class ZombsoleVectorEnv(object):
             torch.cuda.current_stream(self.device).synchronize()  # the host owns the results when step() returns
         return self.obs, self.reward, self._term.view(torch.bool), self._trunc.view(torch.bool), {}  # (0/1 bytes: a view, no kernel)
 
-    def _size_records(self, words):
-        """(Re)allocate the record buffers: ``words`` 32-bit words per env (header + entries)."""
-        words = min(int(words), self.engine.compact_max_words())
-        self.compact_words = words
-        self._records_host = torch.zeros((self.num_envs, words), dtype=torch.int32).pin_memory()
-        self._records_prev = torch.zeros((self.num_envs, words), dtype=torch.int32)
-        self._compact_first = True
-        self._overflows_since_resize = 0
-        if self.streamed:
-            torch.cuda.current_stream(self.device).synchronize()  # (nothing in flight still writes the old records)
-            self._host_step = self.engine.host_stepper(self._records_host, self._records_prev, self._dev_obs, self.obs, self.reward,
-                                                       self._term, self._trunc, self._overflow, self.host_threads)
-            self._host_step_raw = self._host_step.raw
-            # (what step() returns never changes: the env's own buffers, the flag bytes as bool views)
-            self._step_result = (self.obs, self.reward, self._term.view(torch.bool), self._trunc.view(torch.bool))
-        else:
-            self._records = torch.zeros((self.num_envs, words), dtype=torch.int32, device=self.device)
+    # (CompactHostOutputs)
+    def _max_words(self):
+        return self.engine.compact_max_words()
 
-    def _step_streamed(self, actions):
-        """host_outputs="compact": the actions go over from host memory as they are, the kernel writes the pinned records in
-        place (zs_step_host)."""
-        N = self.num_envs
-        if isinstance(actions, torch.Tensor) and actions.dtype == torch.int32 and actions.device.type == "cpu" \
-                and actions.is_contiguous() and actions.numel() in (N, 3 * N):
-            a = actions  # the caller's own buffer, in place: it is free again when step() returns
-        elif isinstance(actions, (list, tuple)) and len(actions) and isinstance(actions[0], dict):
-            a = self._actions_pin
-            a.copy_(torch.from_numpy(np.array([encode_action(x) for x in actions], dtype=np.int32).reshape(N, 1, 3)))
-        else:
-            t = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.asarray(actions))
-            if t.numel() == N:
-                a = self._act_pin
-            elif t.numel() == 3 * N:
-                a = self._actions_pin
-            else:
-                raise ValueError("actions must hold %d discrete ids or %d (type, dx, dy) rows" % (N, N))
-            a.copy_(t.reshape(a.shape))  # (any dtype / device: converted into the env's pinned buffer)
-        over = self._host_step_raw(a.data_ptr(), abi.ACTIONS_DISCRETE if a.numel() == N else abi.ACTIONS_FULL, self._compact_first)
-        self._compact_first = False
-        if over is not None:
-            self._fetch_overflow_rows(over)
-        return self._step_result + ({},)
+    def _host_stepper(self):
+        return self.engine.host_stepper(self._records_host, self._records_prev, self._dev_obs, self.obs, self.reward, self._term,
+                                        self._trunc, self._overflow, self.host_threads)
 
-    def _fetch_overflow_rows(self, over):
-        """Rare: more differing cells than a record holds — those rows come over as they are."""
-        stream = torch.cuda.current_stream(self.device)
-        stream.synchronize()
-        self.compact_overflows += len(over)
-        if len(over) > 16:  # many: one gather on the device, one copy
-            idx = over.to(self.device, dtype=torch.long)
-            self.obs[over.long()] = self._dev_obs[idx].cpu()
-        else:
-            for e in over.tolist():
-                self.obs[e].copy_(self._dev_obs[e], non_blocking=True)
-            stream.synchronize()
-        # box/wall damage persists across episodes, so the differing cells of long-running envs creep up: when more
-        # than one env in 64 no longer fits, or full rows keep being fetched, the records double (up to the size nothing
-        # can overflow)
-        self._overflows_since_resize += len(over)
-        if ((len(over) * 64 > self.num_envs or self._overflows_since_resize > 64)
-                and self.compact_words < self.engine.compact_max_words()):
-            self._size_records(2 * self.compact_words)
+    def _action_rows(self, actions):
+        return np.array([encode_action(x) for x in actions], dtype=np.int32).reshape(self.num_envs, 1, 3)
+
+    def _info(self):
+        return {}
 
     def _step_compact(self, a, fmt):
         eng = self.engine
@@ -264,16 +296,8 @@ class ZombsoleVectorEnv(object):
         """Re-initialise every world (or those selected by ``mask``); gym_env.py:148-164.  ``seed`` is
         accepted for API compatibility and ignored, as in the reference (it only seeds gymnasium's unused
         np_random): the draw stream is fixed by the constructor's ``seed``."""
-        if self.compact:  # (resets are rare next to steps: the full rows come over, and the next step starts afresh)
-            self.engine.reset(mask, self._dev_obs)
-            if mask is None:
-                self.obs.copy_(self._dev_obs, non_blocking=True)
-            else:
-                sel = torch.as_tensor(mask).to(torch.bool).cpu()
-                self.obs[sel] = self._dev_obs.cpu()[sel]
-            torch.cuda.current_stream(self.device).synchronize()
-            self._compact_first = True
-            return self.obs, {}
+        if self.compact:
+            return self._compact_reset(mask)
         self.engine.reset(mask, self.obs)
         if self.host_outputs:
             torch.cuda.current_stream(self.device).synchronize()
