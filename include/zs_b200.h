@@ -234,7 +234,7 @@ int zs_rollout(ZsHandle* h, int32_t n_steps, int64_t first_step_index, const int
  *   word 1      reserved
  *   words 2-3   the reward (float64 bits, little endian)
  *   words 4..   the entries: simple encoding — cell | value << 16; channels — two words: cell | thing << 16, then
- *               (life & 0xffff) | weapon << 16
+ *               (life & 0xffff) | weapon << 16 (value and life are signed 16-bit: a box/wall's may be negative)
  * so that a step costs about 0.5 KB per env over PCIe instead of 5-16 KB.  An env with more differing cells than a
  * record holds (or a value that does not fit) sets the overflow bit and gets its full row written to obs_dev, which the
  * caller fetches for that env alone.  zs_expand_compact (HOST code, threaded) turns the records the caller copied to

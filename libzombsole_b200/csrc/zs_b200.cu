@@ -1328,12 +1328,12 @@ static inline bool expand_write(const ExpandCtx& cx, int e, const uint32_t* r, u
     if (cx.reward) memcpy(cx.reward + e, r + 2, sizeof(double));
     if ((h0 >> 18) & 1u) { pv[0] = h0; return true; }  // the record could not hold this env: the caller copies its row from the device
     if (wpe == 1) {
-        for (int i = 0; i < n; ++i) { const uint32_t w = r[ZS_COMPACT_HEADER + i]; o[w & 0xffffu] = (int32_t)(w >> 16); }
+        for (int i = 0; i < n; ++i) { const uint32_t w = r[ZS_COMPACT_HEADER + i]; o[w & 0xffffu] = (int32_t)(int16_t)(w >> 16); }
     } else {
         for (int i = 0; i < n; ++i) {
             const uint32_t w0 = r[ZS_COMPACT_HEADER + 2 * i], w1 = r[ZS_COMPACT_HEADER + 2 * i + 1];
             const int cell = (int)(w0 & 0xffffu);
-            o[cell] = (int32_t)(w0 >> 16);
+            o[cell] = (int32_t)(int16_t)(w0 >> 16);
             o[(size_t)cells + cell] = (int32_t)(int16_t)(w1 & 0xffffu);
             o[2 * (size_t)cells + cell] = (int32_t)(w1 >> 16);
         }
@@ -1370,11 +1370,11 @@ static inline bool expand_diff(const ExpandCtx& cx, int e, const uint32_t* r, ui
         for (int c = 0; c < C; ++c) o[(size_t)c * cells + cell] = T[(size_t)c * cells + cell];
     };
     auto write = [&](int i) {
-        if (wpe == 1) { const uint32_t w = re[i]; o[w & 0xffffu] = (int32_t)(w >> 16); }
+        if (wpe == 1) { const uint32_t w = re[i]; o[w & 0xffffu] = (int32_t)(int16_t)(w >> 16); }
         else {
             const uint32_t w0 = re[2 * i], w1 = re[2 * i + 1];
             const int cell = (int)(w0 & 0xffffu);
-            o[cell] = (int32_t)(w0 >> 16);
+            o[cell] = (int32_t)(int16_t)(w0 >> 16);
             o[(size_t)cells + cell] = (int32_t)(int16_t)(w1 & 0xffffu);
             o[2 * (size_t)cells + cell] = (int32_t)(w1 >> 16);
         }
@@ -1709,7 +1709,7 @@ static inline bool expand_agents(const AgentExpandCtx& cx, int e, const uint32_t
             if ((unsigned)wx >= (unsigned)w || (unsigned)wy >= (unsigned)w) continue;
             int32_t* const oa = o + (size_t)a * cx.C * ww;
             const int idx = wy * w + wx;
-            oa[idx] = (int32_t)(w0 >> 16);
+            oa[idx] = (int32_t)(int16_t)(w0 >> 16);
             if (wpe == 2) { oa[ww + idx] = (int32_t)(int16_t)(w1 & 0xffffu); oa[2 * ww + idx] = (int32_t)(w1 >> 16); }
         }
     }

@@ -506,12 +506,28 @@ __device__ __forceinline__ int max_life_of_label(int label) { return label == ZS
 // (cell | payload << 16): the world-scope observation patches them every step straight from the list, the first
 // clean_dead_things of a world and the grid rebuild walk it instead of all the statics, and SIDX (one byte per static:
 // 0 not listed, entry + 1, or 255 = listed further back, found by searching for the cell) finds the entry when the
-// box/wall is hit again.  Payload: simple encoding — the cell value itself; channels —
-// label << 12 | (life & 0xfff); 0 — the box/wall is gone from World.things.  Entries are never removed.
+// box/wall is hit again.  Payload (16 bits): 0 — the box/wall is gone from World.things; simple encoding — the cell
+// value v << 1 | 1 (box/wall lives are int16 here, so v lies in [-4660, 1039]; an arithmetic shift of the entry by 17
+// gives v, and 0 for "gone", which shows an empty cell); channels — the life, a life of 0 stored as SPL_LIFE0 (the label
+// is the pristine template's at the cell).  SPL_LIFE0 is -32768: a channels life of exactly -32768 reads back as 0, the
+// one int16 life that does not come out as it is (reserved).  Entries are never removed.
+#define SPL_GONE 0
+#define SPL_LIFE0 (-32768)
 __device__ __forceinline__ int static_payload(const ZsParams& p, int max_life, int life, bool present) {
-    if (!present) return 0;
+    if (!present) return SPL_GONE;
+    if (p.obs_enc != ZS_OBS_SIMPLE) return life != 0 ? life : SPL_LIFE0;
     const int label = max_life == 10 ? ZS_LABEL_BOX : ZS_LABEL_WALL;
-    if (p.obs_enc == ZS_OBS_SIMPLE) { const int adj = life < 100 ? life : 100; return 256 * label + floordiv100(15 * adj); }
-    return (label << 12) | (life & 0xfff);
+    const int adj = life < 100 ? life : 100;
+    return (256 * label + floordiv100(15 * adj)) * 2 + 1;
+}
+__device__ __forceinline__ uint32_t spl_entry(int cell, int pay) { return (uint32_t)cell | ((uint32_t)pay << 16); }
+__device__ __forceinline__ bool spl_gone(uint32_t w) { return (w >> 16) == 0u; }
+// What the observation shows on an entry's cell (a gone box/wall leaves it empty): simple — v0 = the value; channels —
+// v0 = label, v1 = life.
+__device__ __forceinline__ void spl_cell_obs(const ZsParams& p, uint32_t w, int& v0, int& v1) {
+    if (p.obs_enc == ZS_OBS_SIMPLE) { v0 = (int)w >> 17; v1 = 0; return; }
+    const int pay = (int)w >> 16;
+    v0 = spl_gone(w) ? 0 : __ldg(p.tmpl_obs + (w & 0xffffu));
+    v1 = pay == SPL_LIFE0 ? 0 : pay;
 }
 #define SIDX_FAR 255

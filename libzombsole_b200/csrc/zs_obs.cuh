@@ -92,9 +92,12 @@ __device__ __forceinline__ void obs_store_cell(const ZsParams& p, int32_t* obs, 
 // reference shows the thing on a cell, else its decoration (observation.py:41-42); the occupancy grid says which
 // one that is, so every patched cell is written by exactly one lane and the three kinds of patches (damaged or
 // destroyed boxes/walls, dead bodies, mobile things) need no ordering among themselves — only after pass 1.
-__device__ __forceinline__ void obs_store_static(const ZsParams& p, int32_t* obs, int cell, int pay) {
-    if (p.obs_enc == ZS_OBS_SIMPLE) obs[cell] = pay;
-    else { obs[cell] = pay >> 12; obs[p.cells + cell] = (int)((uint32_t)pay << 20) >> 20; obs[2 * p.cells + cell] = 0; }
+__device__ __forceinline__ void obs_store_static(const ZsParams& p, int32_t* obs, uint32_t w) {
+    const int cell = w & 0xffffu;
+    int v0, v1;
+    spl_cell_obs(p, w, v0, v1);
+    if (p.obs_enc == ZS_OBS_SIMPLE) obs[cell] = v0;
+    else { obs[cell] = v0; obs[p.cells + cell] = v1; obs[2 * p.cells + cell] = 0; }
 }
 __device__ __forceinline__ CellInfo thing_info(const ZsParams& p, int s, int life, int meta) {
     CellInfo ci;
@@ -113,10 +116,10 @@ ZS_TPL __device__ __forceinline__ void obs_world_patch(const ZsParams& p, Env& e
     const int n_spl = (e.flags & FL_DMG) ? (int)SPN : 0;                 // boxes/walls whose observation differs
     const int n_dead = (e.flags & FL_DEAD_OVER) ? 0 : (int)DBL(0);        // dead bodies of this world, from the list
     const uint32_t w0 = lane < n_spl ? SPL(lane) : 0xffff0000u;
-    const int cell0 = w0 & 0xffffu, pay0 = w0 >> 16;
+    const int cell0 = w0 & 0xffffu;
     const int dc0 = lane < n_dead ? (int)DBL(1 + lane) : 0;
-    // gone from World.things (payload 0): whatever took the cell patches it itself; a thing on a dead body hides it
-    const bool do_static0 = lane < n_spl && (pay0 != 0 || GRID(cell0) == G_EMPTY);
+    // gone from World.things (SPL_GONE): whatever took the cell patches it itself; a thing on a dead body hides it
+    const bool do_static0 = lane < n_spl && (!spl_gone(w0) || GRID(cell0) == G_EMPTY);
     const bool do_dead0 = lane < n_dead && GRID(dc0) == G_DEAD;
     int tm0 = 0, tl0 = 0;
     uint32_t txy0 = 0;
@@ -124,7 +127,7 @@ ZS_TPL __device__ __forceinline__ void obs_world_patch(const ZsParams& p, Env& e
     if (p.tmpl_smem_off >= 0 && lane == 0) bulk_wait_all();  // pass 1 (TMA) has landed before any cell is patched
     gsync<G, CV>(e);
     PH(12);
-    if (do_static0) obs_store_static(p, obs, cell0, pay0);
+    if (do_static0) obs_store_static(p, obs, w0);
     if (do_dead0) obs_store_cell(p, obs, dc0, body);
     if (ONE) {
         if (tm0 & 0x80) obs_store_cell(p, obs, xy_y(txy0) * p.W + xy_x(txy0), thing_info(p, lane, tl0, tm0));
@@ -141,9 +144,8 @@ ZS_TPL __device__ __forceinline__ void obs_world_patch(const ZsParams& p, Env& e
 #pragma unroll 1
     for (int i = lane + G; i < n_spl; i += G) {
         const uint32_t w = SPL(i);
-        const int cell = w & 0xffffu, pay = w >> 16;
-        if (pay == 0 && GRID(cell) != G_EMPTY) continue;
-        obs_store_static(p, obs, cell, pay);
+        if (spl_gone(w) && GRID(w & 0xffffu) != G_EMPTY) continue;
+        obs_store_static(p, obs, w);
     }
 #pragma unroll 1
     for (int i = lane + G; i < n_dead; i += G) {
@@ -212,10 +214,10 @@ __device__ __forceinline__ bool obs_compact_entries(const ZsParams& p, Env& e, u
         const int pos = n + __popc(m & below_l);
         if (on) {
             if (simple) {
-                bad |= (unsigned)v0 > 0xffffu;
+                bad |= v0 < -32768 || v0 > 32767;
                 if (pos < cap) put(hdr + pos, (uint32_t)cell | ((uint32_t)v0 << 16));
             } else {
-                bad |= (unsigned)v0 > 0xffffu || (unsigned)v2 > 0xffffu || v1 < -32768 || v1 > 32767;
+                bad |= v0 < -32768 || v0 > 32767 || (unsigned)v2 > 0xffffu || v1 < -32768 || v1 > 32767;
                 if (pos < cap) {
                     put(hdr + 2 * pos, (uint32_t)cell | ((uint32_t)v0 << 16));
                     put(hdr + 2 * pos + 1, ((uint32_t)v1 & 0xffffu) | ((uint32_t)v2 << 16));
@@ -229,12 +231,12 @@ __device__ __forceinline__ bool obs_compact_entries(const ZsParams& p, Env& e, u
 #pragma unroll 1
     for (int i0 = 0; i0 < r_spl; i0 += G) {
         const int i = i0 + lane;
-        const uint32_t w = i < n_spl ? SPL(i) : 0xffff0000u;
-        const int cell = w & 0xffffu, pay = w >> 16;
-        // gone from World.things (payload 0): whatever took the cell shows itself; else the cell reads as empty
-        const bool on = i < n_spl && (pay != 0 || GRID(cell) == G_EMPTY);
-        int v0 = pay, v1 = 0;
-        if (!simple) { v0 = pay >> 12; v1 = (int)((uint32_t)pay << 20) >> 20; }
+        const uint32_t w = i < n_spl ? SPL(i) : 0u;
+        const int cell = w & 0xffffu;
+        // gone from World.things (SPL_GONE): whatever took the cell shows itself; else the cell reads as empty
+        const bool on = i < n_spl && (!spl_gone(w) || GRID(cell) == G_EMPTY);
+        int v0 = 0, v1 = 0;
+        if (on) spl_cell_obs(p, w, v0, v1);
         emit(on, cell, v0, v1, 0);
     }
     const int body0 = simple ? 256 * ZS_LABEL_DEAD_BODY : ZS_LABEL_DEAD_BODY;
@@ -320,12 +322,13 @@ ZS_TPL __device__ __forceinline__ int obs_world_record(const ZsParams& p, Env& e
 #pragma unroll 1
     for (int i0 = 0; i0 < r_spl; i0 += G) {
         const int i = i0 + lane;
-        const uint32_t w = i < n_spl ? SPL(i < n_spl ? i : 0) : 0xffff0000u;
-        const int cell = w & 0xffffu, pay = w >> 16;
-        // gone from World.things (payload 0): whatever took the cell shows itself; else the cell reads as empty
-        const bool on = i < n_spl && (pay != 0 || GRID(cell) == G_EMPTY);
-        if (simple) emit(on, cell, pay, 0, 0);
-        else emit(on, cell, pay >> 12, (int)((uint32_t)pay << 20) >> 20, 0);
+        const uint32_t w = i < n_spl ? SPL(i < n_spl ? i : 0) : 0u;
+        const int cell = w & 0xffffu;
+        // gone from World.things (SPL_GONE): whatever took the cell shows itself; else the cell reads as empty
+        const bool on = i < n_spl && (!spl_gone(w) || GRID(cell) == G_EMPTY);
+        int v0 = 0, v1 = 0;
+        if (on) spl_cell_obs(p, w, v0, v1);
+        emit(on, cell, v0, v1, 0);
     }
     const int body0 = simple ? 256 * ZS_LABEL_DEAD_BODY : ZS_LABEL_DEAD_BODY;
     const int n_dead = (e.flags & FL_DEAD_OVER) ? 0 : (int)DBL(0);
@@ -532,10 +535,11 @@ ZS_TPL __device__ __forceinline__ void encode_surroundings(const ZsParams& p, En
 #pragma unroll 1
         for (int i = lane; i < n_spl; i += G) {
             const uint32_t wd = SPL(i);
-            const int cell = wd & 0xffffu, pay = wd >> 16;
-            if (pay == 0 && GRID(cell) != G_EMPTY) continue;  // gone: whatever took the cell shows itself
-            if (simple) into_windows(cell, pay, 0, 0);
-            else into_windows(cell, pay >> 12, (int)((uint32_t)pay << 20) >> 20, 0);
+            const int cell = wd & 0xffffu;
+            if (spl_gone(wd) && GRID(cell) != G_EMPTY) continue;  // gone: whatever took the cell shows itself
+            int v0, v1;
+            spl_cell_obs(p, wd, v0, v1);
+            into_windows(cell, v0, v1, 0);
         }
     }
     const int body0 = simple ? 256 * ZS_LABEL_DEAD_BODY : ZS_LABEL_DEAD_BODY;

@@ -207,12 +207,12 @@ ZS_TPL __device__ __forceinline__ void spl_update_one(const ZsParams& p, const E
         SPN = (uint16_t)idx;
         SIDX(si) = (uint8_t)(idx < SIDX_FAR ? idx : SIDX_FAR);
     } else if (idx == SIDX_FAR) idx = spl_find_far<MPC, G, CV>(p, e, cell);
-    SPL(idx - 1) = (uint32_t)cell | ((uint32_t)pay << 16);
+    SPL(idx - 1) = spl_entry(cell, pay);
 }
 
 // A new world: every box/wall is back in World.things, also the ones with life <= 0 (game.py:154-155).
 // (An entry with a payload already shows its box/wall as present with its current life: only the entries of boxes/walls
-// that were gone — payload 0 — change, so the map tables are only read for those.)  restore_grid: the grid is not
+// that were gone — SPL_GONE — change, so the map tables are only read for those.)  restore_grid: the grid is not
 // rebuilt from the template by the caller; the returning boxes/walls are put back on it here.
 ZS_TPL __device__ __forceinline__ void spl_refresh_present(const ZsParams& p, const Env& e, bool restore_grid = false) {
     ZS_VIEWS;
@@ -220,10 +220,10 @@ ZS_TPL __device__ __forceinline__ void spl_refresh_present(const ZsParams& p, co
 #pragma unroll 1
     for (int i = e.gl; i < n; i += G) {
         const uint32_t w = SPL(i);
-        if ((w >> 16) != 0u) continue;
+        if (!spl_gone(w)) continue;
         const int cell = w & 0xffffu;
         const int si = __ldg(p.cell_static + cell);
-        SPL(i) = (uint32_t)cell | ((uint32_t)static_payload(p, __ldg(p.static_max + si), SL(si), true) << 16);
+        SPL(i) = spl_entry(cell, static_payload(p, __ldg(p.static_max + si), SL(si), true));
         if (restore_grid) GRID(cell) = G_STATIC;
     }
 }
@@ -238,7 +238,7 @@ ZS_TPL __device__ __forceinline__ int spl_clean_fresh(const ZsParams& p, const E
     for (int i = e.gl; i < n; i += G) {
         const int cell = SPL(i) & 0xffffu;
         if (!g_is_static(GRID(cell))) continue;
-        if (SL(__ldg(p.cell_static + cell)) <= 0) { GRID(cell) = G_EMPTY; SPL(i) = (uint32_t)cell; ++gone; }
+        if (SL(__ldg(p.cell_static + cell)) <= 0) { GRID(cell) = G_EMPTY; SPL(i) = spl_entry(cell, SPL_GONE); ++gone; }
     }
     return gone;
 }
@@ -415,10 +415,10 @@ ZS_TPL __device__ __noinline__ void build_grid(const ZsParams& p, GrpId id, int 
 #pragma unroll 4
     for (int i = e.gl; i < (p.cells_pad >> 4); i += G) reinterpret_cast<uint4*>(GRIDP)[i] = __ldg(tg + i);
     gsync<G, CV>(e);
-    if (flags & FL_DMG) {  // boxes/walls that are gone from World.things (payload 0 in the static patch list)
+    if (flags & FL_DMG) {  // boxes/walls that are gone from World.things (SPL_GONE in the static patch list)
         const int n = SPN;
 #pragma unroll 1
-        for (int i = e.gl; i < n; i += G) { const uint32_t w = SPL(i); if ((w >> 16) == 0u) GRID(w & 0xffffu) = G_EMPTY; }
+        for (int i = e.gl; i < n; i += G) { const uint32_t w = SPL(i); if (spl_gone(w)) GRID(w & 0xffffu) = G_EMPTY; }
         gsync<G, CV>(e);
     }
 #pragma unroll 1
@@ -1028,7 +1028,7 @@ ZS_TPL __device__ __forceinline__ int world_step(const ZsParams& p, Env& e) {
                 gsync<G, CV>(e);  // (everybody has read the count before lane 0 rewrites it)
                 if (is_new) { idx = n0 + __popc(new_m & below_l) + 1; SIDX(si) = (uint8_t)(idx < SIDX_FAR ? idx : SIDX_FAR); }
                 else if (idx == SIDX_FAR) idx = spl_find_far<MPC, G, CV>(p, e, cell);
-                if (slead && idx) SPL(idx - 1) = (uint32_t)cell | ((uint32_t)pay << 16);
+                if (slead && idx) SPL(idx - 1) = spl_entry(cell, pay);
                 if (new_m) {
                     if (lane == 0) SPN = (uint16_t)(n0 + __popc(new_m));
                     e.flags |= FL_DMG;
@@ -1520,7 +1520,7 @@ __device__ __forceinline__ int world_step_one(const ZsParams& p, Env& e, int at,
                 gsync<G, CV>(e);  // (everybody has read the count before lane 0 rewrites it)
                 if (is_new) { idx = n0 + __popc(new_m & below_s) + 1; SIDX(si) = (uint8_t)(idx < SIDX_FAR ? idx : SIDX_FAR); }
                 else if (idx == SIDX_FAR) idx = spl_find_far<MPC, G, CV>(p, e, cell);
-                if (slead && idx) SPL(idx - 1) = (uint32_t)cell | ((uint32_t)pay << 16);
+                if (slead && idx) SPL(idx - 1) = spl_entry(cell, pay);
                 if (new_m) {
                     if (s == 0) SPN = (uint16_t)(n0 + __popc(new_m));
                     e.flags |= FL_DMG;
