@@ -243,10 +243,11 @@ int zs_rollout(ZsHandle* h, int32_t n_steps, int64_t first_step_index, const int
  * the same tensor cell by cell; gym_env.py:99-145 returns it with reward and flags.) */
 #define ZS_COMPACT_HEADER 4
 /* zs_compact_words: a good record size for this handle in words (0 if the configuration has no compact form:
- * surroundings scope, per-agent observations, more than 32 slots); zs_compact_max_words: the size no env overflows
- * by count.  The caller picks compact_words (the same value for zs_step_compact and zs_expand_compact of a step) and may
- * grow it when overflows become frequent: box/wall damage persists across episodes (game.py:154-155), so the number of
- * differing cells of a long-running env creeps up. */
+ * surroundings scope, per-agent observations); zs_compact_max_words: the size no env overflows by count.  Games of at
+ * most 32 slots default to 96 words (simple) / 192 (channels); games of more slots to room for every slot plus as many
+ * entries again as a small game gets (224 / 416 words for 101 slots).  The caller picks compact_words (the same value for
+ * zs_step_compact and zs_expand_compact of a step) and may grow it when overflows become frequent: box/wall damage
+ * persists across episodes (game.py:154-155), so the number of differing cells of a long-running env creeps up. */
 int32_t zs_compact_words(const ZsHandle* h);
 int32_t zs_compact_max_words(const ZsHandle* h);
 int zs_step_compact(ZsHandle* h, const int32_t* actions_dev, int32_t action_format, uint32_t* compact_dev,

@@ -37,8 +37,27 @@ __device__ __forceinline__ void discrete_to_action(const ZsParams& p, int id, in
     type = (int)(w & 0xffu); dx = (int)((w >> 8) & 0xffu) - 1; dy = (int)(w >> 16) - 1;
 }
 
+// zs_step_host: the env's record is complete.  ONE system-scope fence per group of envs, by whoever completes the group (a fence
+// per warp takes 8-34 us when 4,096 warps fence at once): the others order their record words before the counter at gpu scope.
+template <int G, bool CV>
+__device__ __forceinline__ void compact_signal(const ZsParams& p, const ZsIO& io, const Env& e, int env) {
+    __threadfence();
+    gsync<G, CV>(e);
+    if (e.gl == 0) {
+        const int grp = env / io.group_envs;
+        const int size = min(io.group_envs, p.N - grp * io.group_envs);
+        if (atomicAdd(io.group_count + grp, 1) == size - 1) {
+            io.group_count[grp] = 0;
+            __threadfence_system();
+            *reinterpret_cast<volatile uint32_t*>(io.host_flags + 16 * grp) = io.ticket;
+        }
+    }
+}
+
 // ---------------------------------------------------------------- the K-step loop, more slots than lanes
-template <int MPC, int G, bool CV, bool SURR>
+// REC: world scope with the compact record compiled in (zs_sim_kernel SHAPE 5): every step leaves as a record (zs_step_compact,
+// zs_step_host), the full row only for an env the record cannot hold.
+template <int MPC, int G, bool CV, bool SURR, bool REC = false>
 __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO& io, Env& e) {
     ZS_CONSTS; ZS_VIEWS;
     const int lane = e.gl, env = e.env;
@@ -71,7 +90,7 @@ __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO&
             obs_out = io.obs + ((size_t)oslot * p.N + env) * p.obs_elems;
             if (++oslot >= io.obs_slots) oslot = 0;
             // pass 1 of the world observation does not depend on the transition: issue its stores now
-            if constexpr (world_obs) obs_world_template<MPC, G, CV>(p, e, obs_out);
+            if constexpr (world_obs && !REC) obs_world_template<MPC, G, CV>(p, e, obs_out);
         }
         // agents alive before the step: the keys of the reference's per-agent dicts (multiagent_env.py:88-97)
         unsigned alive_before = 0;
@@ -172,28 +191,29 @@ __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO&
             initialize_world<MPC, G, false>(p, id_of(e), e.episode + 1, e.flags);
             scalars_from_smem<MPC, G, false>(p, e);
         }
-        if (obs_out) {
+        if constexpr (REC) {
+            // the observation as a compact record with the reward and flags in its header (include/zs_b200.h: zs_step_compact),
+            // staged in the step's scratch (EnvS::act .. zb): the respawn and the world init above were its last users, and the
+            // next step writes it only after the sync at the end of this one
+            uint32_t* const rec = io.compact + (size_t)env * io.compact_words;
+            uint32_t* const stage = reinterpret_cast<uint32_t*>(zs_smem + e.b);
+            int n_ent = 0;
+            const bool over = obs_world_compact<MPC, G, CV>(p, e, rec, io.compact_words - ZS_COMPACT_HEADER, n_ent);
+            if (lane == 0) {
+                stage[0] = (uint32_t)n_ent | (done ? 1u << 16 : 0u) | (trunc ? 1u << 17 : 0u) | (over ? 1u << 18 : 0u); stage[1] = 0u;
+                stage[2] = (uint32_t)__double2loint(rew[0]); stage[3] = (uint32_t)__double2hiint(rew[0]);
+            }
+            compact_flush<MPC, G, CV>(e, rec, ZS_COMPACT_HEADER + n_ent * (p.obs_enc == ZS_OBS_SIMPLE ? 1 : 2));
+            if (over && obs_out) {  // rare: the full row, for the caller to fetch
+                obs_world_template<MPC, G, CV>(p, e, obs_out);
+                obs_world_patch<MPC, G, CV>(p, e, obs_out);
+            }
+            if (io.host_flags) compact_signal<G, CV>(p, io, e, env);
+        } else if (obs_out) {
             if constexpr (world_obs) obs_world_patch<MPC, G, CV>(p, e, obs_out);
             else encode_surroundings<MPC, G, CV>(p, e, obs_out);
         }
         gsync<G, CV>(e);
-    }
-}
-
-// zs_step_host: the env's record is complete.  ONE system-scope fence per group of envs, by whoever completes the group (a fence
-// per warp takes 8-34 us when 4,096 warps fence at once): the others order their record words before the counter at gpu scope.
-template <int G, bool CV>
-__device__ __forceinline__ void compact_signal(const ZsParams& p, const ZsIO& io, const Env& e, int env) {
-    __threadfence();
-    gsync<G, CV>(e);
-    if (e.gl == 0) {
-        const int grp = env / io.group_envs;
-        const int size = min(io.group_envs, p.N - grp * io.group_envs);
-        if (atomicAdd(io.group_count + grp, 1) == size - 1) {
-            io.group_count[grp] = 0;
-            __threadfence_system();
-            *reinterpret_cast<volatile uint32_t*>(io.host_flags + 16 * grp) = io.ticket;
-        }
     }
 }
 
@@ -415,6 +435,8 @@ __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io,
 // SHAPE 4 = surroundings observation with the per-agent compact record (zs_step_compact_agents / zs_step_host_agents; step
 // launches of at most 32 slots only): a kernel of its own, since with the record compiled into SHAPE 2 that kernel spilled more
 // and its device-output steps of config 3's game at 65,536 envs took 6 % longer (profiles/r04_ab_surroundings.txt).
+// SHAPE 5 = world-scope observation with the compact record, more slots than lanes (zs_step_compact / zs_step_host; step
+// launches of 128 and 256 slots only): a kernel of its own, so that the device-output general kernels stay as they are.
 // ROS: the game roster compiled into a standard-rollout-shape kernel (zs_world.cuh: Roster), 0 = read from ZsParams.
 template <int MODE, int MPC, int G, int SHAPE, int OCC, int ROS = 0>
 __global__ void __launch_bounds__(SHAPE == 3 ? 160 : ZS_WPC * 32, OCC) zs_sim_kernel(const __grid_constant__ ZsParams p, const __grid_constant__ ZsIO io) {
@@ -527,7 +549,7 @@ __global__ void __launch_bounds__(SHAPE == 3 ? 160 : ZS_WPC * 32, OCC) zs_sim_ke
     e.ph_last = clock64();
 #endif
     if constexpr (ONE) step_loop_one<MPC, G, CV, FAST, SURR, PROD, ROS, SHAPE == 4>(p, io, e);
-    else step_loop_general<MPC, G, CV, SURR>(p, io, e);
+    else step_loop_general<MPC, G, CV, SURR, SHAPE == 5>(p, io, e);
 #ifdef ZS_PHASE_CLOCKS
     e.ph_last = clock64();
 #endif
@@ -651,6 +673,13 @@ struct DeviceGuard {
 };
 
 static int round_up(int v, int m) { return (v + m - 1) / m * m; }
+// the compact record size that no env can overflow by count: every thing, every box/wall, every listed dead body
+static int compact_max_words(const ZsParams& p) {
+    const int wpe = p.obs_enc == ZS_OBS_SIMPLE ? 1 : 2;
+    const int entries = p.M + p.S + p.cells;  // (dead bodies: at most every cell; far more than ever occurs)
+    const int cap = p.M + p.S + 64;
+    return round_up(ZS_COMPACT_HEADER + wpe * (cap < entries ? cap : entries), 32);
+}
 
 extern "C" __attribute__((visibility("default"))) int zs_abi_version(void) { return ZS_ABI_VERSION; }
 extern "C" __attribute__((visibility("default"))) int zs_set_device(int32_t device) {
@@ -749,7 +778,7 @@ static void launch_sim(const ZsHandle* h, const ZsIO& io, cudaStream_t st) {
     // the standard rollout shape of a batch that one wave of producer-warp CTAs holds: observations through a third warp
     const bool prod = fast && MODE == MODE_STEP && sh.prod_smem_bytes > 0 && pp.tmpl_smem_off >= 0 && io.env_mask == nullptr;
     // SH_: 0 world scope, 1 the standard rollout shape (step launches only), 2 surroundings, 4 surroundings with the per-agent
-    // record (step launches only) (zs_sim_kernel: SHAPE)
+    // record, 5 world scope with the record and more slots than lanes (4 and 5: step launches only) (zs_sim_kernel: SHAPE)
     // Programmatic dependent launch: the kernel's CTAs may be scheduled while the previous kernel of the stream is still
     // draining (they stage the observation template and then wait in griddepcontrol.wait for that kernel to have
     // completed, all its writes visible) — the launch latency and the ramp hide under the predecessor's tail.
@@ -763,12 +792,13 @@ static void launch_sim(const ZsHandle* h, const ZsIO& io, cudaStream_t st) {
     // rollouts lose 1-1.5 % — the early CTAs of the next launch sit on the SMs — so only short step launches ask for it)
     const bool pdl = h->use_pdl == 1 || (h->use_pdl == 2 && MODE == MODE_STEP && io.n_steps < h->short_steps);
     lc.attrs = la; lc.numAttrs = pdl ? 1 : 0;
-#define ZS_LAUNCH_R(MPC_, G_, SH_, O_, R_) cudaLaunchKernelEx(&lc, zs_sim_kernel<MODE, MPC_, G_, MODE == MODE_STEP ? (SH_) : (SH_) == 1 ? 0 : (SH_) == 4 ? 2 : (SH_), MODE == MODE_STEP ? (O_) : ZS_MIN_CTAS, MODE == MODE_STEP ? (R_) : 0>, pp, io)
+#define ZS_LAUNCH_R(MPC_, G_, SH_, O_, R_) cudaLaunchKernelEx(&lc, zs_sim_kernel<MODE, MPC_, G_, MODE == MODE_STEP ? (SH_) : (SH_) == 1 || (SH_) == 5 ? 0 : (SH_) == 4 ? 2 : (SH_), MODE == MODE_STEP ? (O_) : ZS_MIN_CTAS, MODE == MODE_STEP ? (R_) : 0>, pp, io)
 #define ZS_LAUNCH(MPC_, G_, SH_, O_) ZS_LAUNCH_R(MPC_, G_, SH_, O_, 0)
 #define ZS_LAUNCH_F(MPC_, G_, O_) do { if (roster) ZS_LAUNCH_R(MPC_, G_, 1, O_, (MPC_) == 16 ? ZS_ROSTER_BENCH : 0); else if (fast) ZS_LAUNCH(MPC_, G_, 1, O_); \
                                        else if (surr && io.compact) ZS_LAUNCH(MPC_, G_, 4, O_); else if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); \
                                        else ZS_LAUNCH(MPC_, G_, 0, O_); } while (0)
-#define ZS_LAUNCH_G(MPC_, G_, O_) do { if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); else ZS_LAUNCH(MPC_, G_, 0, O_); } while (0)
+#define ZS_LAUNCH_G(MPC_, G_, O_) do { if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); else if (io.compact) ZS_LAUNCH(MPC_, G_, 5, O_); \
+                                       else ZS_LAUNCH(MPC_, G_, 0, O_); } while (0)
     if (prod) {
         pp.prod_off = sh.prod_off; pp.prod_cap = sh.prod_cap; pp.tmpl_smem_off = ZS_PROD_ENVS * sh.smem_per_env;
         lc.gridDim = dim3((pp.N + ZS_PROD_ENVS - 1) / ZS_PROD_ENVS); lc.blockDim = dim3(32 * (ZS_PROD_ENVS / 2 + 1));
@@ -807,6 +837,8 @@ static cudaError_t set_smem_attr_step(int bytes) {
     if (e == cudaSuccess && MPC == 16) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (MPC == 16 ? 1 : 0), OCC, (MPC == 16 ? ZS_ROSTER_BENCH : 0)>, attr, bytes);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, 2, OCC>, attr, bytes);
     if (e == cudaSuccess && MPC <= 32) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (MPC <= 32 ? 4 : 2), OCC>, attr, bytes);
+    constexpr bool rec_g = MPC > 32 && OCC == ZS_OCC_GENERAL;  // (the only occupancy launch_sim runs them at)
+    if (e == cudaSuccess && rec_g) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (rec_g ? 5 : 0), OCC>, attr, bytes);
     return e;
 }
 template <int MPC, int G>
@@ -1069,8 +1101,13 @@ extern "C" __attribute__((visibility("default"))) int zs_create(const ZsConfig* 
     if (const char* force = getenv("ZS_PDL")) h->use_pdl = atoi(force) ? 1 : 0;
     if (const char* force = getenv("ZS_SHORT_STEPS")) h->short_steps = atoi(force);
     h->tmpl_single_step = getenv("ZS_NO_TMA_SINGLE") ? 0 : 1;
-    h->compact_words = (p.mpc <= 32 && p.obs_scope == ZS_OBS_WORLD && !p.obs_per_agent)
-                           ? (p.obs_enc == ZS_OBS_SIMPLE ? 96 : 192) : 0;  // header + 92 entries; the caller grows them
+    // header + 92 entries; with more slots than lanes, room for every slot on top (config 4's maze game: 224 / 416 words).  The
+    // caller grows them.
+    h->compact_words = 0;
+    if (p.obs_scope == ZS_OBS_WORLD && !p.obs_per_agent) {
+        const int wpe = p.obs_enc == ZS_OBS_SIMPLE ? 1 : 2;
+        h->compact_words = p.mpc <= 32 ? (wpe == 1 ? 96 : 192) : std::min(round_up(ZS_COMPACT_HEADER + wpe * (p.M + 92), 32), compact_max_words(p));
+    }
     // (the entry count and the window centres are 16-bit fields: fewer than 65,536 cells is what zs_layout accepts)
     h->agent_compact_words = (p.mpc <= 32 && p.obs_scope == ZS_OBS_SURROUNDINGS && p.obs_per_agent)
                                  ? round_up(ZS_AGENT_COMPACT_HEADER(p.A) + (p.obs_enc == ZS_OBS_SIMPLE ? 1 : 2) * 92, 32) : 0;
@@ -1261,20 +1298,15 @@ extern "C" __attribute__((visibility("default"))) int zs_step_masked(ZsHandle* h
 }
 
 extern "C" __attribute__((visibility("default"))) int32_t zs_compact_words(const ZsHandle* h) { return h ? h->compact_words : 0; }
-// the record size that no env can overflow by count: every thing, every box/wall, every listed dead body
 extern "C" __attribute__((visibility("default"))) int32_t zs_compact_max_words(const ZsHandle* h) {
-    if (!h || !h->compact_words) return 0;
-    const int wpe = h->p.obs_enc == ZS_OBS_SIMPLE ? 1 : 2;
-    const int entries = h->p.M + h->p.S + h->p.cells;  // (dead bodies: at most every cell; far more than ever occurs)
-    const int cap = h->p.M + h->p.S + 64;
-    return round_up(ZS_COMPACT_HEADER + wpe * (cap < entries ? cap : entries), 32);
+    return h && h->compact_words ? compact_max_words(h->p) : 0;
 }
 
 extern "C" __attribute__((visibility("default"))) int zs_step_compact(ZsHandle* h, const int32_t* actions_dev, int32_t action_format, uint32_t* compact_dev,
                                                                        int32_t compact_words, int32_t* obs_dev, void* stream) {
     if (int rc = check_bound(h)) return rc;
     DeviceGuard guard(h);
-    if (!h->compact_words) return fail("this configuration has no compact observation form (world scope, one reward per env, at most 32 slots)");
+    if (!h->compact_words) return fail("this configuration has no compact observation form (world scope, one reward per env)");
     if (!actions_dev || !compact_dev) return fail("zs_step_compact needs an action tensor and a record buffer");
     if (compact_words < ZS_COMPACT_HEADER + 8 || compact_words > 65535) return fail("compact_words out of range");
     if (action_format != ZS_ACTIONS_FULL && action_format != ZS_ACTIONS_DISCRETE) return fail("bad action format");
@@ -1575,7 +1607,7 @@ extern "C" __attribute__((visibility("default"))) int zs_step_host(ZsHandle* h, 
                                                                     int32_t n_threads, void* stream) {
     if (int rc = check_bound(h)) return rc;
     DeviceGuard guard(h);
-    if (!h->compact_words) return fail("this configuration has no compact observation form (world scope, one reward per env, at most 32 slots)");
+    if (!h->compact_words) return fail("this configuration has no compact observation form (world scope, one reward per env)");
     if (!actions_host || !compact_pinned || !prev_host || !obs_host || !overflow_envs_host || !n_overflow) return fail("null argument");
     if (compact_words < ZS_COMPACT_HEADER + 8 || compact_words > 65535) return fail("compact_words out of range");
     if (action_format != ZS_ACTIONS_FULL && action_format != ZS_ACTIONS_DISCRETE) return fail("bad action format");

@@ -266,7 +266,18 @@ __device__ __forceinline__ bool obs_compact_entries(const ZsParams& p, Env& e, u
             }
         }
     }
-    {
+    if constexpr (MPC > G) {  // more slots than lanes (step_loop_general): a ballot round per G slots
+#pragma unroll 1
+        for (int s0 = 0; s0 < p.M; s0 += G) {
+            const int s = s0 + lane;
+            const int m = s < p.M ? (int)TM(s) : 0;
+            const bool on = (m & 0x80) != 0;
+            const uint32_t xy = on ? TXY(s) : 0u;
+            const CellInfo ci = thing_info(p, s, on ? (int)TL(s) : 0, m);
+            if (simple) emit(on, xy_y(xy) * p.W + xy_x(xy), encode_simple(ci), 0, 0);
+            else emit(on, xy_y(xy) * p.W + xy_x(xy), channel_label(p, ci), ci.life, ci.weapon);
+        }
+    } else {
         const bool in_cap = G == MPC || lane < MPC;
         const int m = in_cap ? (int)TM(lane) : 0;
         const bool on = (m & 0x80) != 0;

@@ -186,7 +186,7 @@ class ZombsoleVectorEnv(CompactHostOutputs):
         if self.compact:
             words = self.engine.compact_words()
             if not words:
-                raise ValueError("host_outputs='compact' needs a world-scope observation and at most 32 things per env")
+                raise ValueError("host_outputs='compact' needs a world-scope observation")
             self.obs, self.reward, self._term, self._trunc = self.engine.new_host_outputs()
             self._dev_obs = self.engine.new_obs()  # full rows of the rare envs a record cannot hold
             self._overflow = torch.zeros(num_envs, dtype=torch.int32)
