@@ -21,6 +21,8 @@
  *   zs_encode_obs    observation_handler.get_observation(game)         zombsole/gym/observation.py:36-173
  *   zs_rollout       a K-step loop of the above with same-step auto-reset (what an RL rollout does
  *                    around gym_env.py:99-164); one launch, state stays on chip between steps
+ *   zs_step_final / zs_rollout_final   zs_step / zs_rollout that also return the observation an auto-reset episode
+ *                    ended with (gym_env.py:99-164)
  *   zs_fill_synthetic_actions   Discrete(6|7).sample() for synthetic rollouts (gym_env.py:367)
  *   zs_step_compact_agents / zs_expand_compact_agents / zs_step_host_agents
  *                    MultiagentZombsoleEnv.step with its per-agent windows  zombsole/gym/multiagent_env.py:111-171,
@@ -225,6 +227,24 @@ int zs_encode_obs(ZsHandle* h, int32_t* obs_dev, void* stream);
 int zs_rollout(ZsHandle* h, int32_t n_steps, int64_t first_step_index, const int32_t* actions_dev,
                int32_t action_format, int32_t* obs_dev, int32_t obs_slots, double* reward_dev,
                uint8_t* terminated_dev, uint8_t* truncated_dev, void* stream);
+
+/* ---- final observations of auto-reset episodes (gymnasium's SAME_STEP autoreset: info["final_obs"], info["_final_obs"])
+ * An env whose step ends its episode (terminated or truncated, TimeLimit included) is re-initialised in the same step, and
+ * obs_dev receives the first observation of the new episode.  These two calls also write, for each such env, the
+ * observation of the world the episode ended in to its row of final_obs_dev: exactly what zs_step writes for that step on a
+ * handle with auto_reset = 0 — taken after the transition, the reward and the minimum-zombie respawn, before the world init
+ * (zombsole/gym_env.py:99-164, zombsole/gym/multiagent_env.py:111-184).  final_obs_dev has the layout of obs_dev.  The rows
+ * of envs whose step did not end an episode are unspecified: terminated | truncated says which rows hold a final
+ * observation.  Everything else (outputs, state, episode statistics) is what zs_step / zs_rollout compute.  Both calls need
+ * non-NULL obs_dev and final_obs_dev.
+ * zs_step_final: zs_step on a handle with auto_reset = 1 (it fails on another: nothing would be re-initialised).
+ * zs_rollout_final: zs_rollout; final_obs_dev int32 [obs_slots, N, obs_elems_per_env], step i writes slot i % obs_slots. */
+int zs_step_final(ZsHandle* h, const int32_t* actions_dev, int32_t action_format, int32_t* obs_dev,
+                  int32_t* final_obs_dev, double* reward_dev, uint8_t* terminated_dev, uint8_t* truncated_dev,
+                  uint8_t* agent_mask_dev, int32_t* draws_dev, void* stream);
+int zs_rollout_final(ZsHandle* h, int32_t n_steps, int64_t first_step_index, const int32_t* actions_dev,
+                     int32_t action_format, int32_t* obs_dev, int32_t* final_obs_dev, int32_t obs_slots,
+                     double* reward_dev, uint8_t* terminated_dev, uint8_t* truncated_dev, void* stream);
 
 /* ---- compact host outputs (world-scope observation, one agent's reward per env)
  * The world observation of an env is the map's pristine layer (the same for every env and step) plus a few dozen cells

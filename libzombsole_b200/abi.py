@@ -95,9 +95,13 @@ PROTOTYPES = {
     "zs_reset": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "zs_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                           C.c_void_p, C.c_void_p, C.c_void_p]),
+    "zs_step_final": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "zs_encode_obs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "zs_rollout": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32,
                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "zs_rollout_final": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                   C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "zs_fill_synthetic_actions": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "zs_fill_synthetic_tape": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
     "zs_episode_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),

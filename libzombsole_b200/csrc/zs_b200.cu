@@ -57,7 +57,9 @@ __device__ __forceinline__ void compact_signal(const ZsParams& p, const ZsIO& io
 // ---------------------------------------------------------------- the K-step loop, more slots than lanes
 // REC: world scope with the compact record compiled in (zs_sim_kernel SHAPE 5): every step leaves as a record (zs_step_compact,
 // zs_step_host), the full row only for an env the record cannot hold.
-template <int MPC, int G, bool CV, bool SURR, bool REC = false>
+// FIN: the final observation compiled in (zs_sim_kernel SHAPE 6 / 7): an env that the step re-initialises first writes the
+// observation of the world it ended in to its row of io.final_obs, in the ring slot of the step's own observation.
+template <int MPC, int G, bool CV, bool SURR, bool REC = false, bool FIN = false>
 __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO& io, Env& e) {
     ZS_CONSTS; ZS_VIEWS;
     const int lane = e.gl, env = e.env;
@@ -187,6 +189,9 @@ __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO&
                 atomicAdd(p.stats + 2, (unsigned long long)e.ep_steps);
                 atomicAdd(p.stats + 3, (unsigned long long)e.zd);
             }
+            // the terminal world, after the transition, the reward and the respawn: what zs_step writes without auto-reset
+            // (gym_env.py:99-145)
+            if constexpr (FIN) encode_obs<MPC, G, CV, SURR>(p, e, io.final_obs + (obs_out - io.obs));
             // rare, and possibly only one env of the warp: the divergent flavour
             initialize_world<MPC, G, false>(p, id_of(e), e.episode + 1, e.flags);
             scalars_from_smem<MPC, G, false>(p, e);
@@ -227,7 +232,8 @@ __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO&
 // written by the game warp: no bulk-copy issue, no wait for it, no global stores on the game warps' dependent chain.
 // ROS: a game roster compiled in (zs_world.cuh: Roster; the standard rollout shape only), 0 = the game from ZsParams.
 // REC: surroundings scope with the per-agent compact record compiled in (zs_sim_kernel SHAPE 4).
-template <int MPC, int G, bool CV, bool FAST, bool SURR, bool PROD = false, int ROS = 0, bool REC = false>
+// FIN: the final observation compiled in (zs_sim_kernel SHAPE 6 / 7, as for step_loop_general).
+template <int MPC, int G, bool CV, bool FAST, bool SURR, bool PROD = false, int ROS = 0, bool REC = false, bool FIN = false>
 __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io, Env& e) {
     ZS_CONSTS; ZS_VIEWS;
     const int lane = e.gl, env = e.env;
@@ -346,6 +352,10 @@ __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io,
                 atomicAdd(p.stats + 2, (unsigned long long)e.ep_steps);
                 atomicAdd(p.stats + 3, (unsigned long long)e.zd);
             }
+            // the terminal world, after the transition, the reward and the respawn: what zs_step writes without auto-reset
+            // (gym_env.py:99-145).  The encoders are group-collective, so both envs of a warp write their row: the row of an
+            // env that did not end is not flagged to the caller.
+            if constexpr (FIN) encode_obs<MPC, G, CV, SURR>(p, e, io.final_obs + (obs_out - io.obs));
             if (R::on || p.fast_init) initialize_world_fast<MPC, G, CV, ROS>(p, e, need_init);  // both envs of the warp, converged
             else if (need_init) {  // possibly only one env of the warp: the divergent flavour
                 initialize_world<MPC, G, false>(p, id_of(e), e.episode + 1, e.flags);
@@ -437,12 +447,16 @@ __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io,
 // and its device-output steps of config 3's game at 65,536 envs took 6 % longer (profiles/r04_ab_surroundings.txt).
 // SHAPE 5 = world-scope observation with the compact record, more slots than lanes (zs_step_compact / zs_step_host; step
 // launches of 128 and 256 slots only): a kernel of its own, so that the device-output general kernels stay as they are.
+// SHAPE 6 / 7 = world-scope / surroundings observation with the final observation of every env the step re-initialises
+// (zs_step_final / zs_rollout_final; step launches only): kernels of their own, so that the kernels without it stay as they
+// are (the record of SHAPE 4 compiled into SHAPE 2 made it spill more and slowed config 3 by 6 %).
 // ROS: the game roster compiled into a standard-rollout-shape kernel (zs_world.cuh: Roster), 0 = read from ZsParams.
 template <int MODE, int MPC, int G, int SHAPE, int OCC, int ROS = 0>
 __global__ void __launch_bounds__(SHAPE == 3 ? 160 : ZS_WPC * 32, OCC) zs_sim_kernel(const __grid_constant__ ZsParams p, const __grid_constant__ ZsIO io) {
     ZS_CONSTS;
     constexpr bool PROD = SHAPE == 3;
-    constexpr bool FAST = SHAPE == 1 || PROD, SURR = SHAPE == 2 || SHAPE == 4;
+    constexpr bool FAST = SHAPE == 1 || PROD, SURR = SHAPE == 2 || SHAPE == 4 || SHAPE == 7;
+    constexpr bool FIN = SHAPE == 6 || SHAPE == 7;
     // the step kernel keeps both envs of a warp converged (zs_device.cuh); masked resets and encodes may not
     constexpr bool CV = MODE == MODE_STEP;
     constexpr int EPW = 32 / G;  // envs per warp
@@ -548,8 +562,8 @@ __global__ void __launch_bounds__(SHAPE == 3 ? 160 : ZS_WPC * 32, OCC) zs_sim_ke
 #ifdef ZS_PHASE_CLOCKS
     e.ph_last = clock64();
 #endif
-    if constexpr (ONE) step_loop_one<MPC, G, CV, FAST, SURR, PROD, ROS, SHAPE == 4>(p, io, e);
-    else step_loop_general<MPC, G, CV, SURR, SHAPE == 5>(p, io, e);
+    if constexpr (ONE) step_loop_one<MPC, G, CV, FAST, SURR, PROD, ROS, SHAPE == 4, FIN>(p, io, e);
+    else step_loop_general<MPC, G, CV, SURR, SHAPE == 5, FIN>(p, io, e);
 #ifdef ZS_PHASE_CLOCKS
     e.ph_last = clock64();
 #endif
@@ -770,7 +784,7 @@ static void launch_sim(const ZsHandle* h, const ZsIO& io, cudaStream_t st) {
     // the standard rollout shape gets the kernel with that shape compiled in (step_loop_one)
     const bool fast = MODE == MODE_STEP && pp.mpc <= 32 && pp.A == 1 && !pp.obs_per_agent && pp.minimum_zombies == 0 &&
                       pp.obs_scope == ZS_OBS_WORLD && io.actions && io.fmt == ZS_ACTIONS_DISCRETE && io.obs && io.reward &&
-                      io.terminated && io.truncated && !io.draws && !io.agent_mask;
+                      io.terminated && io.truncated && !io.draws && !io.agent_mask && !io.final_obs;
     // ... and with the handle's game compiled in when it is an instantiated roster (only the bench game's, at 16 slots)
     const bool roster = fast && h->roster == ZS_ROSTER_BENCH && pp.mpc == 16;
     const int occ = MODE == MODE_STEP ? sh.occ : ZS_MIN_CTAS;
@@ -778,7 +792,8 @@ static void launch_sim(const ZsHandle* h, const ZsIO& io, cudaStream_t st) {
     // the standard rollout shape of a batch that one wave of producer-warp CTAs holds: observations through a third warp
     const bool prod = fast && MODE == MODE_STEP && sh.prod_smem_bytes > 0 && pp.tmpl_smem_off >= 0 && io.env_mask == nullptr;
     // SH_: 0 world scope, 1 the standard rollout shape (step launches only), 2 surroundings, 4 surroundings with the per-agent
-    // record, 5 world scope with the record and more slots than lanes (4 and 5: step launches only) (zs_sim_kernel: SHAPE)
+    // record, 5 world scope with the record and more slots than lanes, 6 / 7 world scope / surroundings with the final
+    // observation (4 to 7: step launches only) (zs_sim_kernel: SHAPE)
     // Programmatic dependent launch: the kernel's CTAs may be scheduled while the previous kernel of the stream is still
     // draining (they stage the observation template and then wait in griddepcontrol.wait for that kernel to have
     // completed, all its writes visible) — the launch latency and the ramp hide under the predecessor's tail.
@@ -792,12 +807,14 @@ static void launch_sim(const ZsHandle* h, const ZsIO& io, cudaStream_t st) {
     // rollouts lose 1-1.5 % — the early CTAs of the next launch sit on the SMs — so only short step launches ask for it)
     const bool pdl = h->use_pdl == 1 || (h->use_pdl == 2 && MODE == MODE_STEP && io.n_steps < h->short_steps);
     lc.attrs = la; lc.numAttrs = pdl ? 1 : 0;
-#define ZS_LAUNCH_R(MPC_, G_, SH_, O_, R_) cudaLaunchKernelEx(&lc, zs_sim_kernel<MODE, MPC_, G_, MODE == MODE_STEP ? (SH_) : (SH_) == 1 || (SH_) == 5 ? 0 : (SH_) == 4 ? 2 : (SH_), MODE == MODE_STEP ? (O_) : ZS_MIN_CTAS, MODE == MODE_STEP ? (R_) : 0>, pp, io)
+#define ZS_LAUNCH_R(MPC_, G_, SH_, O_, R_) cudaLaunchKernelEx(&lc, zs_sim_kernel<MODE, MPC_, G_, MODE == MODE_STEP ? (SH_) : (SH_) == 1 || (SH_) == 5 || (SH_) == 6 ? 0 : (SH_) == 4 || (SH_) == 7 ? 2 : (SH_), MODE == MODE_STEP ? (O_) : ZS_MIN_CTAS, MODE == MODE_STEP ? (R_) : 0>, pp, io)
 #define ZS_LAUNCH(MPC_, G_, SH_, O_) ZS_LAUNCH_R(MPC_, G_, SH_, O_, 0)
 #define ZS_LAUNCH_F(MPC_, G_, O_) do { if (roster) ZS_LAUNCH_R(MPC_, G_, 1, O_, (MPC_) == 16 ? ZS_ROSTER_BENCH : 0); else if (fast) ZS_LAUNCH(MPC_, G_, 1, O_); \
-                                       else if (surr && io.compact) ZS_LAUNCH(MPC_, G_, 4, O_); else if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); \
+                                       else if (surr && io.compact) ZS_LAUNCH(MPC_, G_, 4, O_); else if (surr && io.final_obs) ZS_LAUNCH(MPC_, G_, 7, O_); \
+                                       else if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); else if (io.final_obs) ZS_LAUNCH(MPC_, G_, 6, O_); \
                                        else ZS_LAUNCH(MPC_, G_, 0, O_); } while (0)
-#define ZS_LAUNCH_G(MPC_, G_, O_) do { if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); else if (io.compact) ZS_LAUNCH(MPC_, G_, 5, O_); \
+#define ZS_LAUNCH_G(MPC_, G_, O_) do { if (surr && io.final_obs) ZS_LAUNCH(MPC_, G_, 7, O_); else if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); \
+                                       else if (io.compact) ZS_LAUNCH(MPC_, G_, 5, O_); else if (io.final_obs) ZS_LAUNCH(MPC_, G_, 6, O_); \
                                        else ZS_LAUNCH(MPC_, G_, 0, O_); } while (0)
     if (prod) {
         pp.prod_off = sh.prod_off; pp.prod_cap = sh.prod_cap; pp.tmpl_smem_off = ZS_PROD_ENVS * sh.smem_per_env;
@@ -839,6 +856,10 @@ static cudaError_t set_smem_attr_step(int bytes) {
     if (e == cudaSuccess && MPC <= 32) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (MPC <= 32 ? 4 : 2), OCC>, attr, bytes);
     constexpr bool rec_g = MPC > 32 && OCC == ZS_OCC_GENERAL;  // (the only occupancy launch_sim runs them at)
     if (e == cudaSuccess && rec_g) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (rec_g ? 5 : 0), OCC>, attr, bytes);
+    // the final-observation kernels: every occupancy launch_sim runs the world-scope and surroundings kernels at
+    constexpr bool fin = MPC <= 32 || OCC == ZS_OCC_GENERAL;
+    if (e == cudaSuccess && fin) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (fin ? 6 : 0), OCC>, attr, bytes);
+    if (e == cudaSuccess && fin) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (fin ? 7 : 2), OCC>, attr, bytes);
     return e;
 }
 template <int MPC, int G>
@@ -1263,19 +1284,39 @@ extern "C" __attribute__((visibility("default"))) int zs_reset(ZsHandle* h, cons
     return launched(h);
 }
 
-extern "C" __attribute__((visibility("default"))) int zs_step(ZsHandle* h, const int32_t* actions_dev, int32_t action_format, int32_t* obs_dev, double* reward_dev,
-                       uint8_t* terminated_dev, uint8_t* truncated_dev, uint8_t* agent_mask_dev, int32_t* draws_dev, void* stream) {
+// zs_step and zs_step_final
+static int step_launch(ZsHandle* h, const char* who, const int32_t* actions_dev, int32_t action_format, int32_t* obs_dev,
+                       int32_t* final_obs_dev, double* reward_dev, uint8_t* terminated_dev, uint8_t* truncated_dev,
+                       uint8_t* agent_mask_dev, int32_t* draws_dev, void* stream) {
     if (int rc = check_bound(h)) return rc;
     DeviceGuard guard(h);
-    if (!actions_dev) return fail("zs_step needs an action tensor");
+    if (!actions_dev) return fail("%s needs an action tensor", who);
     if (action_format != ZS_ACTIONS_FULL && action_format != ZS_ACTIONS_DISCRETE) return fail("bad action format");
     ZsIO io;
     memset(&io, 0, sizeof(io));
     io.actions = actions_dev; io.fmt = action_format; io.obs = obs_dev; io.obs_slots = 1; io.reward = reward_dev;
     io.terminated = terminated_dev; io.truncated = truncated_dev; io.agent_mask = agent_mask_dev; io.draws = draws_dev;
+    io.final_obs = final_obs_dev;
     io.n_steps = 1;
     launch_sim<MODE_STEP>(h, io, (cudaStream_t)stream);
     return launched(h);
+}
+
+extern "C" __attribute__((visibility("default"))) int zs_step(ZsHandle* h, const int32_t* actions_dev, int32_t action_format, int32_t* obs_dev, double* reward_dev,
+                       uint8_t* terminated_dev, uint8_t* truncated_dev, uint8_t* agent_mask_dev, int32_t* draws_dev, void* stream) {
+    return step_launch(h, "zs_step", actions_dev, action_format, obs_dev, nullptr, reward_dev, terminated_dev, truncated_dev,
+                       agent_mask_dev, draws_dev, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int zs_step_final(ZsHandle* h, const int32_t* actions_dev, int32_t action_format, int32_t* obs_dev,
+                                                                     int32_t* final_obs_dev, double* reward_dev, uint8_t* terminated_dev,
+                                                                     uint8_t* truncated_dev, uint8_t* agent_mask_dev, int32_t* draws_dev,
+                                                                     void* stream) {
+    if (int rc = check_bound(h)) return rc;
+    if (!h->p.auto_reset) return fail("zs_step_final needs a handle with auto_reset = 1: without it no step re-initialises an env");
+    if (!obs_dev || !final_obs_dev) return fail("zs_step_final needs an observation and a final observation tensor");
+    return step_launch(h, "zs_step_final", actions_dev, action_format, obs_dev, final_obs_dev, reward_dev, terminated_dev,
+                       truncated_dev, agent_mask_dev, draws_dev, stream);
 }
 
 extern "C" __attribute__((visibility("default"))) int zs_step_masked(ZsHandle* h, const uint8_t* env_mask_dev, const int32_t* actions_dev, int32_t action_format,
@@ -1813,9 +1854,10 @@ extern "C" __attribute__((visibility("default"))) int zs_encode_obs(ZsHandle* h,
     return launched(h);
 }
 
-extern "C" __attribute__((visibility("default"))) int zs_rollout(ZsHandle* h, int32_t n_steps, int64_t first_step_index, const int32_t* actions_dev,
-                          int32_t action_format, int32_t* obs_dev, int32_t obs_slots, double* reward_dev,
-                          uint8_t* terminated_dev, uint8_t* truncated_dev, void* stream) {
+// zs_rollout and zs_rollout_final
+static int rollout_launch(ZsHandle* h, int32_t n_steps, int64_t first_step_index, const int32_t* actions_dev, int32_t action_format,
+                          int32_t* obs_dev, int32_t* final_obs_dev, int32_t obs_slots, double* reward_dev, uint8_t* terminated_dev,
+                          uint8_t* truncated_dev, void* stream) {
     if (int rc = check_bound(h)) return rc;
     DeviceGuard guard(h);
     if (n_steps < 1) return fail("n_steps must be >= 1");
@@ -1825,9 +1867,26 @@ extern "C" __attribute__((visibility("default"))) int zs_rollout(ZsHandle* h, in
     memset(&io, 0, sizeof(io));
     io.actions = actions_dev; io.fmt = action_format; io.obs = obs_dev; io.obs_slots = obs_slots; io.reward = reward_dev;
     io.terminated = terminated_dev; io.truncated = truncated_dev; io.n_steps = n_steps; io.first_step = first_step_index;
+    io.final_obs = final_obs_dev;
     io.force_auto_reset = 1;
     launch_sim<MODE_STEP>(h, io, (cudaStream_t)stream);
     return launched(h);
+}
+
+extern "C" __attribute__((visibility("default"))) int zs_rollout(ZsHandle* h, int32_t n_steps, int64_t first_step_index, const int32_t* actions_dev,
+                          int32_t action_format, int32_t* obs_dev, int32_t obs_slots, double* reward_dev,
+                          uint8_t* terminated_dev, uint8_t* truncated_dev, void* stream) {
+    return rollout_launch(h, n_steps, first_step_index, actions_dev, action_format, obs_dev, nullptr, obs_slots, reward_dev,
+                          terminated_dev, truncated_dev, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int zs_rollout_final(ZsHandle* h, int32_t n_steps, int64_t first_step_index,
+                                                                        const int32_t* actions_dev, int32_t action_format, int32_t* obs_dev,
+                                                                        int32_t* final_obs_dev, int32_t obs_slots, double* reward_dev,
+                                                                        uint8_t* terminated_dev, uint8_t* truncated_dev, void* stream) {
+    if (!obs_dev || !final_obs_dev) return fail("zs_rollout_final needs an observation and a final observation ring");
+    return rollout_launch(h, n_steps, first_step_index, actions_dev, action_format, obs_dev, final_obs_dev, obs_slots, reward_dev,
+                          terminated_dev, truncated_dev, stream);
 }
 
 extern "C" __attribute__((visibility("default"))) int zs_fill_synthetic_actions(ZsHandle* h, int64_t step_index, int32_t* actions_dev, void* stream) {

@@ -139,6 +139,10 @@ struct ZsIO {
     int32_t n_steps;
     int64_t first_step;
     int32_t force_auto_reset;
+    // [obs_slots, N, obs_elems] or NULL: the observation of the world an episode ended in, for the envs the step re-initialises
+    // (zs_step_final, zs_rollout_final; only the kernels with FIN compiled in write it).  Last, so that the fields every
+    // other kernel reads keep their parameter offsets.
+    int32_t* final_obs;
 };
 
 // weapon tables indexed by weapon code (zombsole/weapons.py:18-25); range2 = floor(max_range^2)

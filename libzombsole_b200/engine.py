@@ -165,6 +165,20 @@ class ZsEngine(object):
                              self._arg(agent_mask, self._FLAG_DTYPES, N * self.A, "agent_mask"),
                              self._arg(draws, torch.int32, N, "draws"), self._stream()))
 
+    def step_final(self, actions, fmt, obs, final_obs, reward, terminated, truncated, agent_mask=None, draws=None):
+        """zs_step_final: ``step`` that also writes, for every env whose episode the step ends (and re-initialises), the
+        observation of the world it ended in to its row of ``final_obs`` (shaped like ``obs``); the other rows are
+        unspecified.  Needs an engine built with auto_reset."""
+        N = self.N
+        check(self.L.zs_step_final(self.h, self._action_arg(actions, fmt, 1), fmt,
+                                   self._arg(obs, torch.int32, N * self.obs_elems, "obs"),
+                                   self._arg(final_obs, torch.int32, N * self.obs_elems, "final_obs"),
+                                   self._arg(reward, torch.float64, N * self.R, "reward"),
+                                   self._arg(terminated, self._FLAG_DTYPES, N, "terminated"),
+                                   self._arg(truncated, self._FLAG_DTYPES, N, "truncated"),
+                                   self._arg(agent_mask, self._FLAG_DTYPES, N * self.A, "agent_mask"),
+                                   self._arg(draws, torch.int32, N, "draws"), self._stream()))
+
     def step_masked(self, mask, actions, fmt, obs, reward, terminated, truncated, agent_mask=None):
         """zs_step_masked: one transition of the worlds selected by ``mask`` (uint8 [N]); the others are not touched."""
         N = self.N
@@ -313,14 +327,26 @@ class ZsEngine(object):
         return obs
 
     def rollout(self, n_steps, first_step_index=0, actions=None, fmt=abi.ACTIONS_DISCRETE, obs=None, reward=None,
-                terminated=None, truncated=None):
+                terminated=None, truncated=None, final_obs=None):
+        """``n_steps`` transitions in one launch with same-step auto-reset.  ``obs`` is [N, ...] or a ring [slots, N, ...];
+        step i writes slot i % slots.  ``final_obs`` (zs_rollout_final; needs ``obs``): a ring of the same shape that receives,
+        in step i's slot, the observation each env whose episode step i ended had before its re-initialisation."""
         n_steps, N = int(n_steps), self.N
         slots = 0 if obs is None else (obs.shape[0] if obs.dim() == len(self.obs_shape) + 2 else 1)
-        check(self.L.zs_rollout(self.h, n_steps, int(first_step_index), self._action_arg(actions, fmt, n_steps), fmt,
-                                self._arg(obs, torch.int32, max(1, slots) * N * self.obs_elems, "obs"), slots,
-                                self._arg(reward, torch.float64, n_steps * N * self.R, "reward"),
-                                self._arg(terminated, self._FLAG_DTYPES, n_steps * N, "terminated"),
-                                self._arg(truncated, self._FLAG_DTYPES, n_steps * N, "truncated"), self._stream()))
+        args = (self._arg(reward, torch.float64, n_steps * N * self.R, "reward"),
+                self._arg(terminated, self._FLAG_DTYPES, n_steps * N, "terminated"),
+                self._arg(truncated, self._FLAG_DTYPES, n_steps * N, "truncated"), self._stream())
+        head = (self.h, n_steps, int(first_step_index), self._action_arg(actions, fmt, n_steps), fmt,
+                self._arg(obs, torch.int32, max(1, slots) * N * self.obs_elems, "obs"))
+        if final_obs is None:
+            check(self.L.zs_rollout(*head, slots, *args))
+            return
+        if obs is None:
+            raise ValueError("final_obs needs obs: the final observations go to the slots of the observation ring")
+        if tuple(final_obs.shape) != tuple(obs.shape):
+            raise ValueError("final_obs must be shaped like obs %s, got %s" % (tuple(obs.shape), tuple(final_obs.shape)))
+        check(self.L.zs_rollout_final(*head, self._arg(final_obs, torch.int32, max(1, slots) * N * self.obs_elems, "final_obs"),
+                                      slots, *args))
 
     def fill_synthetic_actions(self, step_index, actions):
         check(self.L.zs_fill_synthetic_actions(self.h, int(step_index),

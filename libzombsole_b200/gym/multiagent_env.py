@@ -15,12 +15,12 @@ import torch
 
 from .. import abi
 from ..engine import ZsEngine
-from ..gym_env import CompactHostOutputs, encode_action
+from ..gym_env import CompactHostOutputs, FinalObservation, check_final_observation, encode_action
 from ..spaces import Box, Dict, Discrete, Text
 from ..things import Game
 
 
-class MultiagentZombsoleVectorEnv(CompactHostOutputs):
+class MultiagentZombsoleVectorEnv(CompactHostOutputs, FinalObservation):
     metadata = {"render.modes": ["human"]}
     reward_range = (-float("inf"), float("inf"))
     game_actions = [
@@ -36,12 +36,14 @@ class MultiagentZombsoleVectorEnv(CompactHostOutputs):
     def __init__(self, rules_name, player_names, map_name, agent_ids, initial_zombies=0, minimum_zombies=0,
                  render_mode=None, observation_surroundings_width=21, observation_position_encoding_style="channels",
                  agent_weapons="rifle", debug=False, *, num_envs=1, device="cuda", seed=0, env_index_base=0,
-                 max_episode_steps=None, auto_reset=True, host_outputs=False, host_threads=0, compact_words=0):
+                 max_episode_steps=None, auto_reset=True, host_outputs=False, host_threads=0, compact_words=0,
+                 final_observation=False):
         if render_mode is not None:
             if render_mode not in self.metadata["render.modes"]:
                 raise ValueError("render_mode={} is not supported".format(render_mode))
             raise NotImplementedError("rendering is outside the batched simulator's scope (render_mode=None only)")
         self.render_mode = None
+        check_final_observation(final_observation, auto_reset, host_outputs)
         width = observation_surroundings_width
         if (width % 2 == 0) or (width <= 1):  # observation.py:206-207
             raise ValueError("surroundings width must be an odd number greater than 1")
@@ -103,6 +105,7 @@ class MultiagentZombsoleVectorEnv(CompactHostOutputs):
             self._mask = torch.ones((num_envs, self.num_agents), dtype=torch.uint8, device=self.device)
             self._actions = torch.zeros((num_envs, self.num_agents, 3), dtype=torch.int32, device=self.device)
         self._h2d_done, self._h2d_pending = None, False
+        FinalObservation.__init__(self, final_observation)
 
     def game(self, env=0):
         rules_name, player_names, agent_ids, iz, mz = self._ctor
@@ -155,7 +158,10 @@ class MultiagentZombsoleVectorEnv(CompactHostOutputs):
         a, fmt = self._stage_actions(actions)
         if self.compact:
             return self._step_compact(a, fmt)
-        self.engine.step(a, fmt, self.obs, self.reward, self._term, self._trunc, self._mask)
+        if self.final_observation:
+            self.engine.step_final(a, fmt, self.obs, self.final_obs, self.reward, self._term, self._trunc, self._mask)
+        else:
+            self.engine.step(a, fmt, self.obs, self.reward, self._term, self._trunc, self._mask)
         if self.host_outputs:  # the host owns the results (and any pinned action buffer) when step() returns
             P = self.cfg.n_bots
             self.agent_life_host.copy_(self.engine.fields["life"][:, P:P + self.num_agents], non_blocking=True)
@@ -164,8 +170,10 @@ class MultiagentZombsoleVectorEnv(CompactHostOutputs):
         if self._h2d_pending:  # a pinned host action buffer is the caller's again when step() returns
             self._h2d_done.synchronize()
             self._h2d_pending = False
-        return (self.obs, self.reward, self._term.view(torch.bool), self._trunc.view(torch.bool),
-                {"agent_mask": self._mask.view(torch.bool)})  # (0/1 bytes: views, no kernels)
+        info = {"agent_mask": self._mask.view(torch.bool)}  # (0/1 bytes: views, no kernels)
+        if self.final_observation:
+            self._final_info(info)
+        return self.obs, self.reward, self._term.view(torch.bool), self._trunc.view(torch.bool), info
 
     # (CompactHostOutputs)
     def _max_words(self):
@@ -199,12 +207,14 @@ class MultiagentZombsoleVectorEnv(CompactHostOutputs):
             torch.cuda.current_stream(self.device).synchronize()
         return self.obs, {}
 
-    def rollout(self, n_steps, actions=None, first_step_index=0, obs=None, reward=None, terminated=None, truncated=None):
+    def rollout(self, n_steps, actions=None, first_step_index=0, obs=None, reward=None, terminated=None, truncated=None,
+                final_obs=None):
+        """As ZombsoleVectorEnv.rollout; ``final_obs`` is a ring shaped like ``obs``."""
         fmt = abi.ACTIONS_DISCRETE
         if actions is not None and actions.dim() == 4:
             fmt = abi.ACTIONS_FULL
         self.engine.rollout(n_steps, first_step_index, actions, fmt, self.obs if obs is None else obs, reward,
-                            terminated, truncated)
+                            terminated, truncated, final_obs=final_obs)
         return self.obs if obs is None else obs
 
     def close(self):

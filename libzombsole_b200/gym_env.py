@@ -129,7 +129,43 @@ class CompactHostOutputs(object):
         return self.obs, {}
 
 
-class ZombsoleVectorEnv(CompactHostOutputs):
+def check_final_observation(final_observation, auto_reset, host_outputs):
+    """The argument combinations final_observation=True cannot serve."""
+    if not final_observation:
+        return
+    if not auto_reset:
+        raise ValueError("final_observation=True needs auto_reset=True: without auto-reset step() returns the final "
+                         "observation itself")
+    if host_outputs in ("compact", "compact-copy"):
+        raise ValueError("final_observation=True is not available with host_outputs=%r" % (host_outputs,))
+
+
+class FinalObservation(object):
+    """final_observation=True (gymnasium's SAME_STEP autoreset): an env whose step ends its episode is re-initialised in the
+    same step and ``obs`` shows the new episode; the observation of the world it ended in goes to ``final_obs`` (shaped like
+    ``obs``, written by the step kernel in place, also into pinned host memory) and step()'s info carries it as
+    ``"final_obs"`` with the mask ``"_final_obs"`` (bool [N] = terminated | truncated).  Rows outside the mask are
+    unspecified."""
+
+    def __init__(self, final_observation):
+        self.final_observation = bool(final_observation)
+        if self.final_observation:
+            if self.host_outputs:
+                self.final_obs = torch.empty(self.obs.shape, dtype=torch.int32).pin_memory()
+            else:
+                self.final_obs = self.engine.new_obs()
+            self._final_mask = torch.zeros(self.num_envs, dtype=torch.bool, device=self._term.device)
+            if self._term.is_pinned():
+                self._final_mask = self._final_mask.pin_memory()
+
+    def _final_info(self, info):
+        torch.logical_or(self._term, self._trunc, out=self._final_mask)
+        info["final_obs"] = self.final_obs
+        info["_final_obs"] = self._final_mask
+        return info
+
+
+class ZombsoleVectorEnv(CompactHostOutputs, FinalObservation):
     """``num_envs`` independent ZombsoleGymEnv worlds on one GPU (constructor: gym_env.py:49-53)."""
 
     metadata = {"render.modes": ["human"]}
@@ -146,12 +182,14 @@ class ZombsoleVectorEnv(CompactHostOutputs):
     def __init__(self, rules_name, player_names, map_name, agent_id, initial_zombies=0, minimum_zombies=0,
                  render_mode=None, observation_scope="world", observation_position_encoding="simple",
                  agent_weapon="rifle", debug=False, *, num_envs=1, device="cuda", seed=0, env_index_base=0,
-                 max_episode_steps=None, auto_reset=True, host_outputs=False, host_threads=0, compact_words=0):
+                 max_episode_steps=None, auto_reset=True, host_outputs=False, host_threads=0, compact_words=0,
+                 final_observation=False):
         if render_mode is not None:
             if render_mode not in self.metadata["render.modes"]:
                 raise ValueError("render_mode={} is not supported".format(render_mode))
             raise NotImplementedError("rendering is outside the batched simulator's scope (render_mode=None only)")
         self.render_mode = None
+        check_final_observation(final_observation, auto_reset, host_outputs)
         scope, enc, width = abi.parse_observation_scope(observation_scope, observation_position_encoding)
         self.cfg = abi.make_config(rules_name, list(player_names), [agent_id], [agent_weapon], initial_zombies,
                                    minimum_zombies, scope, enc, width, False, num_envs, seed=seed,
@@ -178,7 +216,7 @@ class ZombsoleVectorEnv(CompactHostOutputs):
         if isinstance(host_outputs, str) and host_outputs not in ("compact", "compact-copy", "compact-if-available"):
             raise ValueError("host_outputs must be False, True, 'compact', 'compact-copy' or 'compact-if-available'")
         if host_outputs == "compact-if-available":  # (device outputs where the configuration has no compact record form)
-            host_outputs = "compact" if self.engine.compact_words() else False
+            host_outputs = "compact" if self.engine.compact_words() and not final_observation else False
         self.compact = host_outputs in ("compact", "compact-copy")
         self.streamed = host_outputs == "compact"
         self.host_outputs = bool(host_outputs)
@@ -202,6 +240,7 @@ class ZombsoleVectorEnv(CompactHostOutputs):
         self._actions = torch.zeros((num_envs, 1, 3), dtype=torch.int32, device=self.device)
         self._act_dev = torch.zeros((num_envs, 1), dtype=torch.int32, device=self.device)
         self._h2d_done, self._h2d_pending = None, False
+        FinalObservation.__init__(self, final_observation)
 
     # -- the reference's object protocol for one world of the batch
     def game(self, env=0):
@@ -256,13 +295,17 @@ class ZombsoleVectorEnv(CompactHostOutputs):
         a, fmt = self._stage_actions(actions)
         if self.compact:
             return self._step_compact(a, fmt)
-        self.engine.step(a, fmt, self.obs, self.reward, self._term, self._trunc)
+        if self.final_observation:
+            self.engine.step_final(a, fmt, self.obs, self.final_obs, self.reward, self._term, self._trunc)
+        else:
+            self.engine.step(a, fmt, self.obs, self.reward, self._term, self._trunc)
         if self._h2d_pending:  # a pinned host action buffer is the caller's again when step() returns
             self._h2d_done.synchronize()
             self._h2d_pending = False
         if self.host_outputs:
             torch.cuda.current_stream(self.device).synchronize()  # the host owns the results when step() returns
-        return self.obs, self.reward, self._term.view(torch.bool), self._trunc.view(torch.bool), {}  # (0/1 bytes: a view, no kernel)
+        info = self._final_info({}) if self.final_observation else {}
+        return self.obs, self.reward, self._term.view(torch.bool), self._trunc.view(torch.bool), info  # (0/1 bytes: a view, no kernel)
 
     # (CompactHostOutputs)
     def _max_words(self):
@@ -303,14 +346,17 @@ class ZombsoleVectorEnv(CompactHostOutputs):
             torch.cuda.current_stream(self.device).synchronize()
         return self.obs, {}
 
-    def rollout(self, n_steps, actions=None, first_step_index=0, obs=None, reward=None, terminated=None, truncated=None):
+    def rollout(self, n_steps, actions=None, first_step_index=0, obs=None, reward=None, terminated=None, truncated=None,
+                final_obs=None):
         """``n_steps`` transitions in one kernel launch with same-step auto-reset.  ``actions`` is an int32
-        tensor [n_steps, N] of discrete ids or None for the synthetic uniform stream."""
+        tensor [n_steps, N] of discrete ids or None for the synthetic uniform stream.  ``final_obs``: a ring shaped like
+        ``obs`` (or like the env's observation when ``obs`` is None) that receives, in step i's slot, the observation each env
+        whose episode step i ended had before it was re-initialised (the rows where terminated | truncated)."""
         fmt = abi.ACTIONS_DISCRETE
         if actions is not None and actions.dim() == 3 and actions.shape[-1] == 3:
             fmt = abi.ACTIONS_FULL
         self.engine.rollout(n_steps, first_step_index, actions, fmt, self.obs if obs is None else obs, reward,
-                            terminated, truncated)
+                            terminated, truncated, final_obs=final_obs)
         return self.obs if obs is None else obs
 
     def render(self):
