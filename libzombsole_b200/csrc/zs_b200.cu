@@ -1154,6 +1154,9 @@ extern "C" __attribute__((visibility("default"))) int zs_create(const ZsConfig* 
         sh.warps_per_cta = ZS_WPC;
         if ((p.N + ZS_WPC * epw - 1) / (ZS_WPC * epw) < prop.multiProcessorCount * 5) sh.warps_per_cta = 2;
         if (const char* force = getenv("ZS_WARPS_PER_CTA")) { const int v = atoi(force); if (v == 1 || v == 2 || v == 4) sh.warps_per_cta = v; }
+        // large maps: narrower CTAs (4 -> 2 -> 1 warps) when the envs of the chosen one do not fit in a CTA's shared memory
+        while (sh.warps_per_cta > 1 && (long long)sh.smem_per_env * sh.warps_per_cta * epw > (long long)prop.sharedMemPerBlockOptin)
+            sh.warps_per_cta >>= 1;
         sh.envs_per_cta = sh.warps_per_cta * epw;
         sh.smem_bytes = sh.smem_per_env * sh.envs_per_cta;
         sh.tmpl_smem_off = -1; sh.tmpl_planes = 0; sh.tmpl_pair = 0; sh.tmpl_bytes = 0;

@@ -461,7 +461,10 @@ __device__ __forceinline__ int target_of_cell(const ZsParams& p, int g, int cell
 #define X_ATTACK_S 4
 #define X_HEAL_S 5
 __device__ __forceinline__ unsigned long long pack_move(int actor, int restore, int c, int old) {
-    return (unsigned long long)(X_MOVE | (actor << 3) | (restore << 11) | (c << 16)) | ((unsigned long long)(uint32_t)old << 32);
+    // (the cell in uint32_t: on maps of 32,768 cells or more an int shift overflows, and the sign extension of the low word
+    // would overwrite the old cell in the high word)
+    return (unsigned long long)((uint32_t)(X_MOVE | (actor << 3) | (restore << 11)) | ((uint32_t)c << 16)) |
+           ((unsigned long long)(uint32_t)old << 32);
 }
 __device__ __forceinline__ unsigned long long pack_hit(int kind, int target, int r2, int lo, int n, uint32_t hi) {
     return (unsigned long long)(uint32_t)(kind | (target << 3) | (r2 << 11) | (lo << 18) | (n << 25)) | ((unsigned long long)hi << 32);
@@ -1614,7 +1617,8 @@ ZS_TPL __device__ __forceinline__ int stage_draws(const ZsParams& p, const Env& 
 // the first `count` Fisher-Yates iterations decide placements (spawns.pop() takes from the end); the rest of
 // the shuffle only advances the draw counter.  New things are appended to the dict order (rank0 + i).
 // all_free: the caller knows that nothing stands on any cell of the spawn list (a new world: spawn cells never
-// carry boxes/walls, and player and zombie spawn cells are different cells), so the list is taken as it is.
+// carry boxes/walls, and player and zombie spawn cells are different cells — as long as the players stood on player spawn
+// cells), so the list is taken as it is.
 // Returns the new draw index; the new number of things in the world is left in SCALW(ZS_S_STAMP_COUNTER).
 ZS_TPL __device__ __noinline__ int spawn_in_random(const ZsParams& p, GrpId id, int episode,
                                                    uint32_t t_word, int k, int count, int which, int rank0, bool all_free,
@@ -2045,7 +2049,9 @@ ZS_TPL __device__ __noinline__ int initialize_world(const ZsParams& p, GrpId id,
     gsync<G, CV>(e);
     k = spawn_in_random<MPC, G, false>(p, id, episode, 0u, k, p.A, 0, SCALW(ZS_S_STAMP_COUNTER), p.P == 0, true);
     PH(16);
-    k = spawn_zombies<MPC, G, false>(p, id, episode, 0u, k, p.initial_zombies, SCALW(ZS_S_STAMP_COUNTER), true, true);
+    // (the zombie spawn cells are all free unless the players, lacking spawn cells of their own, stood anywhere: on them too)
+    k = spawn_zombies<MPC, G, false>(p, id, episode, 0u, k, p.initial_zombies, SCALW(ZS_S_STAMP_COUNTER),
+                                     p.n_ps > 0 || p.P + p.A == 0, true);
     PH(17);
 #pragma unroll 1
     for (int a = e.gl; a < p.A; a += G) PREVL(a) = TL(p.P + a);

@@ -89,6 +89,67 @@ CONFIGS = {
                           surroundings_width=21),
 }
 
+
+def _edge_map(name):
+    return os.path.join(MAPS_DIR, name + ".txt")
+
+
+def _single(map_name, scope="world", enc="simple", rules="extermination", players=("terminator", "terminator"), weapon="rifle",
+            zombies=10, minimum=0):
+    return dict(kind="single", rules_name=rules, player_names=list(players), map_name=map_name, agent_ids=[0],
+                agent_weapons=weapon, initial_zombies=zombies, minimum_zombies=minimum, observation_scope=scope,
+                observation_position_encoding=enc)
+
+
+# map geometry at the edges of what zs_create accepts (tests/maps/*.txt; test_map_edges.py asserts the fact each map is for)
+CONFIGS.update({
+    # the bench game (agent + 2 terminators, extermination, rifle, 10 zombies, world/simple): with few enough spawn cells the
+    # standard rollout shape runs the roster kernel.  odd_cells: 13 x 11 = 143 cells (3 mod 4): the world observation's
+    # rows are not 16-byte aligned, so the template is copied cell by cell (no TMA template)
+    "bench_odd_cells": _single(_edge_map("odd_cells")),
+    # strip_row: 81 x 1 (height 1; 81 cells, 1 mod 4): every neighbour above or below is outside the map
+    "bench_strip_row": _single(_edge_map("strip_row")),
+    # wide_max: 2,047 x 32 = 65,504 cells, everything in rows 17-31 (cells >= 34,799) near both ends: moves, hits and
+    # closest-target searches at the largest cell indices and distances; one env needs ~75 KB of shared memory
+    "bench_wide_max": _single(_edge_map("wide_max")),
+    # world observations on a 1,533-cell stock map (1 mod 4)
+    "fort_world": _single("fort", players=["terminator"], weapon="shotgun", zombies=12),
+    # world/channels on odd_cells: three planes of 143 cells each
+    "odd_cells_channels": _single(_edge_map("odd_cells"), enc="channels", players=["sniper"], weapon="gun", zombies=8),
+    # surroundings width 3 (the narrowest window) on a 3-mod-4 map and on a map one cell high
+    "surr3_odd_cells": _single(_edge_map("odd_cells"), scope="surroundings:3", players=["terminator"], zombies=8),
+    "surr3_channels_strip_row": _single(_edge_map("strip_row"), scope="surroundings:3", enc="channels", zombies=4),
+    # surroundings width 255, far wider than the map: 260 KB (simple) / 520 KB (channels) per window.  strip_col (1 x 42)
+    # keeps the per-cell window table under its 32 MB limit (10.9 / 21.9 MB); odd_cells (143 cells: 37 / 74 MB) does not,
+    # so its windows are cut from the padded template planes
+    "surr255_strip_col": _single(_edge_map("strip_col"), scope="surroundings:255", players=["terminator"], zombies=6),
+    "surr255_channels_strip_col": _single(_edge_map("strip_col"), scope="surroundings:255", enc="channels", zombies=4),
+    "surr255_odd_cells": _single(_edge_map("odd_cells"), scope="surroundings:255", players=["terminator"], zombies=8),
+    "surr255_channels_odd_cells": _single(_edge_map("odd_cells"), scope="surroundings:255", enc="channels",
+                                          players=["sniper"], weapon="shotgun", zombies=8),
+    # multi-agent surroundings on a map one cell wide (strip_col: 1 x 42, 42 cells, 2 mod 4) and on wide_max
+    "multi_strip_col": dict(kind="multi", rules_name="extermination", player_names=["terminator"],
+                            map_name=_edge_map("strip_col"), agent_ids=["0", "1", "2"], agent_weapons=["rifle", "knife", "gun"],
+                            initial_zombies=6, minimum_zombies=0, surroundings_width=5),
+    "multi_wide_max": dict(kind="multi", rules_name="extermination", player_names=["terminator"],
+                           map_name=_edge_map("wide_max"), agent_ids=["0", "1", "2", "3"], agent_weapons="shotgun",
+                           initial_zombies=12, minimum_zombies=0, surroundings_width=9),
+    # more than 32 slots (the general kernel) on wide_max and odd_cells
+    "general_wide_max": _single(_edge_map("wide_max"), players=["terminator"], zombies=40),
+    "general_odd_cells": _single(_edge_map("odd_cells"), enc="channels", zombies=32),
+    # survival with a zombie minimum: no_player_spawns (players stand anywhere free), few_spawns (3 player spawn cells for
+    # 3 players, 4 zombie spawn cells for up to 8 zombies: the lean init is off, most respawns find no free spawn cell)
+    "minz_no_player_spawns": _single(_edge_map("no_player_spawns"), enc="channels", rules="survival", players=["terminator"],
+                                     weapon="knife", zombies=4, minimum=6),
+    "minz_few_spawns": _single(_edge_map("few_spawns"), rules="survival", players=["terminator", "sniper"], weapon="axe",
+                               zombies=6, minimum=8),
+    # crowded: no spawn cells at all and 12 things for 10 free cells (the last two zombies find no cell)
+    "crowded": _single(_edge_map("crowded"), players=["terminator"], weapon="knife", zombies=10),
+    # safehouse with its objectives on the map's last row and last column
+    "safehouse_edges": _single(_edge_map("edge_objectives"), rules="safehouse", players=["terminator"], zombies=6),
+})
+
+
 DISCRETE = [(abi.ACT_MOVE, 0, 1), (abi.ACT_MOVE, -1, 0), (abi.ACT_MOVE, 0, -1), (abi.ACT_MOVE, 1, 0),
             (abi.ACT_ATTACK_CLOSEST, 0, 0), (abi.ACT_HEAL, 0, 0), (abi.ACT_HEAL_CLOSEST, 0, 0)]
 

@@ -37,10 +37,27 @@ def _mode(monkeypatch, mode):
 @pytest.mark.parametrize("mode", MODES)
 @pytest.mark.parametrize("enc,N,threads", [("simple", 4096, 0), ("simple", 333, 3), ("channels", 1024, 0)])
 def test_compact_outputs_equal_device_outputs(monkeypatch, enc, N, threads, mode):
+    assert _compare(monkeypatch, mode, N, threads, observation_position_encoding=enc, **KW) == 0
+
+
+# maps at the edges of the accepted geometry (tests/maps): 143 cells (rows not 16-byte aligned) and 65,504 cells (record
+# cells past 32,767), with at most 32 things and with more (the general kernel's record)
+@pytest.mark.parametrize("mode", MODES)
+@pytest.mark.parametrize("name,N", [("bench_odd_cells", 512), ("bench_wide_max", 48), ("general_odd_cells", 256),
+                                    ("general_wide_max", 32)])
+def test_compact_outputs_on_edge_maps(monkeypatch, name, N, mode):
+    import parity_util as pu
+    c = pu.CONFIGS[name]
+    _compare(monkeypatch, mode, N, 0, rules_name=c["rules_name"], player_names=c["player_names"], map_name=c["map_name"],
+             agent_id=0, initial_zombies=c["initial_zombies"], minimum_zombies=c["minimum_zombies"],
+             observation_scope=c["observation_scope"], agent_weapon=c["agent_weapons"],
+             observation_position_encoding=c["observation_position_encoding"])
+
+
+def _compare(monkeypatch, mode, N, threads, **kw):
     mode = _mode(monkeypatch, mode)
-    plain = ZombsoleVectorEnv(num_envs=N, seed=9, max_episode_steps=30, observation_position_encoding=enc, **KW)
-    comp = ZombsoleVectorEnv(num_envs=N, seed=9, max_episode_steps=30, observation_position_encoding=enc,
-                             host_outputs=mode, host_threads=threads, **KW)
+    plain = ZombsoleVectorEnv(num_envs=N, seed=9, max_episode_steps=30, **kw)
+    comp = ZombsoleVectorEnv(num_envs=N, seed=9, max_episode_steps=30, host_outputs=mode, host_threads=threads, **kw)
     o0, _ = plain.reset()
     c0, _ = comp.reset()
     assert torch.equal(o0.cpu(), c0)
@@ -61,9 +78,10 @@ def test_compact_outputs_equal_device_outputs(monkeypatch, enc, N, threads, mode
             assert torch.equal(ro.cpu()[sel], rc[sel])
         if t == 55:
             assert torch.equal(plain.get_observation().cpu(), comp.get_observation())
-    assert comp.compact_overflows == 0
+    overflows = comp.compact_overflows
     plain.close()
     comp.close()
+    return overflows
 
 
 @pytest.mark.parametrize("mode", MODES)

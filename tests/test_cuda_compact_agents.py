@@ -83,6 +83,14 @@ def test_more_games(name, mode):
 
 
 @pytest.mark.parametrize("mode", MODES)
+@pytest.mark.parametrize("name,N", [("multi_strip_col", 256), ("multi_wide_max", 64)])
+def test_edge_maps(name, N, mode):
+    """Maps at the edges of the accepted geometry (tests/maps): one cell wide (every window mostly past the map edge) and
+    65,504 cells (window centres and record cells past 32,767)."""
+    _run(name, N, mode)
+
+
+@pytest.mark.parametrize("mode", MODES)
 def test_two_envs_per_warp(monkeypatch, mode):
     monkeypatch.setenv("ZS_LANES_PER_ENV", "16")
     kw = _kwargs("multi_boxed_2p")

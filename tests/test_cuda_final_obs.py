@@ -26,7 +26,7 @@ gpu = pytest.mark.gpu
 # (config, envs): the lane layouts, both encodings and scopes, 128 and 256 slots, the respawn, randoman bots
 LOCKSTEP = [("c1_bridge_ext", 512), ("c5_bridge_channels", 256), ("gym_surroundings", 256), ("surroundings_channels", 256),
             ("c3_city_evac", 128), ("c4_maze_safehouse", 64), ("fort_max_slots", 32), ("survival_minz", 128),
-            ("bots_randoman", 128)]
+            ("bots_randoman", 128), ("bench_odd_cells", 256), ("bench_wide_max", 32), ("surr255_odd_cells", 16)]
 
 
 def _twins(name, N, seed, mes):
@@ -134,7 +134,8 @@ def _rollout_vs_twin(name, N, K, seed=47, mes=9):
 @pytest.mark.parametrize("K", [1, 7, 64])
 @pytest.mark.parametrize("name,N,lanes", [("c1_bridge_ext", 1024, "16"), ("c1_bridge_ext", 1024, "32"),
                                           ("gym_surroundings", 256, "32"), ("c3_city_evac", 128, "32"),
-                                          ("c4_maze_safehouse", 48, "32")])
+                                          ("c4_maze_safehouse", 48, "32"), ("bench_odd_cells", 256, "16"),
+                                          ("bench_wide_max", 32, "32")])
 def test_rollout_final_equals_single_steps(monkeypatch, name, N, lanes, K, images):
     monkeypatch.setenv("ZS_LANES_PER_ENV", lanes)
     if not images:

@@ -80,6 +80,13 @@ CASES = [
     ("safehouse_small", 32, 120, 0), ("multi_boxed_2p", 64, 80, 0), ("multi_fort_32p", 4, 30, 0),
     ("survival_minz", 32, 120, 25), ("minz_allcells", 16, 80, 0), ("bots_mixed", 16, 60, 0), ("bots_hamsters", 32, 120, 0), ("fort_max_slots", 3, 25, 0), ("no_zombies", 16, 30, 0),
     ("bots_randoman", 64, 150, 0), ("randoman_crowd", 12, 60, 0), ("box_arena", 96, 60, 0),
+    # map geometry at the edges of what zs_create accepts (tests/maps, test_map_edges.py)
+    ("bench_odd_cells", 128, 80, 0), ("bench_strip_row", 128, 80, 0), ("bench_wide_max", 24, 60, 0), ("fort_world", 64, 60, 0),
+    ("odd_cells_channels", 96, 80, 0), ("surr3_odd_cells", 96, 80, 0), ("surr3_channels_strip_row", 96, 80, 0),
+    ("surr255_strip_col", 16, 40, 0), ("surr255_channels_strip_col", 16, 40, 0), ("surr255_odd_cells", 16, 40, 0),
+    ("surr255_channels_odd_cells", 16, 40, 0), ("multi_strip_col", 96, 80, 0), ("multi_wide_max", 16, 40, 0),
+    ("general_wide_max", 16, 40, 0), ("general_odd_cells", 96, 60, 0), ("minz_no_player_spawns", 96, 80, 0),
+    ("minz_few_spawns", 96, 80, 0), ("crowded", 96, 60, 0), ("safehouse_edges", 96, 80, 20),
 ]
 
 

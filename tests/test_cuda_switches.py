@@ -40,6 +40,16 @@ CASES = [
     # observations written by a producer warp per CTA instead of by the game warps themselves (an experiment kept correct)
     ("ZS_PRODUCER", "1", "c1_bridge_ext", 4000, 48),
     ("ZS_PRODUCER", "1", "c5_bridge_channels", 3000, 48),
+    # the same placements on the maps at the edges of the accepted geometry (tests/maps)
+    ("ZS_NO_WINDOW_TABLE", "1", "surr255_strip_col", 64, 24),
+    ("ZS_NO_WINDOW_TABLE", "1", "surr3_channels_strip_row", 256, 40),
+    ("ZS_NO_WINDOW_TABLE", "1", "multi_strip_col", 256, 40),
+    ("ZS_IMAGE_MB", "0", "bench_odd_cells", 1024, 48),
+    ("ZS_IMAGE_MB", "0", "bench_wide_max", 64, 24),
+    ("ZS_IMAGE_MB", "0", "general_odd_cells", 256, 40),
+    ("ZS_IMAGE_MB", "0", "minz_few_spawns", 256, 40),
+    ("ZS_NO_FREE_TABLE", "1", "minz_no_player_spawns", 256, 40),
+    ("ZS_NO_FREE_TABLE", "1", "crowded", 256, 40),
 ]
 
 

@@ -14,6 +14,13 @@ CASES = [
     ("village_evac_mixed", 120, 0), ("c4_maze_safehouse", 40, 0), ("safehouse_small", 150, 0),
     ("multi_boxed_2p", 120, 0), ("multi_fort_32p", 30, 0), ("survival_minz", 150, 33), ("minz_allcells", 100, 0), ("bots_mixed", 80, 0), ("bots_hamsters", 150, 0), ("fort_max_slots", 12, 0), ("no_zombies", 30, 0),
     ("box_arena", 50, 0),
+    # map geometry at the edges of what zs_create accepts (tests/maps)
+    ("bench_odd_cells", 80, 0), ("bench_strip_row", 80, 0), ("bench_wide_max", 30, 0), ("fort_world", 60, 0),
+    ("odd_cells_channels", 80, 0), ("surr3_odd_cells", 80, 0), ("surr3_channels_strip_row", 80, 0),
+    ("surr255_strip_col", 30, 0), ("surr255_channels_strip_col", 30, 0), ("surr255_odd_cells", 30, 0),
+    ("surr255_channels_odd_cells", 30, 0), ("multi_strip_col", 80, 0), ("multi_wide_max", 30, 0),
+    ("general_wide_max", 30, 0), ("general_odd_cells", 60, 0), ("minz_no_player_spawns", 80, 0), ("minz_few_spawns", 80, 0),
+    ("crowded", 60, 0), ("safehouse_edges", 80, 0),
 ]
 
 
