@@ -23,6 +23,8 @@
  *                    around gym_env.py:99-164); one launch, state stays on chip between steps
  *   zs_step_final / zs_rollout_final   zs_step / zs_rollout that also return the observation an auto-reset episode
  *                    ended with (gym_env.py:99-164)
+ *   ZS_AUTORESET_NEXT_STEP   gymnasium's NEXT_STEP autoreset around the reference's step and reset
+ *                    (gym_env.py:99-164, zombsole/gym/multiagent_env.py:111-184)
  *   zs_fill_synthetic_actions   Discrete(6|7).sample() for synthetic rollouts (gym_env.py:367)
  *   zs_step_compact_agents / zs_expand_compact_agents / zs_step_host_agents
  *                    MultiagentZombsoleEnv.step with its per-agent windows  zombsole/gym/multiagent_env.py:111-171,
@@ -107,8 +109,25 @@ typedef struct ZsConfig {
     int32_t surroundings_width;/* odd, > 1 (observation.py:185) */
     int32_t obs_per_agent;     /* 0: one observation per env (agent 0); 1: one per agent [N, A, ...] */
     int32_t max_episode_steps; /* 0 = none; gymnasium TimeLimit of the registered ids (gym_env.py:385) */
-    int32_t auto_reset;        /* 1: zs_step re-initialises an env in the same call when it ends */
+    int32_t auto_reset;        /* 0: the caller resets ended envs (zs_reset); 1: same-step autoreset, zs_step re-initialises
+                                  an env in the same call when it ends; ZS_AUTORESET_NEXT_STEP: next-step autoreset (below) */
 } ZsConfig;
+
+/* ---- next-step autoreset (ZsConfig.auto_reset = ZS_AUTORESET_NEXT_STEP; gymnasium 1.x's AutoresetMode.NEXT_STEP, the
+ * default of its vector envs)
+ * The step that ends an episode (rules, all agents dead, or the TimeLimit) is a step of an auto_reset = 0 handle: its
+ * observation, reward (with the +-10 end reward), flags, agent mask and draws, the world left as it ended, the episode
+ * counted in zs_episode_stats.  The env is then marked pending.  Its next step runs no transition and ignores its action:
+ * it performs the world init zs_reset would perform (the same draws; episode + 1; box/wall damage kept; gym_env.py:148-164,
+ * zombsole/gym/multiagent_env.py:173-184) and returns the new world's observation with reward +0.0 in every reward slot,
+ * terminated = truncated = 0, every agent in the agent mask and, as draws, the init's draw count.  That step clears the
+ * mark and does not count toward the TimeLimit.  Other envs of the launch step normally.
+ * zs_step, zs_step_masked (unselected envs stay pending), zs_rollout, zs_step_compact, zs_step_host, zs_step_compact_agents
+ * and zs_step_host_agents follow it on such a handle; zs_step_final / zs_rollout_final refuse it (the observation of the
+ * ending step already is the final observation).  zs_reset clears the marks of the envs it re-initialises, zs_bind_state
+ * and zs_init_static_life clear all of them; zs_encode_obs of a pending env shows the world it ended in.
+ * Such a handle runs one env per warp in every launch (zs_lanes_per_env = 32, whatever ZS_LANES_PER_ENV says). */
+#define ZS_AUTORESET_NEXT_STEP 2
 
 /* Layout of the caller-owned state buffer: structure-of-arrays, one row per env per field.
  * Field f of env e starts at byte  offset[f] + e * row_bytes[f]. */
@@ -217,7 +236,8 @@ int zs_step_masked(ZsHandle* h, const uint8_t* env_mask_dev, const int32_t* acti
 /* Encode the observation of the current state only. */
 int zs_encode_obs(ZsHandle* h, int32_t* obs_dev, void* stream);
 
-/* n_steps transitions in ONE launch with same-step auto-reset (regardless of cfg.auto_reset).
+/* n_steps transitions in ONE launch with same-step auto-reset (regardless of cfg.auto_reset), or with next-step autoreset on
+ * a handle created with auto_reset = ZS_AUTORESET_NEXT_STEP.
  *   actions_dev  int32 [n_steps, N, A(,3)] or NULL: discrete ids drawn in-kernel from the
  *                synthetic action stream (same values as zs_fill_synthetic_actions with
  *                step_index = first_step_index + i)
@@ -363,6 +383,10 @@ int64_t zs_launch_count(const ZsHandle* h);
 /* Lanes of a warp that work on one env on this handle: 32, or 16 (two envs per warp) for worlds of at
  * most 16 things in batches larger than one resident wave (diagnostics / tests). */
 int32_t zs_lanes_per_env(const ZsHandle* h);
+
+/* Next-step autoreset handles: *dev = the handle's marks, device uint8 [N], 1 = the env's next step is its reset step
+ * (gymnasium's _autoreset_envs).  Owned by the handle; read them on the handle's stream.  Fails on other handles. */
+int zs_autoreset_pending(const ZsHandle* h, const uint8_t** dev);
 
 #ifdef __cplusplus
 }

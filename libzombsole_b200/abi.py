@@ -23,6 +23,9 @@ ACTION_TYPES = {None: ACT_NONE, "": ACT_NONE, "move": ACT_MOVE, "attack_closest"
 ACTIONS_FULL, ACTIONS_DISCRETE = 0, 1
 OBS_WORLD, OBS_SURROUNDINGS = 0, 1
 OBS_SIMPLE, OBS_CHANNELS = 0, 1
+#: ZsConfig.auto_reset values: the caller resets, same-step autoreset, next-step autoreset (ZS_AUTORESET_NEXT_STEP)
+AUTORESET_OFF, AUTORESET_SAME_STEP, AUTORESET_NEXT_STEP = 0, 1, 2
+AUTORESET_MODES = ("same_step", "next_step")
 
 (F_X, F_Y, F_LIFE, F_STAMP, F_META, F_PREV_LIFE, F_STATIC_LIFE, F_DEAD_BODY, F_SCALARS, F_COUNT) = range(10)
 (S_T, S_EPISODE, S_DEATHS, S_ZOMBIE_DEATHS, S_STAMP_COUNTER, S_FLAGS, S_PREV_ZOMBIE_DEATHS, S_EPISODE_STEPS) = range(8)
@@ -107,6 +110,7 @@ PROTOTYPES = {
     "zs_episode_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "zs_launch_count": (C.c_int64, [C.c_void_p]),
     "zs_lanes_per_env": (C.c_int32, [C.c_void_p]),
+    "zs_autoreset_pending": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
 }
 
 
@@ -165,9 +169,20 @@ def agent_weapon_list(agent_weapons, agent_count):
                      f"name as a string or a list of weapon names.")
 
 
+def check_autoreset_mode(autoreset_mode, auto_reset=True, final_observation=False):
+    """The autoreset_mode values and the argument combinations next-step autoreset cannot serve."""
+    if autoreset_mode not in AUTORESET_MODES:
+        raise ValueError("autoreset_mode must be 'same_step' or 'next_step', got %r" % (autoreset_mode,))
+    if autoreset_mode == "next_step" and not auto_reset:
+        raise ValueError("autoreset_mode='next_step' needs auto_reset=True: without auto-reset the caller resets ended envs")
+    if autoreset_mode == "next_step" and final_observation:
+        raise ValueError("autoreset_mode='next_step' does not take final_observation=True: the observation of the step that "
+                         "ends an episode already is its final observation")
+
+
 def make_config(rules_name, player_names, agent_ids, agent_weapons, initial_zombies, minimum_zombies,
                 obs_scope, obs_encoding, surroundings_width, obs_per_agent, num_envs, seed=0, env_index_base=0,
-                max_episode_steps=0, auto_reset=False):
+                max_episode_steps=0, auto_reset=False, autoreset_mode="same_step"):
     if rules_name not in RULES:
         # zombsole/rules/factory.py:19
         raise ValueError(f"{rules_name} is not a valid rule name.  Valid options are extermination, survival, "
@@ -202,7 +217,8 @@ def make_config(rules_name, player_names, agent_ids, agent_weapons, initial_zomb
     cfg.obs_scope, cfg.obs_encoding, cfg.surroundings_width = obs_scope, obs_encoding, surroundings_width
     cfg.obs_per_agent = 1 if obs_per_agent else 0
     cfg.max_episode_steps = int(max_episode_steps or 0)
-    cfg.auto_reset = 1 if auto_reset else 0
+    check_autoreset_mode(autoreset_mode, auto_reset)
+    cfg.auto_reset = (AUTORESET_NEXT_STEP if autoreset_mode == "next_step" else AUTORESET_SAME_STEP) if auto_reset else AUTORESET_OFF
     return cfg
 
 

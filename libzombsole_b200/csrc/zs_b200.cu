@@ -59,7 +59,10 @@ __device__ __forceinline__ void compact_signal(const ZsParams& p, const ZsIO& io
 // zs_step_host), the full row only for an env the record cannot hold.
 // FIN: the final observation compiled in (zs_sim_kernel SHAPE 6 / 7): an env that the step re-initialises first writes the
 // observation of the world it ended in to its row of io.final_obs, in the ring slot of the step's own observation.
-template <int MPC, int G, bool CV, bool SURR, bool REC = false, bool FIN = false>
+// NXT: next-step autoreset compiled in (zs_sim_kernel SHAPE 8 / 9 / 11; one env per warp): an env whose step ends its episode
+// keeps the world it ended in and is marked in io.pending; its next step is the world init instead of a transition, with the
+// outputs of a new episode (reward +0.0, no flags, every agent in the mask, the init's draws).
+template <int MPC, int G, bool CV, bool SURR, bool REC = false, bool FIN = false, bool NXT = false>
 __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO& io, Env& e) {
     ZS_CONSTS; ZS_VIEWS;
     const int lane = e.gl, env = e.env;
@@ -84,6 +87,7 @@ __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO&
     };
     fetch_action(0);
     int oslot = 0;
+    bool pend = NXT && io.pending[env] != 0;
 #pragma unroll 1
     for (int step = 0; step < io.n_steps; ++step) {
         const size_t sn = (size_t)step * p.N + env;
@@ -113,48 +117,65 @@ __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO&
         gsync<G, CV>(e);
         if (step + 1 < io.n_steps) fetch_action(step + 1);
 
-        int k = world_step<MPC, G, CV>(p, e);
-        e.ep_steps += 1;
-
-        // ---- reward tracker update (reward.py:30-41, 77-92), float64 in the reference's operation order.
-        // A tracker whose inputs did not change yields exactly +0.0.
+        int k;
         int life_now[AR];
         double rew[AR];
-        int sum_prev = 0, sum_new = 0;
+        bool ended = false, won = false, agents_alive = true;
+        if (NXT && pend) {
+            // ---- the reset step of next-step autoreset: the world init zs_reset performs (gym_env.py:148-164,
+            // multiagent_env.py:173-184) instead of the transition; a new world's outputs
+            k = initialize_world<MPC, G, false>(p, id_of(e), e.episode + 1, e.flags);
+            scalars_from_smem<MPC, G, false>(p, e);
+            pend = false;
+            alive_before = 0;
 #pragma unroll
-        for (int r = 0; r < AR; ++r) {
-            const int a = lane + r * G;
-            life_now[r] = a < A ? TL(p.P + a) : 0;
-            rew[r] = 0.0;
-            if (!p.obs_per_agent) {
-                if (A > 1) { sum_prev += gadd<G, CV>(e, life_before[r]); sum_new += gadd<G, CV>(e, life_now[r]); }
-            } else if (a < A && (life_before[r] != life_now[r] || zd_before != e.zd))
-                rew[r] = __dsub_rn(total_reward(e.zd, life_now[r]), total_reward(zd_before, life_before[r]));
-        }
-        if (!p.obs_per_agent) {
-            if (A == 1) { sum_prev = life_prev0; sum_new = TL(p.P); }  // one agent: every lane reads the same two words
-            if (sum_prev != sum_new || zd_before != e.zd)
-                rew[0] = __dsub_rn(total_reward(e.zd, sum_new), total_reward(zd_before, sum_prev));
-        }
-#pragma unroll
-        for (int r = 0; r < AR; ++r) { const int a = lane + r * G; if (a < A) PREVL(a) = (int16_t)life_now[r]; }
-        e.prev_zd = e.zd;
-        gsync<G, CV>(e);
-
-        // ---- Game.spawn_zombies_to_maintain_minimum (game.py:196-201)
-        if (p.minimum_zombies > 0) {
-            int zc = 0;
-#pragma unroll 1
-            for (int s0 = NP; s0 < p.M; s0 += G) zc += __popc(gballot<G, CV>(e, s0 + lane < p.M && (TM(s0 + lane) & 0x80)));
-            if (zc < p.minimum_zombies) {
-                k = spawn_zombies<MPC, G, false>(p, id_of(e), e.episode, (uint32_t)(e.t + 1), k, p.minimum_zombies - zc, e.nlive, false, false);
-                e.nlive = SCALW(ZS_S_STAMP_COUNTER);
+            for (int r = 0; r < AR; ++r) {
+                const int a = lane + r * G;
+                life_now[r] = a < A ? TL(p.P + a) : 0;
+                rew[r] = 0.0;
+                alive_before |= gballot<G, CV>(e, a < A) << (r * G);
             }
-        }
+        } else {
+            k = world_step<MPC, G, CV>(p, e);
+            e.ep_steps += 1;
 
-        // ---- rules and end reward (gym_env.py:130-141, multiagent_env.py:143-162)
-        bool ended, won, agents_alive;
-        rules_eval<MPC, G, CV>(p, e, ended, won, agents_alive);
+            // ---- reward tracker update (reward.py:30-41, 77-92), float64 in the reference's operation order.
+            // A tracker whose inputs did not change yields exactly +0.0.
+            int sum_prev = 0, sum_new = 0;
+#pragma unroll
+            for (int r = 0; r < AR; ++r) {
+                const int a = lane + r * G;
+                life_now[r] = a < A ? TL(p.P + a) : 0;
+                rew[r] = 0.0;
+                if (!p.obs_per_agent) {
+                    if (A > 1) { sum_prev += gadd<G, CV>(e, life_before[r]); sum_new += gadd<G, CV>(e, life_now[r]); }
+                } else if (a < A && (life_before[r] != life_now[r] || zd_before != e.zd))
+                    rew[r] = __dsub_rn(total_reward(e.zd, life_now[r]), total_reward(zd_before, life_before[r]));
+            }
+            if (!p.obs_per_agent) {
+                if (A == 1) { sum_prev = life_prev0; sum_new = TL(p.P); }  // one agent: every lane reads the same two words
+                if (sum_prev != sum_new || zd_before != e.zd)
+                    rew[0] = __dsub_rn(total_reward(e.zd, sum_new), total_reward(zd_before, sum_prev));
+            }
+#pragma unroll
+            for (int r = 0; r < AR; ++r) { const int a = lane + r * G; if (a < A) PREVL(a) = (int16_t)life_now[r]; }
+            e.prev_zd = e.zd;
+            gsync<G, CV>(e);
+
+            // ---- Game.spawn_zombies_to_maintain_minimum (game.py:196-201)
+            if (p.minimum_zombies > 0) {
+                int zc = 0;
+#pragma unroll 1
+                for (int s0 = NP; s0 < p.M; s0 += G) zc += __popc(gballot<G, CV>(e, s0 + lane < p.M && (TM(s0 + lane) & 0x80)));
+                if (zc < p.minimum_zombies) {
+                    k = spawn_zombies<MPC, G, false>(p, id_of(e), e.episode, (uint32_t)(e.t + 1), k, p.minimum_zombies - zc, e.nlive, false, false);
+                    e.nlive = SCALW(ZS_S_STAMP_COUNTER);
+                }
+            }
+
+            // ---- rules and end reward (gym_env.py:130-141, multiagent_env.py:143-162)
+            rules_eval<MPC, G, CV>(p, e, ended, won, agents_alive);
+        }
         bool done = false, trunc = false;
         double end_reward = 0.0;
         if (ended) { done = true; end_reward = won ? 10.0 : -10.0; }
@@ -181,7 +202,7 @@ __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO&
         }
         if (!p.obs_per_agent && io.agent_mask && lane < A) io.agent_mask[sn * A + lane] = (alive_before >> lane) & 1u;
 
-        // ---- same-step auto-reset
+        // ---- same-step auto-reset (next-step: the world stays as it ended, its next step re-initialises it)
         if ((done || trunc) && (p.auto_reset || io.force_auto_reset)) {
             if (lane == 0) {
                 atomicAdd(p.stats + 0, 1ull);
@@ -192,9 +213,12 @@ __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO&
             // the terminal world, after the transition, the reward and the respawn: what zs_step writes without auto-reset
             // (gym_env.py:99-145)
             if constexpr (FIN) encode_obs<MPC, G, CV, SURR>(p, e, io.final_obs + (obs_out - io.obs));
-            // rare, and possibly only one env of the warp: the divergent flavour
-            initialize_world<MPC, G, false>(p, id_of(e), e.episode + 1, e.flags);
-            scalars_from_smem<MPC, G, false>(p, e);
+            if constexpr (NXT) pend = true;
+            else {
+                // rare, and possibly only one env of the warp: the divergent flavour
+                initialize_world<MPC, G, false>(p, id_of(e), e.episode + 1, e.flags);
+                scalars_from_smem<MPC, G, false>(p, e);
+            }
         }
         if constexpr (REC) {
             // the observation as a compact record with the reward and flags in its header (include/zs_b200.h: zs_step_compact),
@@ -220,6 +244,7 @@ __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO&
         }
         gsync<G, CV>(e);
     }
+    if constexpr (NXT) { if (lane == 0) io.pending[env] = pend; }
 }
 
 // ---------------------------------------------------------------- the K-step loop, one lane per slot
@@ -233,13 +258,16 @@ __device__ __forceinline__ void step_loop_general(const ZsParams& p, const ZsIO&
 // ROS: a game roster compiled in (zs_world.cuh: Roster; the standard rollout shape only), 0 = the game from ZsParams.
 // REC: surroundings scope with the per-agent compact record compiled in (zs_sim_kernel SHAPE 4).
 // FIN: the final observation compiled in (zs_sim_kernel SHAPE 6 / 7, as for step_loop_general).
-template <int MPC, int G, bool CV, bool FAST, bool SURR, bool PROD = false, int ROS = 0, bool REC = false, bool FIN = false>
+// NXT: next-step autoreset compiled in (zs_sim_kernel SHAPE 8 / 9 / 10, one env per warp; as for step_loop_general).
+template <int MPC, int G, bool CV, bool FAST, bool SURR, bool PROD = false, int ROS = 0, bool REC = false, bool FIN = false,
+          bool NXT = false>
 __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io, Env& e) {
     ZS_CONSTS; ZS_VIEWS;
     const int lane = e.gl, env = e.env;
     ObsMail* const mail = PROD ? reinterpret_cast<ObsMail*>(zs_smem + p.prod_off + (int)(e.b / (uint32_t)p.smem_per_env) * ((int)sizeof(ObsMail) + 8 * p.prod_cap)) : nullptr;
     using R = Roster<ROS>;
     static_assert(!R::on || (FAST && !PROD), "rosters are compiled into the standard rollout shape");
+    static_assert(!NXT || (G == 32 && !FAST && !FIN), "next-step autoreset runs one env per warp, in the generic shapes");
     const int A = FAST ? 1 : p.A, P = R::on ? R::P : p.P, NP = P + A;
     const int aidx = lane - P;
     const bool is_agent = aidx >= 0 && aidx < A;
@@ -265,6 +293,7 @@ __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io,
     int32_t* obs_cur = obs_first;
     int oslot = 0;
     size_t sn = env;  // step * N + env
+    bool pend = NXT && io.pending[env] != 0;
 #pragma unroll 1
     for (int step = 0; step < io.n_steps; ++step, sn += p.N) {
         TR_STEP_BEGIN();
@@ -290,35 +319,50 @@ __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io,
         PH(19);
         PH(0);
 
-        int k = world_step_one<MPC, G, CV, ROS>(p, e, my_at, my_dx, my_dy);
-        e.ep_steps += 1;
-        if (step == io.n_steps - 1) TR(25);
-
-        // ---- reward tracker update (reward.py:30-41, 77-92), float64 in the reference's operation order.
-        // A tracker whose inputs did not change yields exactly +0.0.
-        const int life_now = is_agent ? (int)TL(lane) : 0;
+        int k, life_now;
         double rew = 0.0;
-        if (lane_sum) {
-            const int sum_prev = gadd<G, CV>(e, life_before), sum_new = gadd<G, CV>(e, life_now);
-            if (sum_prev != sum_new || zd_before != e.zd) rew = __dsub_rn(total_reward(e.zd, sum_new), total_reward(zd_before, sum_prev));
-        } else if (is_agent && (life_before != life_now || zd_before != e.zd)) {
-            rew = __dsub_rn(total_reward(e.zd, life_now), total_reward(zd_before, life_before));
-        }
-        if (is_agent) PREVL(aidx) = (int16_t)life_now;
-        e.prev_zd = e.zd;
-
-        // ---- Game.spawn_zombies_to_maintain_minimum (game.py:196-201)
-        if (!FAST && p.minimum_zombies > 0) {
-            const int zc = __popc(gballot<G, CV>(e, lane >= NP && lane < p.M && (TM(lane < p.M ? lane : 0) & 0x80)));
-            if (zc < p.minimum_zombies) {  // rare, and possibly only one env of the warp: the divergent flavour
-                k = spawn_zombies<MPC, G, false>(p, id_of(e), e.episode, (uint32_t)(e.t + 1), k, p.minimum_zombies - zc, e.nlive, false, false);
-                e.nlive = SCALW(ZS_S_STAMP_COUNTER);
+        bool ended = false, won = false, agents_alive = true;
+        if (NXT && pend) {
+            // ---- the reset step of next-step autoreset: the world init zs_reset performs (gym_env.py:148-164,
+            // multiagent_env.py:173-184) instead of the transition; a new world's outputs.  (One env per warp: the branch is
+            // warp-uniform.)
+            if (p.fast_init) k = initialize_world_fast<MPC, G, CV>(p, e, true);
+            else {
+                k = initialize_world<MPC, G, false>(p, id_of(e), e.episode + 1, e.flags);
+                scalars_from_smem<MPC, G, false>(p, e);
             }
-        }
+            pend = false;
+            life_now = is_agent ? (int)TL(lane) : 0;
+            if (want_mask) alive_before = gballot<G, CV>(e, is_agent) >> P;
+        } else {
+            k = world_step_one<MPC, G, CV, ROS>(p, e, my_at, my_dx, my_dy);
+            e.ep_steps += 1;
+            if (step == io.n_steps - 1) TR(25);
 
-        // ---- rules and end reward (gym_env.py:130-141, multiagent_env.py:143-162)
-        bool ended, won, agents_alive;
-        rules_eval<MPC, G, CV, ROS>(p, e, ended, won, agents_alive);
+            // ---- reward tracker update (reward.py:30-41, 77-92), float64 in the reference's operation order.
+            // A tracker whose inputs did not change yields exactly +0.0.
+            life_now = is_agent ? (int)TL(lane) : 0;
+            if (lane_sum) {
+                const int sum_prev = gadd<G, CV>(e, life_before), sum_new = gadd<G, CV>(e, life_now);
+                if (sum_prev != sum_new || zd_before != e.zd) rew = __dsub_rn(total_reward(e.zd, sum_new), total_reward(zd_before, sum_prev));
+            } else if (is_agent && (life_before != life_now || zd_before != e.zd)) {
+                rew = __dsub_rn(total_reward(e.zd, life_now), total_reward(zd_before, life_before));
+            }
+            if (is_agent) PREVL(aidx) = (int16_t)life_now;
+            e.prev_zd = e.zd;
+
+            // ---- Game.spawn_zombies_to_maintain_minimum (game.py:196-201)
+            if (!FAST && p.minimum_zombies > 0) {
+                const int zc = __popc(gballot<G, CV>(e, lane >= NP && lane < p.M && (TM(lane < p.M ? lane : 0) & 0x80)));
+                if (zc < p.minimum_zombies) {  // rare, and possibly only one env of the warp: the divergent flavour
+                    k = spawn_zombies<MPC, G, false>(p, id_of(e), e.episode, (uint32_t)(e.t + 1), k, p.minimum_zombies - zc, e.nlive, false, false);
+                    e.nlive = SCALW(ZS_S_STAMP_COUNTER);
+                }
+            }
+
+            // ---- rules and end reward (gym_env.py:130-141, multiagent_env.py:143-162)
+            rules_eval<MPC, G, CV, ROS>(p, e, ended, won, agents_alive);
+        }
         bool done = false, trunc = false;
         double end_reward = 0.0;
         if (ended) { done = true; end_reward = won ? 10.0 : -10.0; }
@@ -356,7 +400,8 @@ __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io,
             // (gym_env.py:99-145).  The encoders are group-collective, so both envs of a warp write their row: the row of an
             // env that did not end is not flagged to the caller.
             if constexpr (FIN) encode_obs<MPC, G, CV, SURR>(p, e, io.final_obs + (obs_out - io.obs));
-            if (R::on || p.fast_init) initialize_world_fast<MPC, G, CV, ROS>(p, e, need_init);  // both envs of the warp, converged
+            if constexpr (NXT) pend = true;  // next-step autoreset: the world stays as it ended, its next step re-initialises it
+            else if (R::on || p.fast_init) initialize_world_fast<MPC, G, CV, ROS>(p, e, need_init);  // both envs of the warp, converged
             else if (need_init) {  // possibly only one env of the warp: the divergent flavour
                 initialize_world<MPC, G, false>(p, id_of(e), e.episode + 1, e.flags);
                 scalars_from_smem<MPC, G, false>(p, e);
@@ -421,6 +466,7 @@ __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io,
         if (step < 16) TR(4 + step);
         TR_STEP_END(step);
     }
+    if constexpr (NXT) { if (lane == 0) io.pending[env] = pend; }
 #ifdef ZS_PHASE_CLOCKS
     if (blockIdx.x == 0 && threadIdx.x == 0) {
         unsigned long long tot = 0;
@@ -450,13 +496,18 @@ __device__ __forceinline__ void step_loop_one(const ZsParams& p, const ZsIO& io,
 // SHAPE 6 / 7 = world-scope / surroundings observation with the final observation of every env the step re-initialises
 // (zs_step_final / zs_rollout_final; step launches only): kernels of their own, so that the kernels without it stay as they
 // are (the record of SHAPE 4 compiled into SHAPE 2 made it spill more and slowed config 3 by 6 %).
+// SHAPE 8 / 9 / 10 / 11 = next-step autoreset (ZS_AUTORESET_NEXT_STEP handles, one env per warp; step launches only): the
+// counterparts of SHAPE 0 (world scope, with its run-time compact-record branch), 2 (surroundings), 4 (surroundings with the
+// per-agent record) and 5 (world scope with the record, more slots than lanes), so that the kernels of the other handles
+// stay as they are.
 // ROS: the game roster compiled into a standard-rollout-shape kernel (zs_world.cuh: Roster), 0 = read from ZsParams.
 template <int MODE, int MPC, int G, int SHAPE, int OCC, int ROS = 0>
 __global__ void __launch_bounds__(SHAPE == 3 ? 160 : ZS_WPC * 32, OCC) zs_sim_kernel(const __grid_constant__ ZsParams p, const __grid_constant__ ZsIO io) {
     ZS_CONSTS;
     constexpr bool PROD = SHAPE == 3;
-    constexpr bool FAST = SHAPE == 1 || PROD, SURR = SHAPE == 2 || SHAPE == 4 || SHAPE == 7;
+    constexpr bool FAST = SHAPE == 1 || PROD, SURR = SHAPE == 2 || SHAPE == 4 || SHAPE == 7 || SHAPE == 9 || SHAPE == 10;
     constexpr bool FIN = SHAPE == 6 || SHAPE == 7;
+    constexpr bool NXT = SHAPE >= 8;
     // the step kernel keeps both envs of a warp converged (zs_device.cuh); masked resets and encodes may not
     constexpr bool CV = MODE == MODE_STEP;
     constexpr int EPW = 32 / G;  // envs per warp
@@ -562,8 +613,8 @@ __global__ void __launch_bounds__(SHAPE == 3 ? 160 : ZS_WPC * 32, OCC) zs_sim_ke
 #ifdef ZS_PHASE_CLOCKS
     e.ph_last = clock64();
 #endif
-    if constexpr (ONE) step_loop_one<MPC, G, CV, FAST, SURR, PROD, ROS, SHAPE == 4, FIN>(p, io, e);
-    else step_loop_general<MPC, G, CV, SURR, SHAPE == 5, FIN>(p, io, e);
+    if constexpr (ONE) step_loop_one<MPC, G, CV, FAST, SURR, PROD, ROS, SHAPE == 4 || SHAPE == 10, FIN, NXT>(p, io, e);
+    else step_loop_general<MPC, G, CV, SURR, SHAPE == 5 || SHAPE == 11, FIN, NXT>(p, io, e);
 #ifdef ZS_PHASE_CLOCKS
     e.ph_last = clock64();
 #endif
@@ -604,6 +655,12 @@ __global__ void zs_fill_actions_kernel(const __grid_constant__ ZsParams p, uint3
         const int env = r / p.A, a = r - env * p.A;
         actions[i] = synthetic_action(p, p.env_base + (uint32_t)env, step_index + (uint32_t)step, a);
     }
+}
+
+// next-step autoreset: the envs zs_reset re-initialises (env_mask NULL = all) have no reset step pending any more
+__global__ void zs_clear_pending_kernel(uint8_t* pending, const uint8_t* env_mask, int n) {
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        if (env_mask == nullptr || env_mask[i]) pending[i] = 0;
 }
 
 __global__ void zs_stats_kernel(unsigned long long* stats, int64_t* out, int reset) {
@@ -671,6 +728,7 @@ struct ZsHandle {
     int tmpl_single_step;  // launches of fewer than four steps stage the observation template for the TMA as well
     int roster;            // the game as a roster (zs_world.cuh: Roster) when the standard rollout kernel has it compiled in, else 0
     bool img_valid;  // the parked images (ZsParams::img) match the canonical state of every env
+    uint8_t* pending = nullptr;  // next-step autoreset handles only: device uint8 [N], ZsIO::pending
 };
 
 // Makes the handle's device current for the duration of an entry point and puts the caller's back afterwards: the
@@ -765,7 +823,9 @@ extern "C" __attribute__((visibility("default"))) int zs_layout(const ZsConfig* 
 }
 
 template <int MODE>
-static void launch_sim(const ZsHandle* h, const ZsIO& io, cudaStream_t st) {
+static void launch_sim(const ZsHandle* h, const ZsIO& io_in, cudaStream_t st) {
+    ZsIO io = io_in;
+    io.pending = h->pending;
     // staging the observation template for the TMA pays off when a launch runs several steps
     ZsParams pp = h->p;
     const ZsHandle::Shape& sh = h->shape[(MODE == MODE_STEP && io.n_steps >= h->short_steps && io.env_mask == nullptr) ? 0 : 1];
@@ -781,10 +841,12 @@ static void launch_sim(const ZsHandle* h, const ZsIO& io, cudaStream_t st) {
     // start from the parked images when they are current; a launch that goes through every env leaves them current
     pp.img_load = pp.img != nullptr && h->img_valid;
     const dim3 grid((pp.N + sh.envs_per_cta - 1) / sh.envs_per_cta), block(sh.warps_per_cta * 32);
+    // next-step autoreset handles step with the kernels that have it compiled in (zs_sim_kernel: SHAPE 8 to 11)
+    const bool next_step = MODE == MODE_STEP && h->pending != nullptr;
     // the standard rollout shape gets the kernel with that shape compiled in (step_loop_one)
     const bool fast = MODE == MODE_STEP && pp.mpc <= 32 && pp.A == 1 && !pp.obs_per_agent && pp.minimum_zombies == 0 &&
                       pp.obs_scope == ZS_OBS_WORLD && io.actions && io.fmt == ZS_ACTIONS_DISCRETE && io.obs && io.reward &&
-                      io.terminated && io.truncated && !io.draws && !io.agent_mask && !io.final_obs;
+                      io.terminated && io.truncated && !io.draws && !io.agent_mask && !io.final_obs && !next_step;
     // ... and with the handle's game compiled in when it is an instantiated roster (only the bench game's, at 16 slots)
     const bool roster = fast && h->roster == ZS_ROSTER_BENCH && pp.mpc == 16;
     const int occ = MODE == MODE_STEP ? sh.occ : ZS_MIN_CTAS;
@@ -793,7 +855,8 @@ static void launch_sim(const ZsHandle* h, const ZsIO& io, cudaStream_t st) {
     const bool prod = fast && MODE == MODE_STEP && sh.prod_smem_bytes > 0 && pp.tmpl_smem_off >= 0 && io.env_mask == nullptr;
     // SH_: 0 world scope, 1 the standard rollout shape (step launches only), 2 surroundings, 4 surroundings with the per-agent
     // record, 5 world scope with the record and more slots than lanes, 6 / 7 world scope / surroundings with the final
-    // observation (4 to 7: step launches only) (zs_sim_kernel: SHAPE)
+    // observation, 8 to 11 next-step autoreset (one env per warp: compiled for G = 32 only) (4 to 11: step launches only)
+    // (zs_sim_kernel: SHAPE)
     // Programmatic dependent launch: the kernel's CTAs may be scheduled while the previous kernel of the stream is still
     // draining (they stage the observation template and then wait in griddepcontrol.wait for that kernel to have
     // completed, all its writes visible) — the launch latency and the ramp hide under the predecessor's tail.
@@ -807,13 +870,18 @@ static void launch_sim(const ZsHandle* h, const ZsIO& io, cudaStream_t st) {
     // rollouts lose 1-1.5 % — the early CTAs of the next launch sit on the SMs — so only short step launches ask for it)
     const bool pdl = h->use_pdl == 1 || (h->use_pdl == 2 && MODE == MODE_STEP && io.n_steps < h->short_steps);
     lc.attrs = la; lc.numAttrs = pdl ? 1 : 0;
-#define ZS_LAUNCH_R(MPC_, G_, SH_, O_, R_) cudaLaunchKernelEx(&lc, zs_sim_kernel<MODE, MPC_, G_, MODE == MODE_STEP ? (SH_) : (SH_) == 1 || (SH_) == 5 || (SH_) == 6 ? 0 : (SH_) == 4 || (SH_) == 7 ? 2 : (SH_), MODE == MODE_STEP ? (O_) : ZS_MIN_CTAS, MODE == MODE_STEP ? (R_) : 0>, pp, io)
+#define ZS_LAUNCH_R(MPC_, G_, SH_, O_, R_) cudaLaunchKernelEx(&lc, zs_sim_kernel<MODE, MPC_, G_, MODE == MODE_STEP ? (SH_) : (SH_) == 1 || (SH_) == 5 || (SH_) == 6 || (SH_) == 8 || (SH_) == 11 ? 0 : (SH_) == 4 || (SH_) == 7 || (SH_) == 9 || (SH_) == 10 ? 2 : (SH_), MODE == MODE_STEP ? (O_) : ZS_MIN_CTAS, MODE == MODE_STEP ? (R_) : 0>, pp, io)
 #define ZS_LAUNCH(MPC_, G_, SH_, O_) ZS_LAUNCH_R(MPC_, G_, SH_, O_, 0)
-#define ZS_LAUNCH_F(MPC_, G_, O_) do { if (roster) ZS_LAUNCH_R(MPC_, G_, 1, O_, (MPC_) == 16 ? ZS_ROSTER_BENCH : 0); else if (fast) ZS_LAUNCH(MPC_, G_, 1, O_); \
+#define ZS_LAUNCH_F(MPC_, G_, O_) do { if (next_step && (G_) == 32) { if (surr && io.compact) ZS_LAUNCH(MPC_, G_, ((G_) == 32 ? 10 : 4), O_); \
+                                                                      else if (surr) ZS_LAUNCH(MPC_, G_, ((G_) == 32 ? 9 : 2), O_); \
+                                                                      else ZS_LAUNCH(MPC_, G_, ((G_) == 32 ? 8 : 0), O_); } \
+                                       else if (roster) ZS_LAUNCH_R(MPC_, G_, 1, O_, (MPC_) == 16 ? ZS_ROSTER_BENCH : 0); else if (fast) ZS_LAUNCH(MPC_, G_, 1, O_); \
                                        else if (surr && io.compact) ZS_LAUNCH(MPC_, G_, 4, O_); else if (surr && io.final_obs) ZS_LAUNCH(MPC_, G_, 7, O_); \
                                        else if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); else if (io.final_obs) ZS_LAUNCH(MPC_, G_, 6, O_); \
                                        else ZS_LAUNCH(MPC_, G_, 0, O_); } while (0)
-#define ZS_LAUNCH_G(MPC_, G_, O_) do { if (surr && io.final_obs) ZS_LAUNCH(MPC_, G_, 7, O_); else if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); \
+#define ZS_LAUNCH_G(MPC_, G_, O_) do { if (next_step) { if (surr) ZS_LAUNCH(MPC_, G_, 9, O_); else if (io.compact) ZS_LAUNCH(MPC_, G_, 11, O_); \
+                                                        else ZS_LAUNCH(MPC_, G_, 8, O_); } \
+                                       else if (surr && io.final_obs) ZS_LAUNCH(MPC_, G_, 7, O_); else if (surr) ZS_LAUNCH(MPC_, G_, 2, O_); \
                                        else if (io.compact) ZS_LAUNCH(MPC_, G_, 5, O_); else if (io.final_obs) ZS_LAUNCH(MPC_, G_, 6, O_); \
                                        else ZS_LAUNCH(MPC_, G_, 0, O_); } while (0)
     if (prod) {
@@ -860,6 +928,11 @@ static cudaError_t set_smem_attr_step(int bytes) {
     constexpr bool fin = MPC <= 32 || OCC == ZS_OCC_GENERAL;
     if (e == cudaSuccess && fin) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (fin ? 6 : 0), OCC>, attr, bytes);
     if (e == cudaSuccess && fin) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (fin ? 7 : 2), OCC>, attr, bytes);
+    // the next-step autoreset kernels: one env per warp, at the same occupancies
+    constexpr bool nxt = fin && G == 32;
+    if (e == cudaSuccess && nxt) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (nxt ? 8 : 0), OCC>, attr, bytes);
+    if (e == cudaSuccess && nxt) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (nxt ? 9 : 2), OCC>, attr, bytes);
+    if (e == cudaSuccess && nxt) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, MPC, G, (!nxt ? 2 : MPC <= 32 ? 10 : 11), OCC>, attr, bytes);
     return e;
 }
 template <int MPC, int G>
@@ -1117,6 +1190,16 @@ extern "C" __attribute__((visibility("default"))) int zs_create(const ZsConfig* 
         const int v = atoi(force);
         if ((v == 16 && p.mpc == 16 && p.N % 2 == 0) || v == 32) lanes0 = lanes1 = v;
     }
+    // next-step autoreset: an env's reset step skips the transition its partner in a two-env warp would run, which the step
+    // loop's converged primitives cannot do per half warp: one env per warp in every launch
+    if (cfg->auto_reset == ZS_AUTORESET_NEXT_STEP) {
+        lanes0 = lanes1 = 32;
+        void* d = nullptr;
+        if (cudaMalloc(&d, (size_t)p.N) != cudaSuccess) { zs_destroy(h); return fail("out of device memory (autoreset marks)"); }
+        h->dev_allocs.push_back(d);
+        if (cudaMemset(d, 0, (size_t)p.N) != cudaSuccess) { zs_destroy(h); return fail("autoreset marks: cudaMemset failed"); }
+        h->pending = (uint8_t*)d;
+    }
     h->short_steps = 8;
     h->use_pdl = 2;  // programmatic dependent launch: 2 = short step launches only (launch_sim), ZS_PDL=1 every launch, ZS_PDL=0 none
     if (const char* force = getenv("ZS_PDL")) h->use_pdl = atoi(force) ? 1 : 0;
@@ -1248,6 +1331,10 @@ extern "C" __attribute__((visibility("default"))) int zs_bind_state(ZsHandle* h,
     p.SCAL = (int32_t*)(b + h->lay.offset[ZS_F_SCALARS]);
     h->bound_bytes = bytes;
     h->img_valid = false;
+    if (h->pending) {  // (a new state: no env has a reset step pending)
+        DeviceGuard guard(h);
+        CU(cudaMemset(h->pending, 0, (size_t)p.N));
+    }
     return 0;
 }
 
@@ -1273,6 +1360,7 @@ extern "C" __attribute__((visibility("default"))) int zs_init_static_life(ZsHand
     if (int rc = check_bound(h)) return rc;
     DeviceGuard guard(h);
     h->img_valid = false;
+    if (h->pending) CU(cudaMemsetAsync(h->pending, 0, (size_t)h->p.N, (cudaStream_t)stream));
     zs_init_static_life_kernel<<<h->sm_count * 4, 256, 0, (cudaStream_t)stream>>>(h->p);
     return launched(h);
 }
@@ -1284,6 +1372,10 @@ extern "C" __attribute__((visibility("default"))) int zs_reset(ZsHandle* h, cons
     memset(&io, 0, sizeof(io));
     io.env_mask = env_mask_dev; io.obs = obs_dev; io.obs_slots = 1; io.draws = draws_dev;
     launch_sim<MODE_RESET>(h, io, (cudaStream_t)stream);
+    if (h->pending) {
+        if (int rc = launched(h)) return rc;
+        zs_clear_pending_kernel<<<(h->p.N + 255) / 256, 256, 0, (cudaStream_t)stream>>>(h->pending, env_mask_dev, h->p.N);
+    }
     return launched(h);
 }
 
@@ -1317,6 +1409,7 @@ extern "C" __attribute__((visibility("default"))) int zs_step_final(ZsHandle* h,
                                                                      void* stream) {
     if (int rc = check_bound(h)) return rc;
     if (!h->p.auto_reset) return fail("zs_step_final needs a handle with auto_reset = 1: without it no step re-initialises an env");
+    if (h->pending) return fail("zs_step_final needs a handle with auto_reset = 1: under next-step autoreset the observation of the step that ends an episode already is its final observation");
     if (!obs_dev || !final_obs_dev) return fail("zs_step_final needs an observation and a final observation tensor");
     return step_launch(h, "zs_step_final", actions_dev, action_format, obs_dev, final_obs_dev, reward_dev, terminated_dev,
                        truncated_dev, agent_mask_dev, draws_dev, stream);
@@ -1857,7 +1950,8 @@ extern "C" __attribute__((visibility("default"))) int zs_encode_obs(ZsHandle* h,
     return launched(h);
 }
 
-// zs_rollout and zs_rollout_final
+// zs_rollout and zs_rollout_final: auto-reset whatever cfg.auto_reset says — same-step, or next-step on a handle created for it
+// (the kernels of those handles have it compiled in, launch_sim)
 static int rollout_launch(ZsHandle* h, int32_t n_steps, int64_t first_step_index, const int32_t* actions_dev, int32_t action_format,
                           int32_t* obs_dev, int32_t* final_obs_dev, int32_t obs_slots, double* reward_dev, uint8_t* terminated_dev,
                           uint8_t* truncated_dev, void* stream) {
@@ -1887,6 +1981,7 @@ extern "C" __attribute__((visibility("default"))) int zs_rollout_final(ZsHandle*
                                                                         const int32_t* actions_dev, int32_t action_format, int32_t* obs_dev,
                                                                         int32_t* final_obs_dev, int32_t obs_slots, double* reward_dev,
                                                                         uint8_t* terminated_dev, uint8_t* truncated_dev, void* stream) {
+    if (h && h->pending) return fail("zs_rollout_final needs a handle with auto_reset = 0 or 1: under next-step autoreset the observation of the step that ends an episode already is its final observation");
     if (!obs_dev || !final_obs_dev) return fail("zs_rollout_final needs an observation and a final observation ring");
     return rollout_launch(h, n_steps, first_step_index, actions_dev, action_format, obs_dev, final_obs_dev, obs_slots, reward_dev,
                           terminated_dev, truncated_dev, stream);
@@ -1935,3 +2030,8 @@ extern "C" __attribute__((visibility("default"))) int zs_debug_trace(unsigned lo
 
 extern "C" __attribute__((visibility("default"))) int64_t zs_launch_count(const ZsHandle* h) { return h ? h->launches : 0; }
 extern "C" __attribute__((visibility("default"))) int32_t zs_lanes_per_env(const ZsHandle* h) { return h ? h->shape[0].lanes_per_env : 0; }
+extern "C" __attribute__((visibility("default"))) int zs_autoreset_pending(const ZsHandle* h, const uint8_t** dev) {
+    if (!h || !dev) return fail("null argument");
+    *dev = h->pending;
+    return h->pending ? 0 : fail("the handle has no next-step autoreset (auto_reset = ZS_AUTORESET_NEXT_STEP)");
+}

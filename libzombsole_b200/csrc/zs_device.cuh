@@ -143,6 +143,9 @@ struct ZsIO {
     // (zs_step_final, zs_rollout_final; only the kernels with FIN compiled in write it).  Last, so that the fields every
     // other kernel reads keep their parameter offsets.
     int32_t* final_obs;
+    // [N] next-step autoreset (ZS_AUTORESET_NEXT_STEP): 1 = the env's episode has ended and its next step re-initialises it.
+    // Handle-owned; only the kernels with NXT compiled in read or write it.  After final_obs for the same reason.
+    uint8_t* pending;
 };
 
 // weapon tables indexed by weapon code (zombsole/weapons.py:18-25); range2 = floor(max_range^2)

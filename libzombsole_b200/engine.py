@@ -370,3 +370,16 @@ class ZsEngine(object):
 
     def lanes_per_env(self):
         return int(self.L.zs_lanes_per_env(self.h))
+
+    def autoreset_pending(self):
+        """Next-step autoreset engines (zs_autoreset_pending): the handle's marks as a bool [N] device tensor, True = the env's
+        episode has ended and its next step re-initialises it (gymnasium's ``_autoreset_envs``).  A view of memory the library
+        owns and writes, valid while the engine is open: read it, do not write it.  Raises on other engines."""
+        if getattr(self, "_pending", None) is None:
+            ptr = C.c_void_p()
+            check(self.L.zs_autoreset_pending(self.h, C.byref(ptr)))
+
+            class _Marks(object):
+                __cuda_array_interface__ = dict(shape=(self.N,), typestr="|u1", data=(ptr.value, False), version=3, strides=None)
+            self._pending = torch.as_tensor(_Marks(), device=self.device).view(torch.bool)
+        return self._pending

@@ -15,12 +15,12 @@ import torch
 
 from .. import abi
 from ..engine import ZsEngine
-from ..gym_env import CompactHostOutputs, FinalObservation, check_final_observation, encode_action
+from ..gym_env import CompactHostOutputs, FinalObservation, NextStepAutoreset, check_final_observation, encode_action
 from ..spaces import Box, Dict, Discrete, Text
 from ..things import Game
 
 
-class MultiagentZombsoleVectorEnv(CompactHostOutputs, FinalObservation):
+class MultiagentZombsoleVectorEnv(CompactHostOutputs, FinalObservation, NextStepAutoreset):
     metadata = {"render.modes": ["human"]}
     reward_range = (-float("inf"), float("inf"))
     game_actions = [
@@ -37,13 +37,14 @@ class MultiagentZombsoleVectorEnv(CompactHostOutputs, FinalObservation):
                  render_mode=None, observation_surroundings_width=21, observation_position_encoding_style="channels",
                  agent_weapons="rifle", debug=False, *, num_envs=1, device="cuda", seed=0, env_index_base=0,
                  max_episode_steps=None, auto_reset=True, host_outputs=False, host_threads=0, compact_words=0,
-                 final_observation=False):
+                 final_observation=False, autoreset_mode="same_step"):
         if render_mode is not None:
             if render_mode not in self.metadata["render.modes"]:
                 raise ValueError("render_mode={} is not supported".format(render_mode))
             raise NotImplementedError("rendering is outside the batched simulator's scope (render_mode=None only)")
         self.render_mode = None
         check_final_observation(final_observation, auto_reset, host_outputs)
+        abi.check_autoreset_mode(autoreset_mode, auto_reset, final_observation)
         width = observation_surroundings_width
         if (width % 2 == 0) or (width <= 1):  # observation.py:206-207
             raise ValueError("surroundings width must be an odd number greater than 1")
@@ -60,7 +61,7 @@ class MultiagentZombsoleVectorEnv(CompactHostOutputs, FinalObservation):
         self.cfg = abi.make_config(rules_name, list(player_names), list(agent_ids), agent_weapons, initial_zombies,
                                    minimum_zombies, abi.OBS_SURROUNDINGS, abi.OBS_CHANNELS, width, True, num_envs,
                                    seed=seed, env_index_base=env_index_base, max_episode_steps=max_episode_steps,
-                                   auto_reset=auto_reset)
+                                   auto_reset=auto_reset, autoreset_mode=autoreset_mode)
         self.engine = ZsEngine(self.cfg, map_name, device=device)
         self.num_envs = num_envs
         self.num_agents = len(agent_ids)
@@ -106,6 +107,7 @@ class MultiagentZombsoleVectorEnv(CompactHostOutputs, FinalObservation):
             self._actions = torch.zeros((num_envs, self.num_agents, 3), dtype=torch.int32, device=self.device)
         self._h2d_done, self._h2d_pending = None, False
         FinalObservation.__init__(self, final_observation)
+        NextStepAutoreset.__init__(self, autoreset_mode)
 
     def game(self, env=0):
         rules_name, player_names, agent_ids, iz, mz = self._ctor

@@ -165,7 +165,33 @@ class FinalObservation(object):
         return info
 
 
-class ZombsoleVectorEnv(CompactHostOutputs, FinalObservation):
+def _next_step_mode():
+    """gymnasium's AutoresetMode.NEXT_STEP where gymnasium has it, else its value."""
+    try:
+        from gymnasium.vector import AutoresetMode
+        return AutoresetMode.NEXT_STEP
+    except ImportError:
+        return "next_step"
+
+
+class NextStepAutoreset(object):
+    """autoreset_mode="next_step" (gymnasium's AutoresetMode.NEXT_STEP; include/zs_b200.h: ZS_AUTORESET_NEXT_STEP): the step
+    that ends an episode returns its terminal observation, reward and flags and leaves the world as it is; the env's next
+    step ignores its action, re-initialises the world and returns the new episode's first observation with reward 0 and
+    both flags false.  Works with every host_outputs value.  ``metadata["autoreset_mode"]`` says so (an instance copy);
+    ``autoreset_envs`` (bool [N] on the device, read-only) marks the envs whose next step is such a reset step."""
+
+    def __init__(self, autoreset_mode):
+        self.autoreset_mode = autoreset_mode
+        if autoreset_mode == "next_step":
+            self.metadata = dict(type(self).metadata, autoreset_mode=_next_step_mode())
+
+    @property
+    def autoreset_envs(self):
+        return self.engine.autoreset_pending()
+
+
+class ZombsoleVectorEnv(CompactHostOutputs, FinalObservation, NextStepAutoreset):
     """``num_envs`` independent ZombsoleGymEnv worlds on one GPU (constructor: gym_env.py:49-53)."""
 
     metadata = {"render.modes": ["human"]}
@@ -183,18 +209,19 @@ class ZombsoleVectorEnv(CompactHostOutputs, FinalObservation):
                  render_mode=None, observation_scope="world", observation_position_encoding="simple",
                  agent_weapon="rifle", debug=False, *, num_envs=1, device="cuda", seed=0, env_index_base=0,
                  max_episode_steps=None, auto_reset=True, host_outputs=False, host_threads=0, compact_words=0,
-                 final_observation=False):
+                 final_observation=False, autoreset_mode="same_step"):
         if render_mode is not None:
             if render_mode not in self.metadata["render.modes"]:
                 raise ValueError("render_mode={} is not supported".format(render_mode))
             raise NotImplementedError("rendering is outside the batched simulator's scope (render_mode=None only)")
         self.render_mode = None
         check_final_observation(final_observation, auto_reset, host_outputs)
+        abi.check_autoreset_mode(autoreset_mode, auto_reset, final_observation)
         scope, enc, width = abi.parse_observation_scope(observation_scope, observation_position_encoding)
         self.cfg = abi.make_config(rules_name, list(player_names), [agent_id], [agent_weapon], initial_zombies,
                                    minimum_zombies, scope, enc, width, False, num_envs, seed=seed,
                                    env_index_base=env_index_base, max_episode_steps=max_episode_steps,
-                                   auto_reset=auto_reset)
+                                   auto_reset=auto_reset, autoreset_mode=autoreset_mode)
         self.engine = ZsEngine(self.cfg, map_name, device=device)
         self.num_envs = num_envs
         self.device = self.engine.device
@@ -241,6 +268,7 @@ class ZombsoleVectorEnv(CompactHostOutputs, FinalObservation):
         self._act_dev = torch.zeros((num_envs, 1), dtype=torch.int32, device=self.device)
         self._h2d_done, self._h2d_pending = None, False
         FinalObservation.__init__(self, final_observation)
+        NextStepAutoreset.__init__(self, autoreset_mode)
 
     # -- the reference's object protocol for one world of the batch
     def game(self, env=0):
@@ -348,7 +376,7 @@ class ZombsoleVectorEnv(CompactHostOutputs, FinalObservation):
 
     def rollout(self, n_steps, actions=None, first_step_index=0, obs=None, reward=None, terminated=None, truncated=None,
                 final_obs=None):
-        """``n_steps`` transitions in one kernel launch with same-step auto-reset.  ``actions`` is an int32
+        """``n_steps`` transitions in one kernel launch with same-step auto-reset (next-step with autoreset_mode="next_step").  ``actions`` is an int32
         tensor [n_steps, N] of discrete ids or None for the synthetic uniform stream.  ``final_obs``: a ring shaped like
         ``obs`` (or like the env's observation when ``obs`` is None) that receives, in step i's slot, the observation each env
         whose episode step i ended had before it was re-initialised (the rows where terminated | truncated)."""
