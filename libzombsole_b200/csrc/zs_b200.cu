@@ -938,9 +938,14 @@ static cudaError_t set_smem_attr_step(int bytes) {
 template <int MPC, int G>
 static cudaError_t set_smem_attr_for(int bytes) {
     const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
-    cudaError_t e = set_smem_attr_step<MPC, G, ZS_MIN_CTAS>(bytes);
-    if (e == cudaSuccess && MPC <= 32) e = set_smem_attr_step<MPC, G, (MPC <= 32 ? ZS_MIN_CTAS_LOWOCC : ZS_MIN_CTAS)>(bytes);
-    if (e == cudaSuccess && G == 16) e = set_smem_attr_step<MPC, G, (G == 16 ? ZS_MIN_CTAS_G16 : ZS_MIN_CTAS)>(bytes);
+    cudaError_t e = cudaSuccess;
+    // only the occupancies launch_sim runs: the kernels with more slots than lanes step at ZS_OCC_GENERAL alone (compiling
+    // them for the others too would leave step kernels in the library that nothing can launch)
+    if constexpr (MPC <= 32) {
+        e = set_smem_attr_step<MPC, G, ZS_MIN_CTAS>(bytes);
+        if (e == cudaSuccess) e = set_smem_attr_step<MPC, G, ZS_MIN_CTAS_LOWOCC>(bytes);
+    }
+    if constexpr (G == 16) if (e == cudaSuccess) e = set_smem_attr_step<MPC, G, ZS_MIN_CTAS_G16>(bytes);
     if (e == cudaSuccess && G == 16 && MPC == 16) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_STEP, 16, 16, 3, ZS_MIN_CTAS_LOWOCC>, attr, bytes);
     if (e == cudaSuccess && MPC > 32) e = set_smem_attr_step<MPC, G, (MPC > 32 ? ZS_OCC_GENERAL : ZS_MIN_CTAS)>(bytes);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(zs_sim_kernel<MODE_RESET, MPC, G, 0, ZS_MIN_CTAS>, attr, bytes);

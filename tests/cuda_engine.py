@@ -18,6 +18,14 @@ class CudaEngine(object):
         self.draws = torch.zeros(e.N, dtype=torch.int32, device=e.device)
         self._cache = None
 
+    @classmethod
+    def of(cls, eng):
+        """The adapter around an engine made elsewhere (a vector env's): export() and fields() only."""
+        self = cls.__new__(cls)
+        self.eng, self._cache = eng, None
+        self.N, self.A, self.M, self.S, self.cells = eng.N, eng.A, eng.M, eng.S, eng.cells
+        return self
+
     def close(self):
         self.eng.close()
 

@@ -149,6 +149,17 @@ CONFIGS.update({
     "safehouse_edges": _single(_edge_map("edge_objectives"), rules="safehouse", players=["terminator"], zombies=6),
 })
 
+# single-agent world scope with 17-32 things: 32 slots, the world-scope kernels compiled for 32 slots per env
+CONFIGS.update({
+    # the bench game with 20 zombies: agent + 2 terminators + 20 zombies = 23 things
+    "bridge_world_32": _single("bridge", zombies=20),
+    # channels on fort (1,533 cells): agent + terminator + sniper + 24 zombies = 27 things
+    "fort_world_32": _single("fort", enc="channels", players=["terminator", "sniper"], weapon="shotgun", zombies=24),
+    # world scope at 256 slots: agent + 4 bots + 200 zombies, the minimum-zombie respawn
+    "fort_world_256": _single("fort", rules="survival", players=["sniper", "troll", "hamster", "terminator"], weapon="gun",
+                              zombies=200, minimum=195),
+})
+
 
 DISCRETE = [(abi.ACT_MOVE, 0, 1), (abi.ACT_MOVE, -1, 0), (abi.ACT_MOVE, 0, -1), (abi.ACT_MOVE, 1, 0),
             (abi.ACT_ATTACK_CLOSEST, 0, 0), (abi.ACT_HEAL, 0, 0), (abi.ACT_HEAL_CLOSEST, 0, 0)]

@@ -24,12 +24,14 @@ def test_cuda_reproduces_reference_trace(name):
     assert not errs, "\n".join(errs[:3])
 
 
-def lockstep(cfgd, N, T, seed, base=0, mes=0, wild=0.25, discrete=False):
-    """CUDA vs oracle, N envs, T ticks, manual masked resets; compares every output and the state."""
+def lockstep(cfgd, N, T, seed, base=0, mes=0, wild=0.25, discrete=False, auto_reset=False, seen=None):
+    """CUDA vs oracle, N envs, T ticks, manual masked resets; compares every output and the state.  With auto_reset both
+    re-initialise an ended env inside its step (same-step auto-reset) and the episode statistics are compared at the end.
+    `seen` (a dict) receives the number of episodes that ended."""
     from cuda_engine import CudaEngine
     from oracle import oracle as orc
     from libzombsole_b200 import abi
-    cfg, m = pu.build(cfgd, N, seed, env_index_base=base, max_episode_steps=mes)
+    cfg, m = pu.build(cfgd, N, seed, env_index_base=base, max_episode_steps=mes, auto_reset=auto_reset)
     cu, orc_env = CudaEngine(cfg, m), orc.OracleEnv(cfg, m)
     nf = pu.n_fixed_slots(cfgd)
     rs = np.random.RandomState(seed & 0xFFFFFFFF)
@@ -37,6 +39,7 @@ def lockstep(cfgd, N, T, seed, base=0, mes=0, wild=0.25, discrete=False):
     A = cfg.n_agents
     tapes = [pu.action_tape(cfgd, T, rs.randint(1 << 30), wild=wild) for _ in range(min(N, 8))]
     errs = []
+    ended = 0
     assert np.array_equal(cu.encode_obs(), orc_env.encode_obs())
     for t in range(T):
         if discrete:
@@ -62,12 +65,19 @@ def lockstep(cfgd, N, T, seed, base=0, mes=0, wild=0.25, discrete=False):
         if errs:
             break
         done = (want[2] | want[3]).astype(np.uint8)
-        if done.any():
+        ended += int(done.sum())
+        if done.any() and not auto_reset:
             ro_c, ro_o = cu.reset(done), orc_env.reset(done)
             sel = done.astype(bool)
             if not np.array_equal(ro_c[sel], ro_o[sel]):
                 errs.append("tick %d: reset obs differs" % t)
                 break
+    if auto_reset and not errs:
+        got, want = cu.eng.episode_stats().cpu().numpy(), orc_env.stats()
+        if not np.array_equal(got, want):
+            errs.append("episode statistics differ: %s vs %s" % (got, want))
+    if seen is not None:
+        seen["ended"] = ended
     cu.close()
     orc_env.close()
     return errs
@@ -87,6 +97,8 @@ CASES = [
     ("surr255_channels_odd_cells", 16, 40, 0), ("multi_strip_col", 96, 80, 0), ("multi_wide_max", 16, 40, 0),
     ("general_wide_max", 16, 40, 0), ("general_odd_cells", 96, 60, 0), ("minz_no_player_spawns", 96, 80, 0),
     ("minz_few_spawns", 96, 80, 0), ("crowded", 96, 60, 0), ("safehouse_edges", 96, 80, 20),
+    # single-agent world scope with 17-32 things (the 32-slot world-scope kernels)
+    ("bridge_world_32", 64, 80, 0), ("fort_world_32", 64, 60, 0),
 ]
 
 

@@ -15,7 +15,8 @@ CASES = [
     ("ZS_NO_TMA_PAIR", "1", "c1_bridge_ext", 2048, 48),
     ("ZS_SMEM_SKEW", "0", "c1_bridge_ext", 2048, 48),
     ("ZS_OCC", "4", "c1_bridge_ext", 1024, 48),
-    ("ZS_OCC", "6", "c1_bridge_ext", 1024, 48),
+    # (6 is accepted for two-env warps only: 4,096 envs is an even batch of more than 16 envs per SM)
+    ("ZS_OCC", "6", "c1_bridge_ext", 4096, 48),
     ("ZS_OCC", "7", "c1_bridge_ext", 1024, 48),
     ("ZS_WARPS_PER_CTA", "1", "c5_bridge_channels", 512, 48),
     ("ZS_WARPS_PER_CTA", "4", "c1_bridge_ext", 1024, 48),
